@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native 3D RoI hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): RoIs/s of 3D RoIAlign forward on workload C2 = BASELINE.json configs[1]
 ("3D RoIAlign fwd on one synthetic FPN P2 level 256ch x 40x128x128, 512 RoIs, 7x7x7 out, sampling_ratio 2").
@@ -18,6 +18,8 @@ device time.  One JSON line is printed by rank 0 with, besides the contract keys
                 spread is the machine's, not the draw's; after the timed region the ranks also run C4 -> C5 sharded one
                 volume per rank and all-gather the detections over NCCL (the path's only collective)
 `--impl reference` times the reference's own algorithm on the host cores (oracle port, all threads) on the same workload.
+`--dump-outputs DIR` writes what the last timed step returned (a fixed sample of it, see dump_outputs) as .npy files, so
+that two builds can be compared output for output: the inputs are seeded and the same from run to run.
 """
 import argparse
 import ctypes
@@ -56,7 +58,11 @@ def parse_args():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary rows (C3, NMS, backward)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none to write")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -167,6 +173,18 @@ def c2_inputs(torch, dev, rank):
     feats_cl = feats.contiguous(memory_format=torch.channels_last_3d)
     rois_np = synth.c2_rois(C2["K"], seed=2)
     return feats, feats_cl, rois_np
+
+
+DUMP_ROIS = 128   # of the 512 RoIs of a step: 128 x 256 x 7^3 fp32 = 45 MB
+
+
+def dump_outputs(torch, out_dir, out):
+    """The step returns the pooled features [512, 256, 7, 7, 7] fp32 (180 MB).  Writes those of a fixed, seeded
+    sample of DUMP_ROIS RoIs, all channels, in ascending RoI order, as out_dir/roi_align3d_out.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(out.shape[0], DUMP_ROIS, replace=False))
+    sample = out.index_select(0, torch.from_numpy(idx).to(out.device))
+    np.save(os.path.join(out_dir, "roi_align3d_out.npy"), sample.cpu().numpy())
 
 
 def time_steps(torch, fn, steps, warmup, dist=None):
@@ -281,12 +299,18 @@ def main():
 
     # ---- headline: device-resident inputs ----------------------------------------------------------------
     launches = [0]
+    last_out = [None]
 
     def step():
-        layer(feats_cl, rois)
+        out = layer(feats_cl, rois)
         launches[0] += 1
+        if launches[0] == warmup + steps:   # only the last timed step's output is kept: the others reuse one buffer
+            last_out[0] = out
 
     total_ms, per = time_steps(torch, step, steps, warmup, dist)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, last_out[0])
+    last_out[0] = None
     gpu_launches = 2 * steps  # per step: roi_align3d_plan_kernel (7 us) + roi_align3d_fwd_stream_kernel
     value = world * C2["K"] * steps / (total_ms * 1e-3)
     kernel_ms = float(np.median(per))  # per-step event time = plan kernel + streamed kernel (+ the launch gap)

@@ -19,21 +19,3 @@ def oracle():
     import oracle as _oracle
     _oracle.build()
     return _oracle
-
-
-@pytest.fixture(scope="session")
-def ref_ops():
-    """The reference's own kernels built by oracle/build_ref.sh (None when oracle/_ref is absent)."""
-    ref_dir = os.path.join(ROOT, "oracle", "_ref")
-    if ref_dir not in sys.path:
-        sys.path.insert(0, ref_dir)
-    mods = {}
-    try:
-        import torch  # noqa: F401  (the extensions link against libtorch)
-        import ref_nms_cuda
-        import ref_roi_align_cuda
-        mods["nms_cuda"] = ref_nms_cuda
-        mods["roi_align_cuda"] = ref_roi_align_cuda
-    except Exception as e:  # pragma: no cover - depends on the box
-        mods["error"] = repr(e)
-    return mods

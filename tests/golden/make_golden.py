@@ -21,31 +21,32 @@ import synth  # noqa: E402
 out_dir = sys.argv[1] if len(sys.argv) > 1 else HERE
 os.makedirs(out_dir, exist_ok=True)
 dev = torch.device("cuda:0")
-rng = np.random.default_rng(2024)
 
 # ---- RoIAlign3D forward / backward ------------------------------------------------------------------------
-shape = (2, 6, 7, 13, 12)
-feats = rng.standard_normal(shape).astype(np.float32)
+# the features and the output gradients are not stored: synth.roi_align_ref_draws draws them again from a seed
+cfgs = [("c7", 7, 7, 2), ("m14x10", 14, 10, 2), ("b7x3", 7, 3, 2), ("a5", 5, 5, 0)]
+assert tuple(c[0] for c in cfgs) == synth.ROI_ALIGN_REF_TAGS
 rois = np.concatenate([synth.c2_rois(10, seed=11, img=(48, 52, 14), batch=2),
                        synth.adversarial_rois((7, 13, 12), 0.25, 0.5, batch=2)], 0)
-ft, rt = torch.from_numpy(feats).to(dev), torch.from_numpy(rois).to(dev)
-pack = dict(feats=feats, rois=rois, spatial_scale=np.float32(0.25), spatial_scale_depth=np.float32(0.5))
-for tag, ps, pdp, sn in [("c7", 7, 7, 2), ("m14x10", 14, 10, 2), ("b7x3", 7, 3, 2), ("a5", 5, 5, 0)]:
-    r = rois
-    if sn == 0:
-        ok = (rois[:, 3] >= rois[:, 1]) & (rois[:, 4] >= rois[:, 2]) & (rois[:, 6] >= rois[:, 5])
-        r = rois[ok]
+tag_rois = []
+for tag, ps, pdp, sn in cfgs:
+    ok = (rois[:, 3] >= rois[:, 1]) & (rois[:, 4] >= rois[:, 2]) & (rois[:, 6] >= rois[:, 5])
+    tag_rois.append(rois[ok] if sn == 0 else rois)
+feats, gouts = synth.roi_align_ref_draws([(r.shape[0], 6, pdp, ps, ps) for r, (_, ps, pdp, _) in zip(tag_rois, cfgs)])
+shape = feats.shape
+ft = torch.from_numpy(feats).to(dev)
+pack = dict(rois=rois, spatial_scale=np.float32(0.25), spatial_scale_depth=np.float32(0.5),
+            draws_sha256=np.array(synth.roi_align_ref_digest(feats, gouts)))
+for (tag, ps, pdp, sn), r, g in zip(cfgs, tag_rois, gouts):
     rr = torch.from_numpy(r).to(dev)
     out = torch.zeros(r.shape[0], shape[1], pdp, ps, ps, device=dev)
     ra.forward3d(ft, rr, pdp, ps, ps, 0.25, 0.5, sn, out)
-    g = rng.standard_normal(tuple(out.shape)).astype(np.float32)
     grad = torch.zeros(shape, device=dev)
     ra.backward3d(torch.from_numpy(g).to(dev), rr, pdp, ps, ps, 0.25, 0.5, sn, grad)
     torch.cuda.synchronize()
     pack["%s_cfg" % tag] = np.array([ps, pdp, sn], np.int32)
     pack["%s_rois" % tag] = r
     pack["%s_out" % tag] = out.cpu().numpy()
-    pack["%s_gout" % tag] = g
     pack["%s_gin" % tag] = grad.cpu().numpy()     # NB: the reference's non-cubic top_diff index (bug_compat)
 np.savez_compressed(os.path.join(out_dir, "roi_align3d_ref.npz"), **pack)
 

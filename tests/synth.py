@@ -1,4 +1,6 @@
 """Seeded synthetic inputs of BASELINE.md / SURVEY 8(d) (C1..C4), shared by tests and bench.py."""
+import hashlib
+
 import numpy as np
 
 
@@ -47,6 +49,36 @@ def c3_rois(k_per_vol=512, vols=2, seed=4, img=(512, 512, 80)):
     x1, y1, z1 = rng.uniform(0, W - 1 - w), rng.uniform(0, H - 1 - w), rng.uniform(0, D - 1 - d)
     b = np.repeat(np.arange(vols), k_per_vol).astype(np.float64)
     return np.stack([b, x1, y1, x1 + w - 1, y1 + w - 1, z1, z1 + d - 1], axis=1).astype(np.float32)
+
+
+ROI_ALIGN_REF_TAGS = ("c7", "m14x10", "b7x3", "a5")
+
+
+def roi_align_ref_draws(out_shapes):
+    """The random inputs of tests/golden/roi_align3d_ref.npz, drawn from one seeded stream in this order: the
+    features, then one output gradient per shape.  The file does not store them (it would pass 1 MB)."""
+    rng = np.random.default_rng(2024)
+    feats = rng.standard_normal((2, 6, 7, 13, 12)).astype(np.float32)
+    return feats, [rng.standard_normal(s).astype(np.float32) for s in out_shapes]
+
+
+def roi_align_ref_digest(feats, gouts):
+    """sha256 of the drawn arrays, stored beside the reference outputs as "draws_sha256"."""
+    h = hashlib.sha256(feats.tobytes())
+    for g in gouts:
+        h.update(g.tobytes())
+    return h.hexdigest()
+
+
+def load_roi_align_ref(path):
+    """tests/golden/roi_align3d_ref.npz with "feats" and "<tag>_gout" drawn again by roi_align_ref_draws."""
+    z = dict(np.load(path))
+    z["feats"], gouts = roi_align_ref_draws([z["%s_out" % t].shape for t in ROI_ALIGN_REF_TAGS])
+    if roi_align_ref_digest(z["feats"], gouts) != str(z["draws_sha256"]):
+        raise RuntimeError("numpy %s draws a different stream from default_rng(2024) than the one %s was made with: "
+                           "its features and output gradients have to be stored again" % (np.__version__, path))
+    z.update(("%s_gout" % t, g) for t, g in zip(ROI_ALIGN_REF_TAGS, gouts))
+    return z
 
 
 def adversarial_rois(feat_dhw, scale, scale_d, batch=1, seed=7):

@@ -1,10 +1,12 @@
 """GPU parity tests (run on the B200 box: pytest -m gpu).  Everything goes through the C ABI
 (libroi3d_b200.so via the Python host mirror) and is compared with the CPU oracle on the same seeded inputs;
-where oracle/_ref is present the reference's OWN kernels are run beside it, which pins the oracle.
+the reference's OWN kernels are represented by their outputs stored under tests/golden/ (tests/golden/make_golden.py).
 
 Tolerances (BASELINE.json north_star): NMS keep lists bit-exact; RoIAlign forward 1e-5, backward 1e-4,
 measured as max|a-b| / max(1, max|ref|)  (norm-relative: pure elementwise relative error is ill-conditioned on
 zero-mean data, SURVEY section 7)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -12,6 +14,7 @@ import torch
 import synth
 
 pytestmark = pytest.mark.gpu
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 FWD_TOL = 1e-5
 BWD_TOL = 1e-4
@@ -110,17 +113,34 @@ def test_nms_batched_segments(oracle, dev):
         assert np.array_equal(keep_s[s, :num[s]].cpu().numpy(), want_s)
 
 
-def test_nms_against_reference_kernel(oracle, ref_ops, dev):
-    """Pins the oracle: the reference's own nms_cuda_3d (oracle/_ref) on the same boxes."""
-    if "nms_cuda" not in ref_ops:
-        pytest.skip("oracle/_ref not built: %s" % ref_ops.get("error"))
+def _mirrored_copies(dets, keep, copies):
+    """A stored NMS case copied into other octants (copy j negates x, y and / or z by the bits of j, which leaves every
+    IoU inside the copy as it was; boxes of different copies can meet only on a mirror plane, and for the cases copied
+    here no such contact reaches the threshold, which the oracle check confirms) with its scores scaled by 2^-j (exact:
+    the order inside a copy stays, and no two scores are equal).  Greedy NMS then keeps in every copy what it kept in
+    the original, so the reference's keep list of the whole set is the stored one repeated."""
+    n, parts = dets.shape[0], []
+    for j in range(copies):
+        d = dets.copy()
+        for bit, (lo, hi) in enumerate([(0, 2), (1, 3), (4, 5)]):
+            if j >> bit & 1:
+                d[:, [lo, hi]] = -dets[:, [hi, lo]]
+        d[:, 6] = dets[:, 6] * np.float32(2.0 ** -j)
+        parts.append(d)
+    return np.concatenate(parts), np.concatenate([keep + j * n for j in range(copies)])
+
+
+def test_nms_against_reference_kernel(oracle, dev):
+    """The keep lists of the reference's own nms_cuda_3d, stored in tests/golden/nms3d_ref.npz (65 to 1000 boxes), and
+    the three larger cases copied up to 2000-2100 boxes (the full 32-word mask panel) by _mirrored_copies."""
     from roi3d_b200.ops import nms
-    for n, thr, seed in [(2000, 0.7, 0), (2000, 0.3, 1), (777, 0.5, 2)]:
-        dets = synth.c1_boxes(n, seed=seed)
-        t = torch.from_numpy(dets).to(dev)
-        ref = ref_ops["nms_cuda"].nms_3d(t, thr).cpu().numpy()
+    z = np.load(os.path.join(GOLDEN, "nms3d_ref.npz"))
+    for t, copies in [("a", 1), ("b", 1), ("c", 1), ("d", 1), ("a", 7), ("b", 7), ("d", 2)]:
+        dets, ref = _mirrored_copies(z["%s_dets" % t], z["%s_keep" % t], copies)
+        thr = float(z["%s_thr" % t])
+        assert len(np.unique(dets[:, 6])) == len(dets)
         assert np.array_equal(ref, oracle.nms3d(dets, thr)), "oracle disagrees with the reference kernel"
-        assert np.array_equal(nms(t, thr)[1].cpu().numpy(), ref)
+        assert np.array_equal(nms(torch.from_numpy(dets).to(dev), thr)[1].cpu().numpy(), ref)
 
 
 # ------------------------------------------------------------------------------------------- RoIAlign
@@ -233,34 +253,41 @@ def test_roi_align_backward_bug_compat(oracle, dev):
     assert rel_err(ft.grad.cpu().numpy(), want) <= BWD_TOL
 
 
-def test_roi_align_against_reference_kernels(oracle, ref_ops, dev):
-    """Pins the oracle: the reference's own forward3d / backward3d (oracle/_ref) on the same inputs."""
-    if "roi_align_cuda" not in ref_ops:
-        pytest.skip("oracle/_ref not built: %s" % ref_ops.get("error"))
-    from roi3d_b200.ops import RoIAlign3D
-    ra = ref_ops["roi_align_cuda"]
-    shape = (2, 64, 10, 32, 32)
-    f = _feats(shape, 8)
-    rois = np.concatenate([synth.c2_rois(40, seed=9, img=(128, 128, 20), batch=2),
-                           synth.adversarial_rois((10, 32, 32), 0.25, 0.5, batch=2)], 0)
-    ft, rt = torch.from_numpy(f).to(dev), torch.from_numpy(rois).to(dev)
-    for (ps, pdp) in [(7, 7), (14, 14)]:
-        ref_out = torch.zeros(rois.shape[0], 64, pdp, ps, ps, device=dev)
-        ra.forward3d(ft, rt, pdp, ps, ps, 0.25, 0.5, 2, ref_out)
-        torch.cuda.synchronize()
-        want = oracle.roi_align3d_forward(f, rois, ps, pdp, 0.25, 0.5, 2)
-        assert np.array_equal(ref_out.cpu().numpy(), want), "oracle(contract=1) is not bit-identical to the reference"
-        x = cl(ft.clone()).requires_grad_(True)
-        out = RoIAlign3D(ps, pdp, 0.25, 0.5, 2)(x, rt)
-        assert rel_err(out.detach().cpu().numpy(), ref_out.cpu().numpy()) <= FWD_TOL
-        g = torch.from_numpy(_feats(tuple(out.shape), 10)).to(dev)
-        ref_grad = torch.zeros(shape, device=dev)
-        ra.backward3d(g, rt, pdp, ps, ps, 0.25, 0.5, 2, ref_grad)
-        torch.cuda.synchronize()
-        out.backward(g)
-        assert rel_err(x.grad.cpu().numpy(), ref_grad.cpu().numpy()) <= BWD_TOL
-        assert rel_err(oracle.roi_align3d_backward(g.cpu().numpy(), rois, shape, 0.25, 0.5, 2),
-                       ref_grad.cpu().numpy()) <= BWD_TOL
+def test_roi_align_against_reference_kernels(dev):
+    """The outputs of the reference's own forward3d / backward3d, stored in tests/golden/roi_align3d_ref.npz for 6
+    channels, widened to 64 so that the product takes its streamed and planar kernels (they need C % 64 == 0 or
+    C % 4 == 0).  The reference computes each channel from that channel alone and linearly, so a level whose channel c
+    is s_c * feats[:, src_c] (s_c a power of two: exact) has the output s_c * out[:, src_c], and output gradients built
+    the same way have the input gradient s_c * gin[:, src_c].  Non-cubic outputs: the reference's backward reads the
+    wrong top_diff element, so only there does the product run with bug_compat.  Tuning variant 60 puts the cubic
+    7-wide case on the planar forward and backward kernels as well."""
+    import roi3d_b200
+    from roi3d_b200.ops import RoIAlign3D, set_bug_compat
+    z = synth.load_roi_align_ref(os.path.join(GOLDEN, "roi_align3d_ref.npz"))
+    rng = np.random.default_rng(64)
+    src = rng.permutation(np.arange(64) % 6)
+    s = rng.choice(np.float32([-2, -1, -0.5, 0.5, 1, 2]), 64)[None, :, None, None, None]
+
+    def widen(a):
+        return np.ascontiguousarray(a[:, src] * s)
+    f, sc, scd = widen(z["feats"]), float(z["spatial_scale"]), float(z["spatial_scale_depth"])
+    runs = [(t, layout, 0) for t in synth.ROI_ALIGN_REF_TAGS for layout in ("channels_last", "contiguous")]
+    for tag, layout, variant in runs + [("c7", "channels_last", 60)]:
+        ps, pdp, sn = (int(v) for v in z["%s_cfg" % tag])
+        x = torch.from_numpy(f).to(dev)
+        x = (cl(x) if layout == "channels_last" else x).requires_grad_(True)
+        roi3d_b200._lib.set_tuning(0, variant)
+        roi3d_b200._lib.set_tuning(1, variant)
+        set_bug_compat(ps != pdp)
+        try:
+            out = RoIAlign3D(ps, pdp, sc, scd, sn)(x, torch.from_numpy(z["%s_rois" % tag]).to(dev))
+            out.backward(torch.from_numpy(widen(z["%s_gout" % tag])).to(dev))
+        finally:
+            set_bug_compat(False)
+            roi3d_b200._lib.set_tuning(0, 0)
+            roi3d_b200._lib.set_tuning(1, 0)
+        assert rel_err(out.detach().cpu().numpy(), widen(z["%s_out" % tag])) <= FWD_TOL, (tag, layout, variant)
+        assert rel_err(x.grad.cpu().numpy(), widen(z["%s_gin" % tag])) <= BWD_TOL, (tag, layout, variant)
 
 
 # ------------------------------------------------------------------------------- extractor / levels
