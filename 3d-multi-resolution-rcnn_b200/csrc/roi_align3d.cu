@@ -2005,6 +2005,17 @@ int roi3d_extract_backward(const roi3d_level_t *levels, int num_levels, int B, i
   return dispatch_bwd(p, st);
 }
 
+int roi3d_extract_backward_deterministic(const roi3d_level_t *levels, int num_levels, int B, int C, const float *rois_dev,
+                                         int K, int PD, int PH, int PW, int sample_num, float finest_scale,
+                                         const float *grad_out_dev, int accumulate, void *stream) {
+  RoiParams p;
+  int rc = fill_params(p, levels, num_levels, B, C, rois_dev, K, PD, PH, PW, sample_num, finest_scale, true);
+  if (rc) return rc;
+  ROI3D_CHECK_ARG(K == 0 || grad_out_dev != nullptr, "grad_out is NULL");
+  p.grad_out = grad_out_dev;
+  return launch_bwd_det(p, accumulate, (cudaStream_t)stream);
+}
+
 int roi3d_roi_align3d_forward(const float *feats_dev, int layout, int B, int C, int D, int H, int W,
                               const float *rois_dev, int K, int PD, int PH, int PW, float spatial_scale,
                               float spatial_scale_depth, int sample_num, float *out_dev, void *stream) {

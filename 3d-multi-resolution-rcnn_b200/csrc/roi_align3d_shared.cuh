@@ -259,4 +259,9 @@ int launch_bwd_stream(RoiParams &p, cudaStream_t st);
 bool fwd_stream_ok(const RoiParams &p);
 int launch_fwd_stream(RoiParams &p, cudaStream_t st);
 
+// Deterministic backward (roi_align3d_det.cu; any output size, channels-last gradients): one CTA per gradient tile
+// gathers the RoIs that meet it in ascending index and writes each voxel once -- overwriting it (accumulate = 0,
+// every voxel of every level, no zero-fill needed) or adding its finished sum to the old value (accumulate = 1).
+int launch_bwd_det(RoiParams &p, int accumulate, cudaStream_t st);
+
 }  // namespace roi3d

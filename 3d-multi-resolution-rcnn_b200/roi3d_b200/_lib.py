@@ -23,6 +23,21 @@ class Level(ctypes.Structure):
                 ("spatial_scale", c_float), ("spatial_scale_depth", c_float)]
 
 
+def level_array(tensors, scales, scales_d, grads=None, layout=NDHWC):
+    """roi3d_level_t[] for the levels `tensors` ([B,C,D,H,W] each): feature pointers for a forward call, or with
+    `grads` the gradient pointers of a backward call."""
+    arr = (Level * len(tensors))()
+    for i, t in enumerate(tensors):
+        _, _, D, H, W = t.shape
+        arr[i].feats_dev = t.data_ptr() if grads is None else None
+        arr[i].grad_dev = None if grads is None else grads[i].data_ptr()
+        arr[i].layout = layout
+        arr[i].D, arr[i].H, arr[i].W = D, H, W
+        arr[i].spatial_scale = scales[i]
+        arr[i].spatial_scale_depth = scales_d[i]
+    return arr
+
+
 class Roi3dError(RuntimeError):
     pass
 
@@ -51,6 +66,8 @@ def _load():
                                           c_int, c_float, P, P, P]),
         "roi3d_extract_backward": (c_int, [ctypes.POINTER(Level), c_int, c_int, c_int, P, c_int, c_int, c_int, c_int,
                                            c_int, c_float, P, c_int, c_int, P]),
+        "roi3d_extract_backward_deterministic": (c_int, [ctypes.POINTER(Level), c_int, c_int, c_int, P, c_int, c_int,
+                                                         c_int, c_int, c_int, c_float, P, c_int, P]),
         "roi3d_ncdhw_to_ndhwc": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, P]),
         "roi3d_ndhwc_to_ncdhw": (c_int, [P, P, c_int, c_int, c_int, c_int, c_int, P]),
         "roi3d_nms3d_workspace_bytes": (c_size_t, [c_int, c_int]),

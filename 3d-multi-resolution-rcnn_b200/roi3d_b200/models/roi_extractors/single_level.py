@@ -19,20 +19,7 @@ from torch.autograd import Function
 from ... import _lib, ops
 from ..._util import (channels_last_to_contiguous, check_cuda_f32, forward_inputs, is_channels_last_3d, nvtx_range,
                       stream_ptr)
-from ...ops.roi_align.functions.roi_align_3d import _BUG_COMPAT, _out_dims
-
-
-def _level_array(tensors, scales, scales_d, grads=None, layout=_lib.NDHWC):
-    arr = (_lib.Level * len(tensors))()
-    for i, t in enumerate(tensors):
-        _, _, D, H, W = t.shape
-        arr[i].feats_dev = t.data_ptr() if grads is None else None
-        arr[i].grad_dev = None if grads is None else grads[i].data_ptr()
-        arr[i].layout = layout
-        arr[i].D, arr[i].H, arr[i].W = D, H, W
-        arr[i].spatial_scale = scales[i]
-        arr[i].spatial_scale_depth = scales_d[i]
-    return arr
+from ...ops.roi_align.functions.roi_align_3d import _BUG_COMPAT, _out_dims, deterministic_backward
 
 
 class _MultiLevelRoIAlign3D(Function):
@@ -54,7 +41,7 @@ class _MultiLevelRoIAlign3D(Function):
         ctx.input_channels_last = [is_channels_last_3d(f) for f in feats]
         ctx.save_for_backward(rois)
         if K > 0:
-            arr = _level_array(feats_in, scales, scales_d, layout=layout)
+            arr = _lib.level_array(feats_in, scales, scales_d, layout=layout)
             with torch.cuda.device(rois.device), nvtx_range("roi3d.extract.forward"):
                 _lib.check(_lib.lib.roi3d_extract_forward(arr, len(feats), B, C, rois.data_ptr(), K, out_d, out_h,
                                                           out_w, int(sample_num), float(finest_scale),
@@ -74,11 +61,17 @@ class _MultiLevelRoIAlign3D(Function):
         B, C = ctx.shapes[0][:2]
         grads = [torch.empty(s, dtype=grad_out.dtype, device=grad_out.device, memory_format=torch.channels_last_3d)
                  for s in ctx.shapes]
-        arr = _level_array(grads, scales, scales_d, grads=grads)
+        arr = _lib.level_array(grads, scales, scales_d, grads=grads)
         with torch.cuda.device(grad_out.device):
-            _lib.check(_lib.lib.roi3d_extract_backward(arr, nlev, B, C, rois.data_ptr(), K, out_d, out_h, out_w,
-                                                       sample_num, finest_scale, grad_out.data_ptr(), 1,
-                                                       int(_BUG_COMPAT[0]), stream_ptr()))
+            if deterministic_backward("SingleRoIExtractor backward"):
+                # every voxel of every level is written once (no zero-fill, no atomics): the same bits on every run
+                _lib.check(_lib.lib.roi3d_extract_backward_deterministic(
+                    arr, nlev, B, C, rois.data_ptr(), K, out_d, out_h, out_w, sample_num, finest_scale,
+                    grad_out.data_ptr(), 0, stream_ptr()))
+            else:
+                _lib.check(_lib.lib.roi3d_extract_backward(arr, nlev, B, C, rois.data_ptr(), K, out_d, out_h, out_w,
+                                                           sample_num, finest_scale, grad_out.data_ptr(), 1,
+                                                           int(_BUG_COMPAT[0]), stream_ptr()))
         outs = []
         for g, cl, nd in zip(grads, ctx.input_channels_last, need):
             outs.append(None if not nd else (g if cl else channels_last_to_contiguous(g)))

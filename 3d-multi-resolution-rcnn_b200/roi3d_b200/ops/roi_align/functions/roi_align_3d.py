@@ -4,6 +4,8 @@ Mirrors mmdet/ops/roi_align/functions/roi_align_3d.py:9-38,69-89 of the referenc
 arguments, same saved state, same gradient arity), minus its breakpoint() on tuple out_size (:15) and the
 redundant zero-fill of the output (:32).  CPU input raises NotImplementedError exactly as :36-37 does.
 """
+import warnings
+
 import torch
 from torch.autograd import Function
 
@@ -62,10 +64,17 @@ class RoIAlignFunction3D(Function):
             grad_cl = torch.empty((B, C, D, H, W), dtype=grad_output.dtype, device=grad_output.device,
                                   memory_format=torch.channels_last_3d)
             with torch.cuda.device(grad_output.device), nvtx_range("roi3d.roi_align3d.backward"):
-                _lib.check(_lib.lib.roi3d_roi_align3d_backward(
-                    grad_output.data_ptr(), rois.data_ptr(), K, out_d, out_h, out_w, ctx.spatial_scale,
-                    ctx.spatial_scale_depth, ctx.sample_num, grad_cl.data_ptr(), _lib.NDHWC, B, C, D, H, W,
-                    1, int(_BUG_COMPAT[0]), stream_ptr()))
+                if deterministic_backward("RoIAlignFunction3D.backward"):
+                    # every voxel is written once (no zero-fill, no atomics): the same bits on every run
+                    lv = _lib.level_array([grad_cl], [ctx.spatial_scale], [ctx.spatial_scale_depth], grads=[grad_cl])
+                    _lib.check(_lib.lib.roi3d_extract_backward_deterministic(
+                        lv, 1, B, C, rois.data_ptr(), K, out_d, out_h, out_w, ctx.sample_num, 56.0,
+                        grad_output.data_ptr(), 0, stream_ptr()))
+                else:
+                    _lib.check(_lib.lib.roi3d_roi_align3d_backward(
+                        grad_output.data_ptr(), rois.data_ptr(), K, out_d, out_h, out_w, ctx.spatial_scale,
+                        ctx.spatial_scale_depth, ctx.sample_num, grad_cl.data_ptr(), _lib.NDHWC, B, C, D, H, W,
+                        1, int(_BUG_COMPAT[0]), stream_ptr()))
             grad_input = grad_cl if ctx.input_channels_last else channels_last_to_contiguous(grad_cl)
         return grad_input, None, None, None, None, None, None
 
@@ -78,6 +87,24 @@ _BUG_COMPAT = [False]
 
 def set_bug_compat(flag):
     _BUG_COMPAT[0] = bool(flag)
+
+
+def deterministic_backward(op):
+    """True when the backward of `op` has to take the deterministic kernel: torch.use_deterministic_algorithms(True)
+    is in force.  The default backward adds into the gradient with float atomics, so its last bits change from run to
+    run wherever RoIs overlap.  bug_compat exists only in the atomic kernel: with the flag on it raises, as torch does
+    for an op without a deterministic implementation, or under warn_only=True warns and keeps the atomic path."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return False
+    if _BUG_COMPAT[0]:
+        msg = ("%s with set_bug_compat(True) does not have a deterministic implementation, but you set "
+               "'torch.use_deterministic_algorithms(True)'. Call set_bug_compat(False), or use the 'warn_only=True' "
+               "option to run the atomic backward with a warning." % op)
+        if torch.is_deterministic_algorithms_warn_only_enabled():
+            warnings.warn(msg, UserWarning)
+            return False
+        raise RuntimeError(msg)
+    return True
 
 
 roi_align_3d = RoIAlignFunction3D.apply

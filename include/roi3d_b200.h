@@ -123,6 +123,16 @@ int roi3d_extract_backward(const roi3d_level_t *levels, int num_levels, int B, i
                            int K, int PD, int PH, int PW, int sample_num, float finest_scale,
                            const float *grad_out_dev, int zero_fill, int bug_compat, void *stream);
 
+/* Deterministic form of roi3d_extract_backward: the same gradient, the same bits on every run (no float atomics; what
+ * torch.use_deterministic_algorithms(True) asks for).  Each gradient voxel is written once by its owner, which adds
+ * the contributions of the RoIs that touch it in ascending RoI index.  accumulate=0: every voxel of every level's
+ * grad_dev is overwritten, K == 0 included (zeros; no memset needed); accumulate=1: each voxel's finished sum is added
+ * to its old value with one fp32 add.  num_levels == 1 is the plain RoIAlign3D backward.  Channels-last (ROI3D_NDHWC)
+ * gradients only; any output size and channel count; no bug_compat (the correct gradient only). */
+int roi3d_extract_backward_deterministic(const roi3d_level_t *levels, int num_levels, int B, int C,
+                                         const float *rois_dev, int K, int PD, int PH, int PW, int sample_num,
+                                         float finest_scale, const float *grad_out_dev, int accumulate, void *stream);
+
 /* Layout conversion of one level, [B,C,D,H,W] <-> channels-last; used by the host mirror when a caller
  * hands the reference's NCDHW-contiguous tensors to the channels-last kernels. */
 int roi3d_ncdhw_to_ndhwc(const float *src_dev, float *dst_dev, int B, int C, int D, int H, int W, void *stream);
