@@ -645,8 +645,6 @@ static NmsWorkspace carve(void *base, int nseg, int n_max) {
   return w;
 }
 
-int g_nms_mask_variant = 0;  // roi3d_set_tuning key 6: 1 = always the 4-tiles-per-CTA mask kernel
-
 }  // namespace roi3d
 
 using namespace roi3d;
@@ -685,7 +683,7 @@ static int nms3d_launch(const float *dets_dev, const int32_t *seg_counts_dev, co
   ROI3D_LAUNCH_CHECK();
   // tiles of the upper triangle: with few of them, one tile per CTA (4x the threads) fills the GPU better
   const long long tiles = (long long)nseg * cbm * (cbm + 1) / 2;
-  if (tiles <= 4096 && g_nms_mask_variant != 1) {
+  if (tiles <= 4096) {
     if (f64)
       nms3d_mask_q_kernel<true><<<dim3(cbm, cbm, nseg), 256, 0, st>>>(w.sorted, seg_counts_dev, n_max, iou_thr, iou_thr64,
                                                                       w.mask);

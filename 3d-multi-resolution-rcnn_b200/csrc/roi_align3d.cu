@@ -25,7 +25,6 @@
 // RoIs whose footprint exceeds the table capacity, and output widths other than 7/14, take the
 // "generic" path: the same warp-per-(RoI, channel-vector) mapping evaluating the reference's sample
 // loops literally (bit-exact against the oracle with contract=1).
-#include <cuda.h>
 #include <limits.h>
 
 #include "common.cuh"
@@ -529,54 +528,17 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring_kernel
   copy_out_tile<ROWS, PW, CV>(acc, count, stage, lane, NB, it.chunk, C, p.out + out_base, ch_stride);
 }
 
-// ---- TMA bulk-copy (cp.async.bulk, SASS UBLKCP) + mbarrier helpers for the per-warp row ring ----
-__device__ __forceinline__ void mbar_init(unsigned mbar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(mbar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(unsigned mbar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(mbar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned mbar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(mbar)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned mbar, unsigned parity) {
-  unsigned ok = 0;
-  for (int spin = 0; spin < (1 << 24); ++spin) {  // bounded: a byte-count mismatch traps instead of hanging the GPU
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-        : "=r"(ok)
-        : "r"(mbar), "r"(parity)
-        : "memory");
-    if (ok) return;
-  }
-  __trap();
-}
-
-// One TMA descriptor per pyramid level: the channels-last level seen as a 2-D tensor [voxel][channel], box =
-// (RXR voxels) x (one warp's channel chunk).  A whole feature row of the RoI footprint is then ONE
-// cp.async.bulk.tensor instruction issued by one lane (SASS UTMALDG) instead of RX/2 LDGSTS per warp.
-struct alignas(64) TmapSet {
-  CUtensorMap m[ROI3D_MAX_LEVELS];
-};
-__device__ __forceinline__ void tma_load_2d(unsigned dst, const void *tmap, int c0, int c1, unsigned mbar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n" ::"r"(dst),
-      "l"(tmap), "r"(c0), "r"(c1), "r"(mbar)
-      : "memory");
-}
-
 // Shared-memory layout of the ring2 kernel, shared by the kernel and its launcher.
-template <int PW, int ROWS, int CV, int NS, int RXR, int BULK>
+template <int PW, int ROWS, int CV, int NS, int RXR>
 struct Ring2Layout {
   static constexpr int VOX = 32 * CV;
   static constexpr int STRIDE = (RXR + 2) * VOX;
   static constexpr int RING = NS * STRIDE;
   static constexpr int STAGE = ROWS * PW * 33;
-  static constexpr int LISTS = BULK == 2 ? 512 : 480;  // bytes; TMA destinations must be 128-byte aligned
-  static constexpr int ALIGN = BULK == 2 ? 32 : 4;     // floats
+  // bytes: ylist[40] + zlist[40] bytes, yoff[40] + zoff[40] ints (0..400).  The 64 bytes at 416 are spare; the
+  // size is kept so that the shared-memory footprint, and with it the occupancy, stay as measured.
+  static constexpr int LISTS = 480;
+  static constexpr int ALIGN = 4;  // floats
   static constexpr int RING_OR_STAGE = RING > STAGE ? RING : STAGE;
   static constexpr int WARP_FLOATS = (LISTS / 4 + RING_OR_STAGE + ALIGN - 1) / ALIGN * ALIGN;
   static constexpr int SH_FLOATS = RXMAX * Tables<PW>::PWP + RYMAX * 16 + 40 * 16 + 32 + 3 * 32 * 2 + 16;
@@ -591,29 +553,28 @@ struct Ring2Layout {
 // the table build is the per-warp pipeline of roi_align3d_fwd_ring_kernel.
 // ---------------------------------------------------------------------------------------------
 constexpr int RZMAX2 = 40;
-template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB, int BULK, bool F2 = false, bool MULTI = false>
-__global__ void __launch_bounds__(kWarps * 32, MINB)
-    roi_align3d_fwd_ring2_kernel(const RoiParams p, const __grid_constant__ TmapSet tm) {
-  static_assert(!F2 || CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
+constexpr int PP2 = 16;  // padded row length of the CTA-shared y / z tables (PH, PD <= 16)
+template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB, bool MULTI>
+__global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kernel(const RoiParams p) {
+  static_assert(CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
   using TB = Tables<PW>;
-  using LY = Ring2Layout<PW, ROWS, CV, NS, RXR, BULK>;
+  using LY = Ring2Layout<PW, ROWS, CV, NS, RXR>;
   constexpr int PWP = TB::PWP;
   constexpr int VOX = 32 * CV;                 // floats per voxel-chunk
   constexpr int LPV = VOX / 4;                 // lanes (16 B each) per voxel-chunk
   constexpr int VPI = 32 / LPV;                // voxel-chunks copied per warp instruction
   constexpr int STRIDE = LY::STRIDE;           // floats per ring stage (two zero pad voxels)
-  constexpr int LISTS = LY::LISTS;             // ylist[40] + zlist[40] bytes + yoff[40] + zoff[40] ints + 8 mbarriers
+  constexpr int LISTS = LY::LISTS;             // ylist[40] + zlist[40] bytes + yoff[40] + zoff[40] ints
   constexpr int WARP_FLOATS = LY::WARP_FLOATS;
-  constexpr int PP = 16;                       // padded row length of the shared y / z tables (PH, PD <= 16)
   static_assert(LPV <= 32 && VPI >= 1, "voxel chunk wider than a warp copy");
   extern __shared__ __align__(128) float smem_r2[];
   float *smem_all = smem_r2;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
   // ---- CTA-shared per-RoI tables (all warps of a CTA work on the same RoI) ----
   float *SDx = smem_all;                       // [x - xmin][PWP]
-  float *SDy = SDx + RXMAX * PWP;              // [y - ymin][PP], all PH rows
-  float *SDz = SDy + RYMAX * PP;               // [z - zmin][PP], all PD slices
-  int *Sxlo = reinterpret_cast<int *>(SDz + RZMAX2 * PP);
+  float *SDy = SDx + RXMAX * PWP;              // [y - ymin][PP2], all PH rows
+  float *SDz = SDy + RYMAX * PP2;              // [z - zmin][PP2], all PD slices
+  int *Sxlo = reinterpret_cast<int *>(SDz + RZMAX2 * PP2);
   int *Sxhi = Sxlo + 16;
   int *Srng = Sxhi + 16;                       // [3 axes][32 roles][lo, hi]
   int *Sbox = Srng + 3 * 32 * 2;               // xmin, xmax, ymin, ymax, zmin, zmax
@@ -670,13 +631,13 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
   if (!T.empty && T.fits) {
     const int RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
     for (int i = tid; i < RX * PWP; i += kWarps * 32) SDx[i] = 0.0f;
-    for (int i = tid; i < RY * PP; i += kWarps * 32) SDy[i] = 0.0f;
-    for (int i = tid; i < RZ * PP; i += kWarps * 32) SDz[i] = 0.0f;
+    for (int i = tid; i < RY * PP2; i += kWarps * 32) SDy[i] = 0.0f;
+    for (int i = tid; i < RZ * PP2; i += kWarps * 32) SDz[i] = 0.0f;
   }
   __syncthreads();
   if (!T.empty && T.fits && role >= 0) {
     float *tab = role == 0 ? SDx : role == 1 ? SDy : SDz;
-    const int stride = role == 0 ? PWP : PP;
+    const int stride = role == 0 ? PWP : PP2;
     const int mn = role == 0 ? T.xmin : role == 1 ? T.ymin : T.zmin;
     for (int i = 0; i < ax.S; ++i) {
       Tap t = axis_tap(axis_coord(ax, lane, i), asize);
@@ -718,18 +679,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
 #pragma unroll
     for (int j = 0; j < NXU; ++j) tw[pw][j] = j < n ? T.Dx[(lo + j) * PWP + pw] : 0.0f;
   }
-  const unsigned mbar0 = (unsigned)__cvta_generic_to_shared(ylist + 416);
-  const unsigned ring_s = (unsigned)__cvta_generic_to_shared(ring);
-  if constexpr (BULK) {
-    static_assert(NS <= 8, "eight mbarriers per warp");
-    if (lane == 0) {
-      for (int sidx = 0; sidx < NS; ++sidx) mbar_init(mbar0 + sidx * 8, 1);
-      mbar_fence_init();
-    }
-    __syncwarp();
-  }
   int pstage = 0, cstage = 0;  // ring cursors persist across sub-items (every issued row is consumed)
-  unsigned cpar = 0;
 
   for (int g = 0; g < items_per_warp; ++g) {
   const int sub = first + g * kWarps + warp;
@@ -775,7 +725,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
       bool a = false;
       if (yy < RY) {
 #pragma unroll
-        for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP + it.ph0 + r] != 0.0f;
+        for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP2 + it.ph0 + r] != 0.0f;
       }
       const unsigned bal = __ballot_sync(FULL, a);
       if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
@@ -783,7 +733,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
     }
     for (int z0 = 0; z0 < RZ; z0 += 32) {
       const int zz = z0 + lane;
-      const bool a = zz < RZ && SDz[zz * PP + it.pd] != 0.0f;
+      const bool a = zz < RZ && SDz[zz * PP2 + it.pd] != 0.0f;
       const unsigned bal = __ballot_sync(FULL, a);
       if (a) zlist[nz + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)zz;
       nz += __popc(bal);
@@ -792,8 +742,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
     const int nrows = ny * nz;
 
     for (int sidx = 0; sidx < NS; ++sidx) {
-      // (TMA mode: the box always fills slots [0, RXR); taps past RX then read neighbouring voxels with weight 0)
-      float *padp = ring + sidx * STRIDE + (BULK == 2 ? RXR : RX) * VOX;
+      float *padp = ring + sidx * STRIDE + RX * VOX;
       for (int i = lane; i < 2 * VOX; i += 32) padp[i] = 0.0f;
     }
     __syncwarp();
@@ -810,55 +759,28 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
                         (long long)cv_v * C;
     float *dst0 = ring + cv_p * 4 + cv_v * VOX;
     // row offsets in units of 4 floats (16 B; C % 4 == 0), < 2^31 for any level the dispatcher accepts
-    if constexpr (BULK == 2) {  // TMA coordinates are voxel indices
-      for (int i = lane; i < nz; i += 32) zoff[i] = (int)zlist[i] * it.L.H * it.L.W;
-      for (int i = lane; i < ny; i += 32) yoff[i] = (int)ylist[i] * it.L.W;
-    } else {
-      for (int i = lane; i < nz; i += 32) zoff[i] = (int)(((long long)zlist[i] * slice_elems) >> 2);
-      for (int i = lane; i < ny; i += 32) yoff[i] = (int)(((long long)ylist[i] * row_elems) >> 2);
-    }
+    for (int i = lane; i < nz; i += 32) zoff[i] = (int)(((long long)zlist[i] * slice_elems) >> 2);
+    for (int i = lane; i < ny; i += 32) yoff[i] = (int)(((long long)ylist[i] * row_elems) >> 2);
     __syncwarp();
-    const int vbase = (((it.ok ? it.b : 0) * it.L.D + T.zmin) * it.L.H + T.ymin) * it.L.W + T.xmin;
-    const void *tmap = &tm.m[it.lvl];
     int pz = 0, py = 0;
-    // BULK == 1: lane v issues one cp.async.bulk of this warp's channel chunk of voxel v (<= 128*CV bytes,
-    // contiguous); BULK == 2: one tensor copy per row; completion is counted in bytes on the stage's mbarrier.
-    const unsigned chunk_bytes = (unsigned)min(VOX, C - it.chunk * VOX) * 4u;
-    const float *srcb = fb_roi + ((long long)T.zmin * it.L.H + T.ymin) * row_elems + (long long)T.xmin * C +
-                        (long long)it.chunk * VOX;
     auto issue = [&]() {
-      if constexpr (BULK == 2) {
-        if (lane == 0) {
-          const unsigned mb = mbar0 + pstage * 8;
-          mbar_expect_tx(mb, (unsigned)(RXR * VOX * 4));
-          tma_load_2d(ring_s + (unsigned)(pstage * STRIDE) * 4u, tmap, it.chunk * VOX, vbase + zoff[pz] + yoff[py], mb);
-        }
-      } else if constexpr (BULK == 1) {
-        const float *src = srcb + ((long long)(zoff[pz] + yoff[py]) << 2);
-        const unsigned mb = mbar0 + pstage * 8;
-        if (lane == 0) mbar_expect_tx(mb, (unsigned)RX * chunk_bytes);
-        __syncwarp();
-        for (int v = lane; v < RX; v += 32)
-          bulk_g2s(ring_s + (unsigned)(pstage * STRIDE + v * VOX) * 4u, src + (long long)v * C, chunk_bytes, mb);
-      } else {
-        const float *src = src0 + ((long long)(zoff[pz] + yoff[py]) << 2);
-        float *dst = dst0 + pstage * STRIDE;
-        if (piece_ok) {
+      const float *src = src0 + ((long long)(zoff[pz] + yoff[py]) << 2);
+      float *dst = dst0 + pstage * STRIDE;
+      if (piece_ok) {
 #pragma unroll 2
-          for (int v = cv_v; v < RX; v += VPI) {
-            cp_async16(dst, src);
-            dst += VPI * VOX, src += (long long)VPI * C;
-          }
+        for (int v = cv_v; v < RX; v += VPI) {
+          cp_async16(dst, src);
+          dst += VPI * VOX, src += (long long)VPI * C;
         }
-        cp_async_commit();
       }
+      cp_async_commit();
       if (++pz == nz) pz = 0, ++py;
       if (++pstage == NS) pstage = 0;
     };
 #pragma unroll
     for (int r = 0; r < NS - 1; ++r) {
       if (r < nrows) issue();
-      else if constexpr (!BULK) cp_async_commit();
+      else cp_async_commit();
     }
     int r = 0;
     for (int yi = 0; yi < ny; ++yi) {
@@ -868,47 +790,25 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
 #pragma unroll
         for (int c = 0; c < CV; ++c) t1[pw][c] = 0.0f;
       for (int zi = 0; zi < nz; ++zi, ++r) {
-        if constexpr (BULK) {
-          mbar_wait(mbar0 + cstage * 8, cpar);
-        } else {
-          cp_async_wait<NS - 2>();
-          __syncwarp();
-        }
-        const float wz = SDz[zlist[zi] * PP + it.pd];
+        cp_async_wait<NS - 2>();
+        __syncwarp();
+        const float wz = SDz[zlist[zi] * PP2 + it.pd];
         const float *row = ring + cstage * STRIDE;
-        if (++cstage == NS) cstage = 0, cpar ^= 1u;
+        if (++cstage == NS) cstage = 0;
         float tz[PW][CV];
 #pragma unroll
         for (int pw = 0; pw < PW; ++pw) {
           const float *q = row + soff[pw];
-          if constexpr (F2) {
-            // sm_100 packed fp32 (FFMA2 / FMUL2): both channels of the lane in one issue slot; each half is
-            // rounded exactly like the scalar fmul / fma, so the pinned arithmetic is unchanged
-            float2 z2;
-#pragma unroll
-            for (int j = 0; j < NXU; ++j) {
-              const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
-              const float2 w2 = make_float2(tw[pw][j], tw[pw][j]);
-              z2 = j == 0 ? __fmul2_rn(w2, t) : __ffma2_rn(w2, t, z2);
-            }
-            tz[pw][0] = z2.x, tz[pw][1] = z2.y;
-          } else {
+          // sm_100 packed fp32 (FFMA2 / FMUL2): both channels of the lane in one issue slot; each half is
+          // rounded exactly like the scalar fmul / fma, so the pinned arithmetic is unchanged
+          float2 z2;
 #pragma unroll
           for (int j = 0; j < NXU; ++j) {
-            float f[CV];
-            if constexpr (CV == 4) {
-              const float4 t = *reinterpret_cast<const float4 *>(q + j * VOX);
-              f[0] = t.x, f[1] = t.y, f[2] = t.z, f[3] = t.w;
-            } else if constexpr (CV == 2) {
-              const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
-              f[0] = t.x, f[1] = t.y;
-            } else {
-              f[0] = q[j * VOX];
-            }
-#pragma unroll
-            for (int c = 0; c < CV; ++c) tz[pw][c] = j == 0 ? tw[pw][0] * f[c] : fmaf(tw[pw][j], f[c], tz[pw][c]);
+            const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
+            const float2 w2 = make_float2(tw[pw][j], tw[pw][j]);
+            z2 = j == 0 ? __fmul2_rn(w2, t) : __ffma2_rn(w2, t, z2);
           }
-          }
+          tz[pw][0] = z2.x, tz[pw][1] = z2.y;
         }
         if (long_bins) {  // one warp-uniform test per row; bins wider than NXU taps are rare
 #pragma unroll
@@ -927,42 +827,32 @@ __global__ void __launch_bounds__(kWarps * 32, MINB)
         }
 #pragma unroll
         for (int pw = 0; pw < PW; ++pw) {
-          if constexpr (F2) {
-            const float2 o = __ffma2_rn(make_float2(wz, wz), make_float2(tz[pw][0], tz[pw][1]),
-                                        make_float2(t1[pw][0], t1[pw][1]));
-            t1[pw][0] = o.x, t1[pw][1] = o.y;
-          } else {
-#pragma unroll
-            for (int c = 0; c < CV; ++c) t1[pw][c] = fmaf(wz, tz[pw][c], t1[pw][c]);
-          }
+          const float2 o = __ffma2_rn(make_float2(wz, wz), make_float2(tz[pw][0], tz[pw][1]),
+                                      make_float2(t1[pw][0], t1[pw][1]));
+          t1[pw][0] = o.x, t1[pw][1] = o.y;
         }
         __syncwarp();
         if (r + NS - 1 < nrows) issue();
-        else if constexpr (!BULK) cp_async_commit();
+        else cp_async_commit();
       }
       // y-stage, once per feature row index y
       const int yy = ylist[yi];
       float wy[ROWS];
 #pragma unroll
-      for (int rr = 0; rr < ROWS; ++rr) wy[rr] = rr < it.rows ? SDy[yy * PP + it.ph0 + rr] : 0.0f;
+      for (int rr = 0; rr < ROWS; ++rr) wy[rr] = rr < it.rows ? SDy[yy * PP2 + it.ph0 + rr] : 0.0f;
 #pragma unroll
       for (int rr = 0; rr < ROWS; ++rr) {
         if (wy[rr] != 0.0f) {
 #pragma unroll
           for (int pw = 0; pw < PW; ++pw) {
-            if constexpr (F2) {
-              const float2 o = __ffma2_rn(make_float2(wy[rr], wy[rr]), make_float2(t1[pw][0], t1[pw][1]),
-                                          make_float2(acc[rr][pw][0], acc[rr][pw][1]));
-              acc[rr][pw][0] = o.x, acc[rr][pw][1] = o.y;
-            } else {
-#pragma unroll
-              for (int c = 0; c < CV; ++c) acc[rr][pw][c] = fmaf(wy[rr], t1[pw][c], acc[rr][pw][c]);
-            }
+            const float2 o = __ffma2_rn(make_float2(wy[rr], wy[rr]), make_float2(t1[pw][0], t1[pw][1]),
+                                        make_float2(acc[rr][pw][0], acc[rr][pw][1]));
+            acc[rr][pw][0] = o.x, acc[rr][pw][1] = o.y;
           }
         }
       }
     }
-    if constexpr (!BULK) cp_async_wait<0>();
+    cp_async_wait<0>();
   }
 
   // ---- epilogue: divide by the sample count, transpose through smem, stream out ----
@@ -993,9 +883,8 @@ __device__ __noinline__ void literal_tile_bwd(const Item &it, float *gb, int C, 
     }
 }
 
-template <int PW, int ROWS, int CV, int RXR, bool F2 = false>
+template <int PW, int ROWS, int CV, int RXR>
 __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const RoiParams p) {
-  static_assert(!F2 || CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
   using TB = Tables<PW>;
   constexpr int PWP = TB::PWP;
   constexpr int VOX = 32 * CV;
@@ -1142,16 +1031,9 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
     for (int r = 0; r < ROWS; ++r) {
       if (wy[r] != 0.0f) {
 #pragma unroll
-        for (int pw = 0; pw < PW; ++pw) {
-          if constexpr (F2) {  // FFMA2: both channels in one issue slot, each half rounded like fmaf
-            const float2 o = __ffma2_rn(make_float2(wy[r], wy[r]), make_float2(g[r][pw][0], g[r][pw][1]),
-                                        make_float2(u[pw][0], u[pw][1]));
-            u[pw][0] = o.x, u[pw][1] = o.y;
-          } else {
+        for (int pw = 0; pw < PW; ++pw)
 #pragma unroll
-            for (int c = 0; c < CV; ++c) u[pw][c] = fmaf(wy[r], g[r][pw][c], u[pw][c]);
-          }
-        }
+          for (int c = 0; c < CV; ++c) u[pw][c] = fmaf(wy[r], g[r][pw][c], u[pw][c]);
       }
     }
     // x-expansion, once per y: ux[xx] = sum_pw Dx[xx][pw] * u[pw]   (kept per lane in shared memory)
@@ -1167,15 +1049,9 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
 #pragma unroll
       for (int c = 0; c < CV; ++c) v[c] = 0.0f;
 #pragma unroll
-      for (int pw = 0; pw < PW; ++pw) {
-        if constexpr (F2) {
-          const float2 o = __ffma2_rn(make_float2(wx[pw], wx[pw]), make_float2(u[pw][0], u[pw][1]), make_float2(v[0], v[1]));
-          v[0] = o.x, v[1] = o.y;
-        } else {
+      for (int pw = 0; pw < PW; ++pw)
 #pragma unroll
-          for (int c = 0; c < CV; ++c) v[c] = fmaf(wx[pw], u[pw][c], v[c]);
-        }
-      }
+        for (int c = 0; c < CV; ++c) v[c] = fmaf(wx[pw], u[pw][c], v[c]);
 #pragma unroll
       for (int c = 0; c < CV; ++c) ux[xx * VOX + lane * CV + c] = v[c];
     }
@@ -1197,13 +1073,8 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
       for (int zi = 0; zi < 4; ++zi) {
         if (zi < nz) {
           float v[CV];
-          if constexpr (F2) {
-            const float2 o = __fmul2_rn(make_float2(zw[zi], zw[zi]), make_float2(uv[0], uv[1]));
-            v[0] = o.x, v[1] = o.y;
-          } else {
 #pragma unroll
-            for (int c = 0; c < CV; ++c) v[c] = zw[zi] * uv[c];
-          }
+          for (int c = 0; c < CV; ++c) v[c] = zw[zi] * uv[c];
           redv<CV>(q + zo[zi], v);
         }
       }
@@ -1226,21 +1097,21 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
 // scatter -- each expanded voxel value goes from registers straight into its (typically 2-3) vector reds,
 // two voxels per iteration for instruction-level parallelism, with no shared-memory round trip.
 // ---------------------------------------------------------------------------------------------
-template <int PW, int ROWS, int CV, bool F2, int MINB, int PP>
+template <int PW, int ROWS, int CV, int MINB>
 __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(const RoiParams p) {
-  static_assert(!F2 || CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
+  static_assert(CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
   using TB = Tables<PW>;
   constexpr int PWP = TB::PWP;
   constexpr int STAGE = CV * ROWS * PW * 33;     // all CV slots of the grad tile at once
   constexpr int LISTS = 80;
   constexpr int WARP_FLOATS = (LISTS / 4 + STAGE + 3) / 4 * 4;
-  constexpr int SH_FLOATS = (RXMAX + 1) * PWP + RYMAX * PP + RZMAX2 * PP + RXMAX + 8;
+  constexpr int SH_FLOATS = (RXMAX + 1) * PWP + RYMAX * PP2 + RZMAX2 * PP2 + RXMAX + 8;
   extern __shared__ __align__(16) float smem_all[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
   float *SDx = smem_all;                         // [x - xmin][PWP] (+1 row: the paired x loop may read one past RX)
-  float *SDy = SDx + (RXMAX + 1) * PWP;          // [y - ymin][PP]
-  float *SDz = SDy + RYMAX * PP;                 // [z - zmin][PP]
-  int *Sxany = reinterpret_cast<int *>(SDz + RZMAX2 * PP);
+  float *SDy = SDx + (RXMAX + 1) * PWP;          // [y - ymin][PP2]
+  float *SDz = SDy + RYMAX * PP2;                // [z - zmin][PP2]
+  int *Sxany = reinterpret_cast<int *>(SDz + RZMAX2 * PP2);
   int *Sbox = Sxany + RXMAX;
   float *sm = smem_all + ((SH_FLOATS + 3) / 4 * 4) + warp * WARP_FLOATS;
 
@@ -1367,14 +1238,14 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
   const int RX = xmax - xmin + 1, RY = ymax - ymin + 1, RZ = zmax - zmin + 1;
   if (!empty && fits) {
     for (int i = tid; i < (RX + 1) * PWP; i += kWarps * 32) SDx[i] = 0.0f;
-    for (int i = tid; i < RY * PP; i += kWarps * 32) SDy[i] = 0.0f;
-    for (int i = tid; i < RZ * PP; i += kWarps * 32) SDz[i] = 0.0f;
+    for (int i = tid; i < RY * PP2; i += kWarps * 32) SDy[i] = 0.0f;
+    for (int i = tid; i < RZ * PP2; i += kWarps * 32) SDz[i] = 0.0f;
     for (int i = tid; i < RX; i += kWarps * 32) Sxany[i] = 0;
   }
   __syncthreads();
   if (!empty && fits && role >= 0) {
     float *tab = role == 0 ? SDx : role == 1 ? SDy : SDz;
-    const int stride = role == 0 ? PWP : PP;
+    const int stride = role == 0 ? PWP : PP2;
     const int mn = role == 0 ? xmin : role == 1 ? ymin : zmin;
     for (int i = 0; i < ax.S; ++i) {
       Tap t = axis_tap(axis_coord(ax, lane, i), asize);
@@ -1412,7 +1283,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
     bool a = false;
     if (yy < RY) {
 #pragma unroll
-      for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP + it.ph0 + r] != 0.0f;
+      for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP2 + it.ph0 + r] != 0.0f;
     }
     const unsigned bal = __ballot_sync(FULL, a);
     if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
@@ -1420,7 +1291,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
   }
   for (int z0 = 0; z0 < RZ; z0 += 32) {
     const int zz = z0 + lane;
-    const bool a = zz < RZ && SDz[zz * PP + it.pd] != 0.0f;
+    const bool a = zz < RZ && SDz[zz * PP2 + it.pd] != 0.0f;
     const unsigned bal = __ballot_sync(FULL, a);
     if (a) zlist[nz + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)zz;
     nz += __popc(bal);
@@ -1437,7 +1308,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
 #pragma unroll
   for (int zi = 0; zi < 4; ++zi) {
     const int zrel = zi < nz ? zlist[zi] : 0;
-    zw[zi] = zi < nz ? SDz[zrel * PP + it.pd] : 0.0f;
+    zw[zi] = zi < nz ? SDz[zrel * PP2 + it.pd] : 0.0f;
     zo[zi] = (long long)zrel * slice_elems;
   }
   for (int yi = 0; yi < ny; ++yi) {
@@ -1450,18 +1321,13 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
       for (int c = 0; c < CV; ++c) u[pw][c] = 0.0f;
 #pragma unroll
     for (int r = 0; r < ROWS; ++r) {
-      const float wy = r < it.rows ? SDy[yy * PP + it.ph0 + r] : 0.0f;
+      const float wy = r < it.rows ? SDy[yy * PP2 + it.ph0 + r] : 0.0f;
       if (wy != 0.0f) {
 #pragma unroll
         for (int pw = 0; pw < PW; ++pw) {
-          if constexpr (F2) {
-            const float2 o = __ffma2_rn(make_float2(wy, wy), make_float2(g[r][pw][0], g[r][pw][1]),
-                                        make_float2(u[pw][0], u[pw][1]));
-            u[pw][0] = o.x, u[pw][1] = o.y;
-          } else {
-#pragma unroll
-            for (int c = 0; c < CV; ++c) u[pw][c] = fmaf(wy, g[r][pw][c], u[pw][c]);
-          }
+          const float2 o = __ffma2_rn(make_float2(wy, wy), make_float2(g[r][pw][0], g[r][pw][1]),
+                                      make_float2(u[pw][0], u[pw][1]));
+          u[pw][0] = o.x, u[pw][1] = o.y;
         }
       }
     }
@@ -1487,14 +1353,9 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
       for (int pw = 0; pw < PW; ++pw)
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
-          if constexpr (F2) {
-            const float2 o = __ffma2_rn(make_float2(wx[h][pw], wx[h][pw]), make_float2(u[pw][0], u[pw][1]),
-                                        make_float2(v[h][0], v[h][1]));
-            v[h][0] = o.x, v[h][1] = o.y;
-          } else {
-#pragma unroll
-            for (int c = 0; c < CV; ++c) v[h][c] = fmaf(wx[h][pw], u[pw][c], v[h][c]);
-          }
+          const float2 o = __ffma2_rn(make_float2(wx[h][pw], wx[h][pw]), make_float2(u[pw][0], u[pw][1]),
+                                      make_float2(v[h][0], v[h][1]));
+          v[h][0] = o.x, v[h][1] = o.y;
         }
       // all products and addresses first, then the reds back to back: distinct registers per red, so a red still
       // waiting in the memory pipeline does not stall the next one on a register it has yet to read
@@ -1505,13 +1366,8 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
 #pragma unroll
         for (int zi = 0; zi < 4; ++zi) {
           ad[h][zi] = q + h * (long long)C + zo[zi];
-          if constexpr (F2) {
-            const float2 t = __fmul2_rn(make_float2(zw[zi], zw[zi]), make_float2(v[h][0], v[h][1]));
-            o[h][zi][0] = t.x, o[h][zi][1] = t.y;
-          } else {
-#pragma unroll
-            for (int c = 0; c < CV; ++c) o[h][zi][c] = zw[zi] * v[h][c];
-          }
+          const float2 t = __fmul2_rn(make_float2(zw[zi], zw[zi]), make_float2(v[h][0], v[h][1]));
+          o[h][zi][0] = t.x, o[h][zi][1] = t.y;
         }
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
@@ -1521,7 +1377,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
           if (zi < nz) redv<CV>(ad[h][zi], o[h][zi]);
         for (int zi = 4; zi < nz; ++zi) {
           const int zrel = zlist[zi];
-          const float wz = SDz[zrel * PP + it.pd];
+          const float wz = SDz[zrel * PP2 + it.pd];
           float t[CV];
 #pragma unroll
           for (int c = 0; c < CV; ++c) t[c] = wz * v[h][c];
@@ -1713,10 +1569,7 @@ static int transpose_launch(const float *src, float *dst, int B, int rows, int c
 // Dispatch
 // ---------------------------------------------------------------------------------------------
 static int g_fwd_variant = 0;  // 0 = auto; see roi3d_set_tuning
-static int g_fwd_items_per_warp = 0;  // 0 = auto
 extern int g_host_pipeline_kb;        // host_api.cu
-extern int g_fwd_stream_cfg, g_fwd_stream_debug;  // roi_align3d_stream.cu  // roi_align3d_stream.cu
-extern int g_nms_mask_variant;        // nms3d.cu
 extern int g_planar_smem_floats;      // roi_align3d_planar.cu
 extern int g_topk_sieve;              // proposal.cu
 extern thread_local cudaEvent_t g_timing_ev[2];  // roi_align3d_stream.cu
@@ -1761,28 +1614,26 @@ static int launch_fwd_ring(RoiParams &p, cudaStream_t st) {
   return ROI3D_OK;
 }
 
-template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB = 0, int BULK = 0, bool F2 = false, bool MULTI = false, int ITEMS = 1>
+template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB = 0, bool MULTI = false, int ITEMS = 1>
 static int launch_fwd_ring2(RoiParams &p, cudaStream_t st) {
-  using LY = Ring2Layout<PW, ROWS, CV, NS, RXR, BULK>;
+  using LY = Ring2Layout<PW, ROWS, CV, NS, RXR>;
   const size_t smem = LY::BYTES;
   p.nchunk = ceil_div(p.C, 32 * CV);
   p.nphg = ceil_div(p.PH, ROWS);
   p.items_per_roi = p.nchunk * p.PD * p.nphg;
-  p.items_per_warp = !MULTI ? 1 : g_fwd_items_per_warp > 0 ? g_fwd_items_per_warp : ITEMS;
+  p.items_per_warp = MULTI ? ITEMS : 1;
   p.ctas_per_roi = ceil_div(p.items_per_roi, kWarps * p.items_per_warp);
   p.total_items = (long long)p.K * p.items_per_roi;
   const long long blocks = (long long)p.K * p.ctas_per_roi;
   ROI3D_CHECK_ARG(blocks < 2147483647LL, "roi_align3d forward: too many work items");
-  static_assert(BULK == 0, "the bulk-copy / TMA row rings were measured slower and are not instantiated");
-  static TmapSet tm;  // kernel argument of the (uninstantiated) TMA row ring
-  auto kern = roi_align3d_fwd_ring2_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB, BULK, F2, MULTI>;
+  auto kern = roi_align3d_fwd_ring2_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB, MULTI>;
   ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p, tm);
+  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
   ROI3D_LAUNCH_CHECK();
   return ROI3D_OK;
 }
 
-template <int PW, int ROWS, int CV, int RXR, bool F2 = false>
+template <int PW, int ROWS, int CV, int RXR>
 static int launch_bwd(RoiParams &p, cudaStream_t st) {
   using TB = Tables<PW>;
   constexpr int VOX = 32 * CV;
@@ -1793,7 +1644,7 @@ static int launch_bwd(RoiParams &p, cudaStream_t st) {
   p.nchunk = ceil_div(p.C, 32 * CV);
   p.nphg = ceil_div(p.PH, ROWS);
   p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
-  auto kern = roi_align3d_bwd_cl_kernel<PW, ROWS, CV, RXR, F2>;
+  auto kern = roi_align3d_bwd_cl_kernel<PW, ROWS, CV, RXR>;
   ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long blocks = ceil_div_ll(p.total_items, kWarps);
   ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "roi_align3d backward: too many work items");
@@ -1802,13 +1653,13 @@ static int launch_bwd(RoiParams &p, cudaStream_t st) {
   return ROI3D_OK;
 }
 
-template <int PW, int ROWS, int CV, bool F2 = false, int MINB = 0, int PP = 16>
+template <int PW, int ROWS, int CV, int MINB = 0>
 static int launch_bwd2(RoiParams &p, cudaStream_t st) {
-  ROI3D_CHECK_ARG(p.PH <= PP && p.PD <= PP, "roi_align3d backward: table rows narrower than PH / PD");
+  ROI3D_CHECK_ARG(p.PH <= PP2 && p.PD <= PP2, "roi_align3d backward: table rows narrower than PH / PD");
   using TB = Tables<PW>;
   constexpr int STAGE = CV * ROWS * PW * 33;
   constexpr int WARP_FLOATS = (80 / 4 + STAGE + 3) / 4 * 4;
-  constexpr int SH_FLOATS = (RXMAX + 1) * TB::PWP + RYMAX * PP + RZMAX2 * PP + RXMAX + 8;
+  constexpr int SH_FLOATS = (RXMAX + 1) * TB::PWP + RYMAX * PP2 + RZMAX2 * PP2 + RXMAX + 8;
   const size_t smem = ((size_t)((SH_FLOATS + 3) / 4 * 4) + (size_t)kWarps * WARP_FLOATS) * sizeof(float);
   p.nchunk = ceil_div(p.C, 32 * CV);
   p.nphg = ceil_div(p.PH, ROWS);
@@ -1817,7 +1668,7 @@ static int launch_bwd2(RoiParams &p, cudaStream_t st) {
   p.total_items = (long long)p.K * p.items_per_roi;
   const long long blocks = (long long)p.K * p.ctas_per_roi;
   ROI3D_CHECK_ARG(blocks < 2147483647LL, "roi_align3d backward: too many work items");
-  auto kern = roi_align3d_bwd2_kernel<PW, ROWS, CV, F2, MINB, PP>;
+  auto kern = roi_align3d_bwd2_kernel<PW, ROWS, CV, MINB>;
   ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
   ROI3D_LAUNCH_CHECK();
@@ -1850,8 +1701,8 @@ static int pick_cv(const RoiParams &p, bool bwd) {
   return cv;
 }
 
-// Forward kernel selection.  g_fwd_variant (roi3d_set_tuning key 0): 0 = auto, 1 = one channel per lane (the
-// fallback for C % 2 != 0), 50 = the per-warp ring kernel even where the streamed kernel applies (A/B), 99 = literal.
+// Forward kernel selection.  g_fwd_variant (roi3d_set_tuning key 0): 0 = auto, 50 = the per-warp ring kernel even
+// where the streamed kernel applies (A/B), 60 = the planar kernel on channels-last 7-wide outputs, 99 = literal.
 static int dispatch_fwd(RoiParams &p, cudaStream_t st) {
   if (p.K == 0) return ROI3D_OK;
   const int cvmax = pick_cv(p, false);
@@ -1872,46 +1723,43 @@ static int dispatch_fwd(RoiParams &p, cudaStream_t st) {
   bool ring_ok = p.C % 4 == 0;
   for (int l = 0; l < p.num_levels; ++l) ring_ok = ring_ok && aligned(p.lv[l].feats, 16);
   if (p.PW == 7) {
-    if (ring_ok && cvmax >= 2 && v != 1) {
-      if (p.PH <= 16 && p.PD <= 16) return launch_fwd_ring2<7, 7, 2, 3, 5, 18, 2, 0, true>(p, st);
+    if (ring_ok && cvmax >= 2) {
+      if (p.PH <= 16 && p.PD <= 16) return launch_fwd_ring2<7, 7, 2, 3, 5, 18, 2>(p, st);
       return launch_fwd_ring<7, 7, 2, 3, 4, 18, 2>(p, st);  // per-warp tables (PH or PD > 16)
     }
-    if (v == 1 || cvmax == 1) return launch_fwd<7, 7, 1, 3>(p, st);
+    if (cvmax == 1) return launch_fwd<7, 7, 1, 3>(p, st);
     return launch_fwd<7, 7, 2, 3>(p, st);
   }
   if (p.PW == 14) {
-    if (ring_ok && cvmax >= 2 && v != 1) {
-      if (p.PH <= 16 && p.PD <= 16) return launch_fwd_ring2<14, 4, 2, 3, 3, 18, 0, 0, true, true, 7>(p, st);
+    if (ring_ok && cvmax >= 2) {
+      if (p.PH <= 16 && p.PD <= 16) return launch_fwd_ring2<14, 4, 2, 3, 3, 18, 0, true, 7>(p, st);
       return launch_fwd_ring<14, 4, 2, 3, 3, 18>(p, st);  // per-warp tables (PH or PD > 16)
     }
-    if (v == 1 || cvmax == 1) return launch_fwd<14, 7, 1, 3>(p, st);
+    if (cvmax == 1) return launch_fwd<14, 7, 1, 3>(p, st);
     return launch_fwd<14, 4, 2, 3>(p, st);
   }
   if (cvmax >= 2) return launch_generic<2>(p, true, st);
   return launch_generic<1>(p, true, st);
 }
 
-// Backward kernel selection.  g_bwd_variant (key 1): 0 = auto, 1 = one channel per lane, 3 = per-warp tables, 99 = literal.
+// Backward kernel selection.  g_bwd_variant (key 1): 0 = auto, 50 = the CTA-shared-table kernel even where the
+// streamed or planar kernel applies (A/B), 60 = the planar backward on 7-wide outputs.
 static int dispatch_bwd(RoiParams &p, cudaStream_t st) {
   if (p.K == 0) return ROI3D_OK;
   const int cvmax = pick_cv(p, true);
   const int v = g_bwd_variant;
-  if (v == 99) {
-    if (cvmax >= 2) return launch_generic<2>(p, false, st);
-    return launch_generic<1>(p, false, st);
-  }
   if (p.PW == 7) {
     if (v == 60 && bwd_planar_ok(p)) return launch_bwd_planar(p, st);   // (A/B: the planar backward on 7-wide outputs)
     if (v == 0 && bwd_stream_ok(p)) return launch_bwd_stream(p, st);    // one red per voxel (roi_align3d_stream.cu)
-    if (v == 1 || cvmax == 1) return launch_bwd<7, 7, 1, 40>(p, st);
-    if ((v == 0 || v == 50) && p.PH <= 16 && p.PD <= 16 && cvmax >= 2) return launch_bwd2<7, 7, 2, true>(p, st);
-    return launch_bwd<7, 7, 2, 26>(p, st);  // per-warp tables (v == 3, or PH / PD > 16)
+    if (cvmax == 1) return launch_bwd<7, 7, 1, 40>(p, st);
+    if ((v == 0 || v == 50) && p.PH <= 16 && p.PD <= 16) return launch_bwd2<7, 7, 2>(p, st);
+    return launch_bwd<7, 7, 2, 26>(p, st);  // per-warp tables (PH / PD > 16, or v == 60 where the planar kernel does not apply)
   }
   if (p.PW == 14) {
     if ((v == 0 || v == 60) && bwd_planar_ok(p)) return launch_bwd_planar(p, st);   // transposed planar stages (roi_align3d_planar.cu)
-    if (v == 1 || cvmax == 1) return launch_bwd<14, 7, 1, 40>(p, st);
-    if ((v == 0 || v == 50) && p.PH <= 16 && p.PD <= 16 && cvmax >= 2) return launch_bwd2<14, 2, 2, true, 4>(p, st);  // 2 ph rows per warp
-    return launch_bwd<14, 4, 2, 30>(p, st);  // per-warp tables (v == 3, or PH / PD > 16)
+    if (cvmax == 1) return launch_bwd<14, 7, 1, 40>(p, st);
+    if ((v == 0 || v == 50) && p.PH <= 16 && p.PD <= 16) return launch_bwd2<14, 2, 2, 4>(p, st);  // 2 ph rows per warp
+    return launch_bwd<14, 4, 2, 30>(p, st);  // per-warp tables (PH / PD > 16, or v == 60 where the planar kernel does not apply)
   }
   if (cvmax >= 2) return launch_generic<2>(p, false, st);
   return launch_generic<1>(p, false, st);
@@ -1961,16 +1809,18 @@ int roi3d_set_kernel_timing_events(void *start_event, void *stop_event) {
 }
 
 int roi3d_set_tuning(int key, int value) {
+  const bool ok = key == 0    ? value == 0 || value == 50 || value == 60 || value == 99
+                  : key == 1  ? value == 0 || value == 50 || value == 60
+                  : key == 4  ? value >= -1
+                  : key == 10 ? value >= 0
+                  : key == 11 ? value == -1 || value == 0 || value == 2
+                              : false;
+  ROI3D_CHECK_ARG(ok, "roi3d_set_tuning: unsupported key %d / value %d", key, value);
   if (key == 0) g_fwd_variant = value;
   else if (key == 1) g_bwd_variant = value;
-  else if (key == 2) g_fwd_items_per_warp = value;
   else if (key == 4) g_host_pipeline_kb = value;
-  else if (key == 6) g_nms_mask_variant = value;
-  else if (key == 7) g_fwd_stream_cfg = value;
-  else if (key == 9) g_fwd_stream_debug = value;
   else if (key == 10) g_planar_smem_floats = value;
-  else if (key == 11) g_topk_sieve = value;
-  else return ROI3D_EINVAL;
+  else g_topk_sieve = value;
   return ROI3D_OK;
 }
 

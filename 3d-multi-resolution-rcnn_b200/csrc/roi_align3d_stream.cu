@@ -108,7 +108,6 @@ struct StreamArgs {
   const CUtensorMap *maps[ST_MAX_LEVELS];  // [xcls][ycls] per level, device memory
   int total_items;
   int pdhw;           // PD * 49
-  int debug;          // developer experiments: bit 0 = owners skip the arithmetic, bit 1 = no output store
 };
 
 // shared-memory carve-up (bytes from the base) for a ring of NS slots of SLOT bytes
@@ -524,7 +523,7 @@ __device__ __forceinline__ void owner_loop(const StreamArgs &a, unsigned char *s
       }
       TileDesc dt = d;
       for (;;) {  // tiles of the item
-        if (dt.nrows > 0 && !(a.debug & 1)) {
+        if (dt.nrows > 0) {
           const float *tile = reinterpret_cast<const float *>(smem + L::RING + slot * SLOT) + (NC ? lane * SN_S + first : lane * 2) + xo;
           if (!NC && (pflags & PLAN_X3))
             owner_tile<3, NPH, NC>(dt.nrows, dt.z, dt.y, dt.rowfloats, P, tile, ph0, RY, ylo, yhi1, xw, t2, acc, rot);
@@ -704,7 +703,7 @@ __device__ __forceinline__ void storer_loop(const StreamArgs &a, unsigned char *
     const int *sd = reinterpret_cast<const int *>(smem + L::SDESC + (n & 1) * 16);
     if (sd[2]) break;
     float *dst = a.p.out + ((long long)sd[0] * a.p.C + (long long)sd[1] * ST_CH) * a.pdhw;
-    if (!(a.debug & 2)) st_bulk_s2g(dst, stage_s, bytes);
+    st_bulk_s2g(dst, stage_s, bytes);
     asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
     asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");
     st_mbar_arrive(sfree);
@@ -1241,9 +1240,9 @@ int launch_cfg(const RoiParams &p, StreamArgs &a, cudaStream_t st, int sm_count)
   if (rc) return rc;
   StreamPlan *plans = reinterpret_cast<StreamPlan *>(ws);
   int *counter = reinterpret_cast<int *>(ws + plan_bytes);
-  const int sort = (p.K <= ST_SORT_MAX && !(a.debug & 4)) ? 1 : 0;
+  const int sort = p.K <= ST_SORT_MAX ? 1 : 0;
   const int grid = a.total_items < sm_count ? a.total_items : sm_count;
-  roi_align3d_plan_kernel<<<ceil_div(p.K, 8), 256, sort ? p.K * sizeof(float) : 0, st>>>(p, plans, counter, NC && sort && !(a.debug & 16) ? 2 : sort, SLOT, NC ? 2 * grid : 3 * grid, NC ? 1 : 0);
+  roi_align3d_plan_kernel<<<ceil_div(p.K, 8), 256, sort ? p.K * sizeof(float) : 0, st>>>(p, plans, counter, NC && sort ? 2 : sort, SLOT, NC ? 2 * grid : 3 * grid, NC ? 1 : 0);
   ROI3D_LAUNCH_CHECK();
   a.plans = plans, a.counter = counter;
   static PerDeviceSmemOptIn opt_in;   // (one per instantiation = per kernel)
@@ -1273,9 +1272,6 @@ int launch_cfg(const RoiParams &p, StreamArgs &a, cudaStream_t st, int sm_count)
 // streamed forward kernel, so that a benchmark can time the dominant kernel by itself (without the plan kernel).
 thread_local cudaEvent_t g_timing_ev[2] = {nullptr, nullptr};
 
-int g_fwd_stream_cfg = 0;       // roi3d_set_tuning key 7: ring geometry of the streamed kernel (0 = default)
-int g_fwd_stream_debug = 0;     // key 9: developer experiments (bit 0: owners skip the arithmetic, bit 1: no output store, bit 2: no sort, bit 4: NCDHW twin in largest-first order)
-
 int launch_fwd_stream(RoiParams &p, cudaStream_t st) {
   int sm_count = 0;
   {
@@ -1287,7 +1283,6 @@ int launch_fwd_stream(RoiParams &p, cudaStream_t st) {
   for (int l = 0; l < ST_MAX_LEVELS; ++l) a.maps[l] = nullptr;
   a.total_items = p.K * (p.C / ST_CH);
   a.pdhw = p.PD * 49;
-  a.debug = g_fwd_stream_debug;
   if (p.layout == ROI3D_NCDHW) {   // cp.async producers, no tensor maps
     return launch_cfg<3, SN_SLOT, true>(p, a, st, sm_count);
   }
@@ -1297,11 +1292,7 @@ int launch_fwd_stream(RoiParams &p, cudaStream_t st) {
   }
   // ring geometry (measured on C2, whole call): 3 x 42 KB 154 us, 4 x 32 KB 156 us, 4 x 30 KB 160 us, 5 x 24 KB 166 us,
   // 4 x 20 KB 185 us, 8 x 15 KB 215 us -- per-tile hand-offs cost more than a shallower ring
-  switch (g_fwd_stream_cfg) {
-    case 1: return launch_cfg<4, 32768>(p, a, st, sm_count);
-    case 2: return launch_cfg<5, 24576>(p, a, st, sm_count);
-    default: return launch_cfg<3, 43008>(p, a, st, sm_count);
-  }
+  return launch_cfg<3, 43008>(p, a, st, sm_count);
 }
 
 bool bwd_stream_ok(const RoiParams &p) {
@@ -1324,7 +1315,6 @@ int launch_bwd_stream(RoiParams &p, cudaStream_t st) {
   for (int l = 0; l < ST_MAX_LEVELS; ++l) a.maps[l] = nullptr;
   a.total_items = p.K * (p.C / ST_CH);
   a.pdhw = p.PD * 49;
-  a.debug = 0;
   const size_t plan_bytes = (size_t)p.K * sizeof(StreamPlan);
   unsigned char *ws = nullptr;
   bool pooled = false;

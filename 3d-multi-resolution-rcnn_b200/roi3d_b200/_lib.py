@@ -114,7 +114,7 @@ def _load():
 lib, EXPORTS = _load()
 
 # developer knob: pick a kernel variant for the whole process (see roi3d_set_tuning in the header)
-for _key, _env in ((0, "ROI3D_FWD_VARIANT"), (1, "ROI3D_BWD_VARIANT"), (2, "ROI3D_FWD_ITEMS")):
+for _key, _env in ((0, "ROI3D_FWD_VARIANT"), (1, "ROI3D_BWD_VARIANT")):
     if os.environ.get(_env):
         lib.roi3d_set_tuning(_key, int(os.environ[_env]))
 

@@ -266,16 +266,16 @@ int roi3d_mask_target(const uint8_t *gt_masks_dev, int G, int D, int H, int W, c
                       const int64_t *gt_inds_host, int n, int Md, int Mh, int Mw, float *out_dev, void *workspace_dev,
                       size_t workspace_bytes, void *stream);
 
-/* Experiment knob (not part of the reference surface): key 0 = forward kernel variant (0 = auto, 1 = one channel per
- * lane, 50 = per-warp ring kernel where the streamed kernel would apply, 60 = planar kernel on channels-last 7-wide
- * outputs, 99 = literal reference-order path); key 1 = backward kernel variant (0 = auto: streamed / planar where they
- * apply, 50 = per-warp kernel, 60 = planar backward on 7-wide outputs, 1, 3 = per-warp tables, 99 = literal); key 2 =
- * sub-items one ring-kernel warp walks per RoI (0 = auto); key 4 = volume size in KB from which
- * roi3d_roi_align3d_forward_host pipelines its copies (0 = auto, 32 MB; -1 = never); key 6 = NMS mask kernel variant;
- * key 7 = ring geometry of the streamed forward kernel (0 = 3 x 42 KB, 1 = 4 x 32 KB, 2 = 5 x 24 KB); key 9 = streamed
- * kernel experiments (bit 0: no arithmetic, bit 1: no output store, bit 2: no largest-first order); key 10 = plane
- * storage of the planar kernels per CTA in floats (0 = 18432); key 11 = top-k sieve path (0 = on where it applies,
- * -1 = digit passes only, 2 = the sieve gives up on every segment so that its fallback runs -- tests). */
+/* Developer knob (not part of the reference surface).  Accepted key / value pairs, anything else returns ROI3D_EINVAL:
+ *   key 0 = forward kernel: 0 = auto, 50 = per-warp ring kernel where the streamed kernel would apply, 60 = planar
+ *           kernel on channels-last 7-wide outputs, 99 = literal reference-order path;
+ *   key 1 = backward kernel: 0 = auto (streamed / planar where they apply), 50 = per-warp kernel, 60 = planar backward
+ *           on 7-wide outputs;
+ *   key 4 = volume size in KB from which roi3d_roi_align3d_forward_host pipelines its copies (0 = auto, 32 MB;
+ *           -1 = never; any value >= -1);
+ *   key 10 = plane storage of the planar kernels per CTA in floats (0 = 18432; any value >= 0);
+ *   key 11 = top-k sieve path: 0 = on where it applies, -1 = digit passes only, 2 = the sieve gives up on every
+ *           segment so that its fallback runs (tests). */
 int roi3d_set_tuning(int key, int value);
 
 /* Measurement hook (not part of the reference surface): two cudaEvent_t (as void*) that the calling thread's next

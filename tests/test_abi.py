@@ -100,3 +100,24 @@ def test_argument_errors_are_codes_with_messages_not_prints_or_exits():
     assert lib.roi3d_nms3d_batched(None, None, 0, 0, 0.5, None, None, None, None, 0, None) == 0
     n = ctypes.c_int32(7)
     assert lib.roi3d_nms3d_host(None, 0, 0.5, None, ctypes.addressof(n)) == 0 and n.value == 0
+
+
+def test_set_tuning_accepts_exactly_the_documented_pairs():
+    """roi3d_set_tuning takes the key / value pairs its header comment lists and refuses every other one with a message
+    naming both, so that a call for a removed or misspelt variant cannot silently run the default kernels."""
+    from roi3d_b200 import _lib
+    lib = _lib.lib
+    accepted = [(0, 0), (0, 50), (0, 60), (0, 99), (1, 0), (1, 50), (1, 60), (4, -1), (4, 0), (4, 1024),
+                (10, 0), (10, 5000), (11, -1), (11, 0), (11, 2)]
+    rejected = [(2, 0), (2, 7), (6, 0), (6, 1), (7, 0), (7, 1), (9, 0), (9, 2), (0, 1), (0, 40), (1, 1), (1, 3),
+                (1, 99), (4, -2), (10, -1), (11, 1), (11, 5), (77, 0)]
+    try:
+        for key, value in accepted:
+            assert lib.roi3d_set_tuning(key, value) == 0, (key, value)
+        for key, value in rejected:
+            assert lib.roi3d_set_tuning(key, value) == -1, (key, value)
+            msg = lib.roi3d_last_error().decode()
+            assert "key %d" % key in msg and "value %d" % value in msg, msg
+    finally:
+        for key in (0, 1, 4, 10, 11):
+            assert lib.roi3d_set_tuning(key, 0) == 0

@@ -1,4 +1,6 @@
-"""Run one hot-path op a few times (for ncu).  usage: prof_one.py {c2fwd|c2bwd|c3fwd|c3bwd|nms|topk} [variant]"""
+"""Run one hot-path op a few times (for ncu).  usage: prof_one.py {c2fwd|c2bwd|c3fwd|c3bwd|nms|topk} [variant]
+
+variant (roi3d_set_tuning key 0 / 1): forward 0 = auto, 50, 60 or 99; backward 0 = auto, 50 or 60."""
 import os
 import sys
 
