@@ -74,6 +74,8 @@ typedef struct roi3d_level {
  *   mmdet/ops/roi_align/src/roi_align_cuda.cpp:68-94, roi_align_kernel.cu:316-337 (kernel :214-291).
  * out_dev: [K, C, PD, PH, PW] contiguous, fully overwritten (no pre-zeroing needed, unlike
  *   functions/roi_align_3d.py:32).  feats: [B,C,D,H,W] in `layout` (ROI3D_NDHWC or ROI3D_NCDHW, see above).
+ * A RoI whose (int)batch_idx lies outside [0, B) reads no feature voxel: its output row is 0 (NaN where its sample
+ *   count is 0, as for any RoI).
  * ---------------------------------------------------------------------------------------------- */
 int roi3d_roi_align3d_forward(const float *feats_dev, int layout, int B, int C, int D, int H, int W,
                               const float *rois_dev, int K, int PD, int PH, int PW, float spatial_scale,
@@ -95,6 +97,7 @@ int roi3d_roi_align3d_forward_rows(const float *feats_dev, int layout, int B, in
  *   functions/roi_align_3d.py:84 does); pass zero_fill=1 to have the library clear it first.
  * bug_compat=1 reproduces the reference's top_diff index for non-cubic outputs
  *   (roi_align_kernel.cu:554-555; SURVEY F2); default 0 = the mathematically correct gradient.
+ * A RoI whose (int)batch_idx lies outside [0, B) adds nothing to grad_in_dev.
  * ---------------------------------------------------------------------------------------------- */
 int roi3d_roi_align3d_backward(const float *grad_out_dev, const float *rois_dev, int K, int PD, int PH, int PW,
                                float spatial_scale, float spatial_scale_depth, int sample_num,

@@ -138,11 +138,13 @@ def argsort_desc_stable(scores):
 
 def roi_align3d_forward(feats, rois, out_size, out_size_depth, spatial_scale, spatial_scale_depth,
                         sample_num=0, contract=True):
-    """ROIAlignForward3D (roi_align_kernel.cu:214-291).  feats [B,C,D,H,W] (NCDHW), rois [K,7]."""
+    """ROIAlignForward3D (roi_align_kernel.cu:214-291).  feats [B,C,D,H,W] (NCDHW), rois [K,7]; out_size is an int
+    (square bins) or a (PH, PW) pair."""
     feats, rois = _f32(feats), _f32(rois).reshape(-1, 7)
     B, C, D, H, W = feats.shape
     K = rois.shape[0]
-    PD, PH, PW = int(out_size_depth), int(out_size), int(out_size)
+    PH, PW = (out_size, out_size) if np.ndim(out_size) == 0 else out_size
+    PD, PH, PW = int(out_size_depth), int(PH), int(PW)
     out = np.empty((K, C, PD, PH, PW), dtype=np.float32)
     if K:
         lib().oracle_roi_align3d_forward(_p(feats), B, C, D, H, W, _p(rois), K, PD, PH, PW,

@@ -1541,10 +1541,15 @@ PLANAR_CASES = [
 ]
 
 
+# Channels-last levels reach the planar kernel only with C % 4 == 0 (16-byte copies of four channels of a voxel); the
+# odd-channel case runs channels-last in test_roi_align_kernel_coverage.py under the kernel that takes it.
+PLANAR_RUNS = [pytest.param(case, layout, smem_floats, id="%d-%s-case%d" % (smem_floats, layout, i))
+               for smem_floats in (0, 5000) for layout in ("NCDHW", "NDHWC") for i, case in enumerate(PLANAR_CASES)
+               if layout == "NCDHW" or case[0][1] % 4 == 0]
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("case", PLANAR_CASES)
-@pytest.mark.parametrize("layout", ["NCDHW", "NDHWC"])
-@pytest.mark.parametrize("smem_floats", [0, 5000])
+@pytest.mark.parametrize("case,layout,smem_floats", PLANAR_RUNS)
 def test_roi_align_forward_planar_kernel(oracle, dev, case, layout, smem_floats):
     """The planar kernel: the reference's NCDHW layout read natively (no conversion), and channels-last through the
     same kernel (tuning variant 60); 7- and 14-wide outputs, ragged channel groups, adversarial and over-wide RoIs.
