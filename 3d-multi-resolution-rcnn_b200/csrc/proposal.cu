@@ -58,10 +58,12 @@ struct SegState {           // device, per segment
   int k_rem;                // how many keys still to take inside the current prefix
   int k_take;               // min(k, len)
   int cand_count;
-  int bnd_count;            // keys inside the boundary bin after the second digit pass (topk_split_kernel)
+  int bnd_count;            // keys inside the boundary bin after the second digit pass (topk_split_kernel); read as
+                            // unsigned: a segment of more than 2^31 elements can put more than INT_MAX keys there
   unsigned eff_len;         // elements taking part: len, or the number of set mask bytes (known after digit pass 0)
   float sieve_t;            // sieve path: raw-score threshold picked from a sample of the segment (topk_sample_kernel)
-  int sieve_count;          // sieve path: elements with a raw score >= sieve_t (may exceed the list's capacity)
+  int sieve_count;          // sieve path: elements with a raw score >= sieve_t (may exceed the list's capacity; unsigned
+                            // like bnd_count)
   int need_slow;            // 1: the digit passes run for this segment (sieve off, or its result could not be proven exact)
 };
 
@@ -226,7 +228,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_hist_kernel(const float *__
   const SegDesc d = tab.s[seg];
   if (d.len <= small_max) return;   // (0 when the tail kernel is not in use: k > kBitonicMax)
   const SegState st = state[seg];
-  const bool use_b = bnd != nullptr && st.bnd_count <= kBndCap;
+  const bool use_b = bnd != nullptr && (unsigned)st.bnd_count <= (unsigned)kBndCap;
   const long long len = use_b ? (long long)st.bnd_count : (long long)d.len;
   if ((long long)blockIdx.x * kItemsPerCta >= len) return;
   if (st.k_take <= 0) return;
@@ -512,7 +514,7 @@ __global__ void __launch_bounds__(kKeyThreads) topk_split_keys_kernel(const SegT
           if (gp < k) cand[(long long)seg * k + gp] = key;
         } else {
           const int gp = atomicAdd(&state[seg].bnd_count, 1);
-          if (gp < kBndCap) bnd[(long long)seg * kBndCap + gp] = key;
+          if ((unsigned)gp < (unsigned)kBndCap) bnd[(long long)seg * kBndCap + gp] = key;
         }
       }
     }
@@ -527,8 +529,10 @@ __global__ void __launch_bounds__(kKeyThreads) topk_split_keys_kernel(const SegT
     const int n = min(s_n[which], kSplitStage), gb = s_base[which];
     const int cap = which == 0 ? k : kBndCap;
     unsigned long long *dst = which == 0 ? cand + (long long)seg * k : bnd + (long long)seg * kBndCap;
-    for (int i = threadIdx.x; i < n; i += kKeyThreads)
-      if (gb + i < cap) dst[gb + i] = stage[which][i];
+    for (int i = threadIdx.x; i < n; i += kKeyThreads) {
+      const unsigned at = (unsigned)gb + (unsigned)i;
+      if (at < (unsigned)cap) dst[at] = stage[which][i];
+    }
   }
 }
 
@@ -542,7 +546,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_collect_kernel(const float 
   const SegDesc d = tab.s[seg];
   const long long base = (long long)blockIdx.x * kItemsPerCta;
   const SegState st = state[seg];
-  const bool use_b = bnd != nullptr && st.bnd_count <= kBndCap;  // keys above the boundary bin are in cand already
+  const bool use_b = bnd != nullptr && (unsigned)st.bnd_count <= (unsigned)kBndCap;  // keys above the boundary bin are in cand already
   const long long len = use_b ? (long long)st.bnd_count : (long long)d.len;
   if (base >= len) return;
   if (st.k_take <= 0) return;
@@ -627,7 +631,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_split_kernel(const float *_
           if (pos < k) cand[(long long)seg * k + pos] = key;
         } else {
           const int pos = atomicAdd(&state[seg].bnd_count, 1);
-          if (pos < kBndCap) bnd[(long long)seg * kBndCap + pos] = key;
+          if ((unsigned)pos < (unsigned)kBndCap) bnd[(long long)seg * kBndCap + pos] = key;
         }
       }
     }
@@ -637,7 +641,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_split_kernel(const float *_
 // Boundary bin larger than the buffer (mass ties): forget the split, the full-data passes and collect take over.
 __global__ void topk_after_split_kernel(SegState *state, int nseg) {
   const int s = threadIdx.x;
-  if (s < nseg && state[s].bnd_count > kBndCap) state[s].cand_count = 0;
+  if (s < nseg && (unsigned)state[s].bnd_count > (unsigned)kBndCap) state[s].cand_count = 0;
 }
 
 // rank-by-counting sort of the (unique) candidate keys, descending.  grid (ceil(k/256), nseg).
@@ -833,7 +837,7 @@ __global__ void __launch_bounds__(kKeyThreads) topk_sieve_kernel(const float *__
       stage[pos] = key;
     } else {   // staging full (a segment of a few CTAs puts a large share of its elements on the list)
       const int gp = atomicAdd(&st->sieve_count, 1);
-      if (gp < cap) list[gp] = key;
+      if ((unsigned)gp < (unsigned)cap) list[gp] = key;
     }
   }
   __syncthreads();
@@ -842,8 +846,10 @@ __global__ void __launch_bounds__(kKeyThreads) topk_sieve_kernel(const float *__
   if (threadIdx.x == 0) s_base = atomicAdd(&st->sieve_count, n);
   __syncthreads();
   const int gb = s_base;
-  for (int i = threadIdx.x; i < n; i += kKeyThreads)
-    if (gb + i < cap) list[gb + i] = stage[i];
+  for (int i = threadIdx.x; i < n; i += kKeyThreads) {
+    const unsigned at = (unsigned)gb + (unsigned)i;
+    if (at < (unsigned)cap) list[at] = stage[i];
+  }
 }
 
 constexpr int kBitonicMax = 4096;
@@ -1013,7 +1019,7 @@ __global__ void __launch_bounds__(kTailThreads) topk_tail_kernel(const float *__
     // ---- sieve path: select the k largest of the list, sort, prove that nothing outside the list can belong (see above)
     const SegState st = state[seg];
     const int cap = k + kBndCap, nc = st.sieve_count;
-    if (nc < k || nc > cap || phase == 3) return;   // need_slow stays 1
+    if ((unsigned)nc < (unsigned)k || (unsigned)nc > (unsigned)cap || phase == 3) return;   // need_slow stays 1
     for (int i = tid; i < nc; i += kTailThreads) sk[i] = cand[(long long)seg * cap + i];
     __syncthreads();
     unsigned long long *sk2 = sk + kSmallMax;
@@ -1088,7 +1094,7 @@ __global__ void __launch_bounds__(kTailThreads) topk_tail_kernel(const float *__
     n_out = st.k_take;
     by_index = small_by_index && st.eff_len <= (unsigned)k;
     if (n_out > 0) {
-      if (st.bnd_count <= kBndCap) {
+      if ((unsigned)st.bnd_count <= (unsigned)kBndCap) {
         // ---- the k_rem largest keys of the boundary bin join the cand_count certain ones
         const int nb = st.bnd_count, need = st.k_rem, c = n_out - need;
         const int np2 = pow2_at_least(nb);
@@ -1401,6 +1407,10 @@ using namespace roi3d;
 
 extern "C" {
 
+// Longest segment: the kernels index a segment's elements with 32-bit unsigned integers and add up to one flat-grid
+// chunk (kFirstItemsPerCta = 32768 elements) to an index before they compare it with the end, so the length keeps
+// 64 K of margin below 2^32.
+static const long long kMaxSegLen = 0xFFFF0000LL;
 static const size_t kStateBytes = 4096;                                     // kMaxSeg * sizeof(SegState) + tickets, rounded up
 static const size_t kHistBytes = (size_t)kMaxSeg * kBins * sizeof(unsigned);  // 512 KiB
 
@@ -1468,7 +1478,8 @@ int roi3d_topk_segmented_masked(const float *scores_dev, const int64_t *seg_off,
     SegTable tab;
     long long maxlen = 0, koff = 0;   // maxlen: over the segments that go through the digit passes
     for (int s = 0; s < ns; ++s) {
-      ROI3D_CHECK_ARG(seg_len[s0 + s] >= 0 && seg_len[s0 + s] < 4294967295LL, "segment %d too long", s0 + s);
+      ROI3D_CHECK_ARG(seg_len[s0 + s] >= 0 && seg_len[s0 + s] <= kMaxSegLen, "segment %d: length %lld outside [0, %lld]", s0 + s,
+                      (long long)seg_len[s0 + s], kMaxSegLen);
       tab.s[s].off = seg_off[s0 + s];
       tab.s[s].len = (unsigned)seg_len[s0 + s];
       if (seg_adhw) {

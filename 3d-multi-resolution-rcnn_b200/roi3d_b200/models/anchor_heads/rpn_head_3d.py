@@ -90,11 +90,14 @@ def _topk_segmented_desc(dev, ptrs, lens, adhw, k, apply_sigmoid, small_in_index
     nseg = len(ptrs)
     # the host-side descriptor arrays only depend on the segments' relative addresses and shapes, which repeat from call
     # to call: built once per signature (three numpy constructions per call otherwise)
-    base = min(ptrs)
-    dkey = (tuple([q - base for q in ptrs]), tuple(lens), None if adhw is None else tuple(map(tuple, adhw)))
+    # an empty segment reads nothing and its tensor's address may be 0: it takes offset 0 and plays no part in the base
+    live = [q for q, n in zip(ptrs, lens) if n > 0]
+    base = min(live) if live else None
+    rel = [q - base if n > 0 else 0 for q, n in zip(ptrs, lens)]
+    dkey = (tuple(rel), tuple(lens), None if adhw is None else tuple(map(tuple, adhw)))
     desc = _DESC_CACHE.get(dkey)
     if desc is None:
-        off = np.array([(q - base) // 4 for q in ptrs], dtype=np.int64)
+        off = np.array([r // 4 for r in rel], dtype=np.int64)
         ln = np.array(lens, dtype=np.int64)
         adhw_a = np.array(adhw, dtype=np.int32) if adhw is not None else None
         if len(_DESC_CACHE) > 64:
@@ -107,6 +110,8 @@ def _topk_segmented_desc(dev, ptrs, lens, adhw, k, apply_sigmoid, small_in_index
     # base workspace + one u32 key per score (the first digit pass stores the keys, later passes re-read them from L2)
     nbytes = _lib.lib.roi3d_topk_workspace_bytes_keys(nseg, k, total_len)
     _buf, ws = workspace(dev, nbytes)
+    if base is None:   # every segment empty: no score is read, but the entry wants a device address
+        base = ws
     mask_p = (ctypes.c_void_p * nseg)(*mask_ptrs) if mask_ptrs is not None else None
     cnt = torch.empty((nseg,), dtype=torch.int32, device=dev) if report else None
     srt = torch.empty((nseg,), dtype=torch.uint8, device=dev) if report else None

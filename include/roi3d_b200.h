@@ -301,7 +301,12 @@ int roi3d_roi_align3d_forward_host(const float *feats_host, int layout, int B, i
  * scores_dev + seg_off[s]) the k_s = min(k, n_s) largest, DESCENDING, ties -> lower index.
  * Replaces: scores.topk(cfg.nms_pre), rpn_head_3d.py:108-112, and the final topk :147.
  * apply_sigmoid=1 ranks sigmoid(x) = 1/(1+exp(-x)) (rpn_head_3d.py:90) and returns those values.
- * seg_off/seg_len are HOST arrays (int64) of length nseg.
+ * Values are ranked and returned through an order-preserving key, not copied: -0.0 ranks equal to +0.0 (the tie goes
+ * to the lower index) and comes back as +0.0; every NaN, of either sign and with any payload, ranks above +inf, ties
+ * with the other NaNs, and comes back as 0x7FFFFFFF.  Every other value comes back bit for bit.  (torch.topk returns
+ * the element itself.)
+ * seg_off/seg_len are HOST arrays (int64) of length nseg; 0 <= seg_len[s] <= 0xFFFF0000 (4294901760), a longer
+ *   segment returns ROI3D_EINVAL before anything is launched.
  * seg_adhw (HOST int32 [nseg,4] = A,D,H,W, or NULL): when given (A>0), segment s is an [A,D,H,W] score map
  *   and indices are LOGICAL positions after permute(2,3,1,0).reshape(-1) (rpn_head_3d.py:87-89), i.e.
  *   ((y*W + x)*D + z)*A + a -- the order grid_anchors enumerates anchors in -- both for the returned index

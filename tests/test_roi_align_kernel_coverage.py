@@ -13,20 +13,14 @@ and size, and 1/16 voxel outside -1 and size, one axis at a time), RoIs whose ba
 and, where the level is wide enough, one RoI wider than the 40-voxel tables (the literal fallback inside the same
 launch).  K is odd, so the last CTA of the per-warp kernels is partial.
 """
-import os
-import re
-import shutil
-import subprocess
 from collections import namedtuple
 
 import numpy as np
 import pytest
 
 import synth
+from kernel_inventory import built_kernels, kernel_key, launched_kernels, library_kernels
 from test_gpu_parity import BWD_TOL, FWD_TOL, rel_err
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "3d-multi-resolution-rcnn_b200", "lib", "libroi3d_b200.so")
 
 SCALE, SCALE_D = 0.25, 0.5
 STRIDES, STRIDES_D = [4, 8, 16, 32, 64], [2, 4, 8, 16, 32]
@@ -38,54 +32,9 @@ HELPERS = ("roi_align3d_plan_kernel", "roi_align3d_order_kernel", "roi_align3d_d
 
 
 # ------------------------------------------------------------------------------------------------ kernel names
-def _demangle(names):
-    if not names:
-        return []
-    cxxfilt = shutil.which("c++filt")
-    assert cxxfilt, "c++filt (binutils) is needed to demangle kernel names"
-    out = subprocess.run([cxxfilt], input="\n".join(names), capture_output=True, text=True, check=True).stdout
-    return out.splitlines()
-
-
-def kernel_key(name):
-    """Base name plus template argument list with the spaces removed: `void roi3d::roi_align3d_fwd_cl_kernel<14, 7, 1,
-    3>(roi3d::RoiParams)` -> `roi_align3d_fwd_cl_kernel<14,7,1,3>`.  None for a name that is not a `*_kernel`."""
-    if name.startswith("_Z"):
-        name = _demangle([name])[0]
-    m = re.search(r"(\w+_kernel)\s*([<(]|$)", name)
-    if m is None:
-        return None
-    key = m.group(1)
-    if m.group(2) == "<":
-        depth, i = 0, m.start(2)
-        for j in range(i, len(name)):
-            depth += {"<": 1, ">": -1}.get(name[j], 0)
-            if depth == 0:
-                key += name[i:j + 1]
-                break
-    return re.sub(r"\s+", "", key)
-
-
-def launched_kernels(fn):
-    """Run fn() under torch.profiler with CUDA activities and return the demangled names of the kernels that ran
-    (memcpy / memset records excluded).  CUPTI sees every launch of the context, those of libroi3d_b200.so included."""
-    import torch
-    from torch.autograd import DeviceType
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    names = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA
-             and not e.name.startswith(("Memcpy", "Memset", "cudaMem"))]
-    assert names, "the profiler recorded no kernel: nothing would be checked"
-    return names
-
-
 def compute_kernels(names):
     """The RoIAlign3D compute kernels among launched kernel names (library kernels other than the helpers)."""
-    keys = [kernel_key(n) for n in names if "roi3d::" in n or n.startswith("_ZN5roi3d")]
-    return sorted({k for k in keys if k is not None and k.split("<")[0] not in HELPERS})
+    return sorted(k for k in library_kernels(names) if k.split("<")[0] not in HELPERS)
 
 
 # ------------------------------------------------------------------------------------------------ the map
@@ -520,21 +469,10 @@ def test_roi_align_kernel_row(oracle, dev, r):
 
 
 # ------------------------------------------------------------------------------------------------ CPU checks
-def _built_roi_align_kernels():
-    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cuobjdump = os.path.join(os.path.dirname(nvcc), "cuobjdump")
-    assert os.path.exists(LIB), "%s is not built" % LIB
-    assert os.path.exists(cuobjdump), "%s not found" % cuobjdump
-    elf = subprocess.run([cuobjdump, "-elf", LIB], capture_output=True, text=True, check=True).stdout
-    mangled = sorted(set(re.findall(r"\.text\.([A-Za-z0-9_$]+)", elf)))
-    keys = {kernel_key(n) for n in _demangle(mangled)}
-    return {k for k in keys if k is not None and k.startswith("roi_align3d_")}
-
-
 def test_every_roi_align_kernel_has_a_coverage_row():
     """The RoIAlign3D instantiations in the built library are exactly the COVERAGE kernels plus the helpers: a kernel
     added without a row here fails this test on any machine."""
-    built = _built_roi_align_kernels()
+    built = built_kernels("roi_align3d_")
     covered = {kernel_key(r.kernel) for r in COVERAGE}
     helpers = {h for h in HELPERS if h.startswith("roi_align3d_")}
     assert not covered & helpers
