@@ -1,5 +1,5 @@
-"""`nms(dets, iou_thr, device_id=None)`: the reference's dispatch wrapper (mmdet/ops/nms/nms_wrapper.py:8-52)
-over the B200 3D NMS.
+"""`nms(dets, iou_thr, device_id=None)` and `soft_nms(dets, iou_thr, method, sigma, min_score)`: the reference's
+dispatch wrappers (mmdet/ops/nms/nms_wrapper.py:8-52, :55-81) over the B200 3D NMS and 3D soft-NMS.
 
 Same surface: Tensor or ndarray in, `(dets[inds, :], inds)` out in the input's type; N == 0 returns an empty
 long index; `inds` are ORIGINAL row indices in ascending order (nms_kernel.cu:253-256).
@@ -11,6 +11,12 @@ Differences, all deliberate:
     silently running the reference's 2-D `nms_cpu` on columns 0-4 (nms_wrapper.py:47-48, SURVEY F3);
   * the sweep runs on the device: one 4-byte D2H read (the kept count) instead of the reference's blocking
     copy of the whole bit matrix plus a host loop (nms_kernel.cu:225-249).
+
+soft_nms is the reference's soft_nms_cpu loop (mmdet v0.6.0, soft_nms_cpu.pyx) in 3-D on [N,7] rows, run on the
+device by roi3d_soft_nms3d_batched and equal to that loop bit for bit (include/roi3d_b200.h states the limits):
+rows come back in selection order with the score each had when it was selected, `inds` are original row indices.
+The reference's own soft_nms is 2-D, runs on the CPU and stops in a debugger on entry (nms_wrapper.py:56).  As for
+nms, a CPU tensor and input other than [N,7] raise NotImplementedError; an ndarray runs on the current CUDA device.
 """
 import ctypes
 
@@ -107,7 +113,65 @@ def nms(dets, iou_thr, device_id=None):
     return dets[inds, :], inds
 
 
+SOFT_NMS_METHODS = {'linear': 1, 'gaussian': 2}
+SOFT_NMS_MAX_ROWS = 4096   # rows per segment the kernel takes (one CTA holds a segment's boxes in shared memory)
+
+
+def soft_nms3d_batched(dets, seg_counts, iou_thr, method='linear', sigma=0.5, min_score=1e-3):
+    """Batched device soft-NMS.  dets [nseg, n_max, 7] fp32 CUDA, n_max <= 4096; seg_counts int32 [nseg] CUDA or None.
+    Returns (out_dets [nseg, n_max, 7] fp32, inds [nseg, n_max] int64, num_keep [nseg] int32): per segment the first
+    num_keep rows in selection order, with the scores they had when selected, and their row indices; nothing syncs."""
+    if method not in SOFT_NMS_METHODS:
+        raise ValueError('Invalid method for SoftNMS: {}'.format(method))
+    check_cuda_f32(dets, "dets", ndim=3, last=7)
+    dets = dets.contiguous()
+    nseg, n_max, _ = dets.shape
+    dev = dets.device
+    out = torch.empty((nseg, n_max, 7), dtype=torch.float32, device=dev)
+    inds = torch.empty((nseg, n_max), dtype=torch.int64, device=dev)
+    num = torch.empty((nseg,), dtype=torch.int32, device=dev)
+    if seg_counts is not None:
+        assert seg_counts.dtype == torch.int32 and seg_counts.is_cuda and seg_counts.numel() == nseg
+        seg_counts = seg_counts.contiguous()
+    with device_guard(dev), nvtx_range("roi3d.soft_nms3d_batched"):
+        _lib.check(_lib.lib.roi3d_soft_nms3d_batched(
+            dets.data_ptr(), None if seg_counts is None else seg_counts.data_ptr(), nseg, n_max,
+            SOFT_NMS_METHODS[method], float(iou_thr), float(sigma), float(min_score), out.data_ptr(), inds.data_ptr(),
+            num.data_ptr(), stream_ptr()))
+    return out, inds, num
+
+
 def soft_nms(dets, iou_thr, method='linear', sigma=0.5, min_score=1e-3):
-    """Out of scope (SURVEY section 2): unused by configs/3d-multi-resolution-rcnn.py, and the reference's
-    own implementation stops in a debugger on entry (nms_wrapper.py:56)."""
-    raise NotImplementedError("soft_nms is not part of the 3D RoI hot path")
+    """Dispatch wrapper with the reference's signature (nms_wrapper.py:55): (new_dets, inds), a new tensor and int64
+    indices on the input's device for a CUDA tensor (one host read: the count), float32 / int64 ndarrays for an
+    ndarray (run on the current CUDA device)."""
+    if isinstance(dets, torch.Tensor):
+        is_numpy = False
+    elif isinstance(dets, np.ndarray):
+        is_numpy = True
+    else:
+        raise TypeError('dets must be either a Tensor or numpy array, but got {}'.format(type(dets)))
+    if method not in SOFT_NMS_METHODS:
+        raise ValueError('Invalid method for SoftNMS: {}'.format(method))
+
+    if is_numpy:
+        if dets.ndim != 2 or dets.shape[1] != 7:
+            raise NotImplementedError("soft_nms: only [N,7] 3D boxes are supported, got shape %s" % (dets.shape,))
+        if dets.shape[0] == 0:
+            return np.zeros((0, 7), dtype=np.float32), np.zeros(0, dtype=np.int64)
+        d = torch.from_numpy(np.ascontiguousarray(dets, dtype=np.float32)).to(torch.cuda.current_device())
+        out, inds, num = soft_nms3d_batched(d[None], None, iou_thr, method, sigma, min_score)
+        m = int(num.item())
+        return out[0, :m].cpu().numpy(), inds[0, :m].cpu().numpy()
+
+    if dets.shape[0] == 0:
+        return dets.new_zeros((0,) + tuple(dets.shape[1:])), dets.new_zeros(0, dtype=torch.long)
+    if not dets.is_cuda:
+        raise NotImplementedError(
+            "soft_nms: CPU tensors are not supported by the B200 path (the reference runs 2-D soft_nms_cpu on "
+            "columns 0-4); move dets to the GPU.")
+    if dets.dim() != 2 or dets.shape[1] != 7:
+        raise NotImplementedError("soft_nms: only [N,7] 3D boxes are supported, got shape %s" % (tuple(dets.shape),))
+    out, inds, num = soft_nms3d_batched(dets.detach().unsqueeze(0), None, iou_thr, method, sigma, min_score)
+    m = int(num.item())  # the one host read: the result length is data dependent
+    return out[0, :m], inds[0, :m]

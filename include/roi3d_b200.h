@@ -186,6 +186,25 @@ int roi3d_nms3d_eval_batched(const float *dets_dev, const int32_t *seg_counts_de
                              int64_t *keep_dev, int64_t *keep_by_score_dev, int32_t *num_keep_dev,
                              void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* 3D soft-NMS, batched over independent segments (one segment = one class or one volume), one launch, no host sync.
+ * Restates: soft_nms_cpu, mmdet/ops/nms/src/soft_nms_cpu.pyx (mmdet v0.6.0), reached through soft_nms,
+ *   mmdet/ops/nms/nms_wrapper.py:55-81, and multiclass_nms_3d with nms type 'soft_nms' (bbox_nms.py:75-77); the
+ *   reference's loop is 2-D and runs on the CPU, this is its 3-D form with a depth axis and the score in column 6.
+ * dets_dev: [nseg, n_max, 7] fp32 (x1,y1,x2,y2,z1,z2,score); segment s uses its first seg_counts_dev[s] rows
+ *   (seg_counts_dev == NULL: every segment has n_max rows).  n_max <= 4096; a larger n_max returns ROI3D_EINVAL
+ *   before anything is launched.
+ * method: 1 = linear (weight 1 - iou where iou > iou_thr), 2 = gaussian (weight exp(-iou^2 / sigma)); any other value
+ *   returns ROI3D_EINVAL.  iou_thr, sigma and min_score are fp32, as the reference's Cython parameters are.
+ * Outputs, in selection order: out_dets_dev [nseg, n_max, 7] the selected rows with the score each had when it was
+ *   selected, inds_dev int64 [nseg, n_max] their row indices in the segment, num_keep_dev int32 [nseg] the number of
+ *   rows left (rows past num_keep are not written).  The result equals the reference loop bit for bit for finite
+ *   coordinates (ties go to the first position in the loop's current row order; a NaN score is selected only at
+ *   position i and never dropped), except that a gaussian weight can differ in its last fp32 bit where CUDA's double
+ *   exp and the host libm's round differently across an fp32 rounding boundary. */
+int roi3d_soft_nms3d_batched(const float *dets_dev, const int32_t *seg_counts_dev, int nseg, int n_max, int method,
+                             float iou_thr, float sigma, float min_score, float *out_dets_dev, int64_t *inds_dev,
+                             int32_t *num_keep_dev, void *stream);
+
 /* Host-buffer form of one NMS call: what mmdet.ops.nms(dets_numpy, thr, device_id) does
  * (mmdet/ops/nms/nms_wrapper.py:29-32,42-52).  keep_host capacity n; returns count in *num_keep_host. */
 int roi3d_nms3d_host(const float *dets_host, int n, float iou_thr, int64_t *keep_host, int32_t *num_keep_host);
