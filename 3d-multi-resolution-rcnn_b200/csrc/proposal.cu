@@ -1399,6 +1399,81 @@ __global__ void __launch_bounds__(256) gather_rows7_kernel(const float *__restri
   for (int q = 0; q < 7; ++q) dst[q] = src[q];
 }
 
+// ------------------------------------------------------------------------------------------------
+// `min_bbox_size` filter of get_bboxes_single (mmdet v0.6.0 RPNHead): keep a row iff (x2 - x1) + 1 >= m and
+// (y2 - y1) + 1 >= m, each operation one fp32 rounding as torch evaluates it; NaN fails.  Depth is not compared.
+// Stable in-place compaction of the first counts_in[s] rows of each segment, one CTA per segment: per chunk of
+// kFilterThreads * kFilterRows rows every thread holds its rows in registers, warp ballots give each (row slot, warp)
+// its count, warp 0 scans the counts, and the survivors are written at the running offset.  A write never reaches
+// past the chunk being processed (the offset never exceeds the chunk start), and every read of the chunk happens
+// before the first barrier, so rows are not overwritten before they are read.  Two barriers per chunk also order the
+// shared counts and offsets across chunks: a chunk's counts are written after the previous chunk's second barrier,
+// its offsets after its own first one.  The count lands in counts_out[s].
+// ------------------------------------------------------------------------------------------------
+constexpr int kFilterThreads = 512;
+constexpr int kFilterRows = 4;                                   // rows per thread per chunk
+constexpr int kFilterWarps = kFilterThreads / 32;
+constexpr int kFilterSlots = kFilterRows * kFilterWarps;         // (row slot, warp) counts per chunk, scanned by warp 0
+static_assert(kFilterSlots == 64, "warp 0 scans two slots per lane");
+
+__global__ void __launch_bounds__(kFilterThreads) filter_min_size_rows7_kernel(float *__restrict__ dets, int k,
+                                                                                const int32_t *counts_in, float m,
+                                                                                int32_t *counts_out) {
+  __shared__ int slot_cnt[kFilterSlots];
+  __shared__ int slot_off[kFilterSlots + 1];
+  const int s = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int n = min(max(counts_in[s], 0), k);
+  float *d = dets + (long long)s * k * 7;
+  int kept = 0;   // rows written so far (the same in every thread)
+  for (int base = 0; base < n; base += kFilterThreads * kFilterRows) {
+    float r[kFilterRows][7];
+    bool pass[kFilterRows];
+    unsigned ball[kFilterRows];
+#pragma unroll
+    for (int j = 0; j < kFilterRows; ++j) {
+      const int i = base + j * kFilterThreads + threadIdx.x;
+      pass[j] = false;
+      if (i < n) {
+#pragma unroll
+        for (int q = 0; q < 7; ++q) r[j][q] = d[(long long)i * 7 + q];
+        const float w = __fadd_rn(__fsub_rn(r[j][2], r[j][0]), 1.0f);
+        const float h = __fadd_rn(__fsub_rn(r[j][3], r[j][1]), 1.0f);
+        pass[j] = (w >= m) && (h >= m);
+      }
+      ball[j] = __ballot_sync(0xffffffffu, pass[j]);
+      if (lane == 0) slot_cnt[j * kFilterWarps + warp] = __popc(ball[j]);
+    }
+    __syncthreads();
+    if (warp == 0) {   // exclusive scan of the 64 slot counts in (row slot, warp) order = row order
+      const int a = slot_cnt[2 * lane], b = slot_cnt[2 * lane + 1];
+      int incl = a + b;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+      }
+      slot_off[2 * lane] = incl - a - b;
+      slot_off[2 * lane + 1] = incl - b;
+      if (lane == 31) slot_off[kFilterSlots] = incl;
+    }
+    __syncthreads();
+    const unsigned below = (1u << lane) - 1u;
+#pragma unroll
+    for (int j = 0; j < kFilterRows; ++j) {
+      if (!pass[j]) continue;
+      const int i = base + j * kFilterThreads + threadIdx.x;
+      const int o = kept + slot_off[j * kFilterWarps + warp] + __popc(ball[j] & below);
+      if (o != i) {
+#pragma unroll
+        for (int q = 0; q < 7; ++q) d[(long long)o * 7 + q] = r[j][q];
+      }
+    }
+    kept += slot_off[kFilterSlots];
+  }
+  __syncthreads();   // counts_out may be counts_in: every thread has read its count
+  if (threadIdx.x == 0) counts_out[s] = kept;
+}
+
 int g_topk_sieve = 0;   // roi3d_set_tuning key 11: 0 = sieve path where it applies, -1 = digit passes only, 2 = sieve gives up (tests)
 
 }  // namespace roi3d
@@ -1724,6 +1799,18 @@ int roi3d_gather_rows7(const float *rows_dev, int nseg, int rows_per_seg, const 
   ROI3D_CHECK_ARG(rows_dev && idx_dev && out_dev, "NULL pointer");
   gather_rows7_kernel<<<dim3(ceil_div(n, 256), nseg), 256, 0, (cudaStream_t)stream>>>(rows_dev, rows_per_seg, idx_dev, n,
                                                                                       out_dev);
+  ROI3D_LAUNCH_CHECK();
+  return ROI3D_OK;
+}
+
+int roi3d_filter_min_size_rows7(float *dets_dev, int nseg, int k, const int32_t *counts_in_dev, float min_size,
+                                int32_t *counts_out_dev, void *stream) {
+  ROI3D_CHECK_ARG(nseg >= 0 && k >= 0, "bad sizes: nseg=%d k=%d", nseg, k);
+  ROI3D_CHECK_ARG(min_size == min_size, "min_size is NaN");
+  if (nseg == 0) return ROI3D_OK;
+  ROI3D_CHECK_ARG((dets_dev || k == 0) && counts_in_dev && counts_out_dev, "NULL pointer");
+  filter_min_size_rows7_kernel<<<nseg, kFilterThreads, 0, (cudaStream_t)stream>>>(dets_dev, k, counts_in_dev, min_size,
+                                                                                 counts_out_dev);
   ROI3D_LAUNCH_CHECK();
   return ROI3D_OK;
 }

@@ -99,6 +99,7 @@ def _load():
         "roi3d_topk_segmented_masked": (c_int, [P, P, P, P, P, c_int, c_int, c_int, c_int, P, P, P, P, P, c_size_t, P]),
         "roi3d_rpn_collect": (c_int, [P, c_int, c_int, c_int, P, P, P, P, c_int, P, P, P, P]),
         "roi3d_gather_rows7": (c_int, [P, c_int, c_int, P, c_int, P, P]),
+        "roi3d_filter_min_size_rows7": (c_int, [P, c_int, c_int, P, c_float, P, P]),
         "roi3d_decode_proposals": (c_int, [P, c_int, c_int, c_int, c_int, c_float, c_float, P, P, P, c_int, P, P,
                                            c_float, c_float, c_float, P, P]),
         "roi3d_decode_proposals_batched": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, c_int, P, P, P, P]),

@@ -16,8 +16,13 @@ one segmented top-k for the final cut, and a single host read of the result leng
 The head's cached inside-flag masks `pos_indices` / `pos_indices_test` (anchor_head_3d.py:212,239-243) are honoured
 the way rpn_head_3d.py:97-106 applies them: on a level with more than nms_pre anchors, when the mask has the level's
 shape, only the masked-in anchors take part in the top-k (the mask goes into the segmented top-k; nothing is
-compacted).  Not reproduced: the `min_bbox_size > 0` branch, which stops in a debugger in the reference (:125-132)
-and raises here.
+compacted).
+
+`min_bbox_size > 0` drops, per (image, level), the decoded proposals whose width or height ((x2 - x1) + 1, (y2 - y1) + 1
+in fp32) is below it, before that level's NMS, as mmdetection v0.6.0's RPNHead does; the fork's own branch stops in a
+debugger (:125-132).  Depth is not compared: z is measured in slices, x and y in pixels, and one pixel threshold on the
+depth would drop nearly every fine-level proposal (the level-0 anchors are 8 x 8 pixels by 4 slices).  The survivors
+keep their order, so score-sorted levels stay sorted and index-order levels stay in anchor order.
 """
 import ctypes
 
@@ -206,7 +211,7 @@ class RPNProposal3D(object):
             key = (tuple(t.data_ptr() for t in list(cls_scores) + list(bbox_preds) + masks_now),
                    tuple(tuple(t.shape) for t in list(cls_scores) + list(bbox_preds)),
                    tuple(tuple(m['img_shape']) for m in img_metas),
-                   tuple(_cfg_get(cfg, n) for n in ('nms_pre', 'nms_post', 'max_num', 'nms_thr')))
+                   tuple(_cfg_get(cfg, n) for n in ('nms_pre', 'nms_post', 'max_num', 'nms_thr', 'min_bbox_size')))
             entry = self._graphs.get(key)
             if entry is None:
                 self._enqueue(cls_scores, bbox_preds, img_metas, cfg)  # warm-up: scratch, descriptor cache, attributes
@@ -241,8 +246,7 @@ class RPNProposal3D(object):
         nms_post = int(_cfg_get(cfg, 'nms_post'))
         max_num = int(_cfg_get(cfg, 'max_num'))
         nms_thr = float(_cfg_get(cfg, 'nms_thr'))
-        if _cfg_get(cfg, 'min_bbox_size', 0) > 0:
-            raise NotImplementedError("min_bbox_size > 0 is broken in the reference (rpn_head_3d.py:125-132)")
+        min_size = float(_cfg_get(cfg, 'min_bbox_size', 0))
         across = bool(_cfg_get(cfg, 'nms_across_levels', False))
         L, B = len(cls_scores), len(img_metas)
         dev = cls_scores[0].device
@@ -334,6 +338,14 @@ class RPNProposal3D(object):
                 ptrs, adhw.ctypes.data, lvl.ctypes.data, img.ctypes.data, B * L, L, A, base.ctypes.data,
                 strides.ctypes.data, dstrides.ctypes.data, idx.data_ptr(), val.data_ptr(), k, means.ctypes.data,
                 stds.ctypes.data, dets.data_ptr(), stream_ptr()))
+        if min_size > 0:
+            # 2b. min_bbox_size: compact each segment's rows in place, in order, into a NEW count tensor (seg_counts may
+            #     be the cached descriptor of this shape signature)
+            kept = torch.empty_like(seg_counts)
+            with torch.cuda.device(dev):
+                _lib.check(_lib.lib.roi3d_filter_min_size_rows7(dets.data_ptr(), B * L, k, seg_counts.data_ptr(), min_size,
+                                                                kept.data_ptr(), stream_ptr()))
+            seg_counts = kept
 
         # 3. one batched NMS; kept rows in descending-score order
         #    (a score-sorted level only contributes proposals[:nms_post]: its sweep stops once that many are kept)

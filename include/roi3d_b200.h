@@ -374,6 +374,17 @@ int roi3d_rpn_collect(const float *dets_dev, int num_images, int num_levels, int
 /* out[s][j] = rows[s][idx[s][j]] for 7-float rows (idx < 0 -> zeros): the final `proposals[topk_inds]`, :147-148. */
 int roi3d_gather_rows7(const float *rows_dev, int nseg, int rows_per_seg, const int64_t *idx_dev, int n,
                        float *out_dev, void *stream);
+/* The `min_bbox_size` filter of get_bboxes_single (mmdet v0.6.0 RPNHead, between delta2bbox and NMS; the fork's own
+ * branch stops in a debugger, rpn_head_3d.py:125-132), for decoded rows dets_dev [nseg, k, 7] (x1,y1,x2,y2,z1,z2,score):
+ * of the first min(max(counts_in_dev[s], 0), k) rows of segment s, keep a row iff (x2 - x1) + 1 >= min_size and
+ * (y2 - y1) + 1 >= min_size, each - and + one fp32 operation as torch evaluates them (a NaN width drops the row); depth
+ * is not compared.  The kept rows are moved to the front of their segment IN PLACE, in their original order, and their
+ * number is written to counts_out_dev[s] (int32 [nseg]; may be counts_in_dev).  Rows past the new count are left
+ * undefined.  One launch, no host synchronisation.  The rule applies to any min_size; a caller that skips the filter for
+ * min_size <= 0, as the reference does, does not call this.  NaN min_size, negative sizes and NULL pointers return
+ * ROI3D_EINVAL. */
+int roi3d_filter_min_size_rows7(float *dets_dev, int nseg, int k, const int32_t *counts_in_dev, float min_size,
+                                int32_t *counts_out_dev, void *stream);
 
 /* Anchor base + decode of selected anchors for one level, fused:
  *   anchors as AnchorGenerator3D.grid_anchors would generate them
