@@ -111,6 +111,370 @@ __device__ __forceinline__ void build_tables(Tables<PW> &T, const Item &it, int 
   __syncwarp();
 }
 
+// CTA-shared per-RoI tables of the ring2 and bwd2 kernels, whose warps all work on one RoI.
+//   Dx[(x - xmin) * PWP + pw], Dy[(y - ymin) * PP2 + ph] (all PH rows), Dz[(z - zmin) * PP2 + pd] (all PD slices);
+//   box = xmin, xmax, ymin, ymax, zmin, zmax.  The x extras are each kernel's own: the forward (XANY = false) keeps
+//   xlo / xhi[pw] relative to xmin, the backward (XANY = true) keeps xany[x - xmin] and one more zero row of Dx,
+//   which its paired x loop may read one past RX.
+constexpr int RZMAX2 = 40;
+constexpr int PP2 = 16;  // padded row length of the CTA-shared y / z tables (PH, PD <= 16)
+template <int PW, bool XANY>
+struct CtaTables {
+  static constexpr int PWP = Tables<PW>::PWP;
+  static constexpr int DX_ROWS = XANY ? RXMAX + 1 : RXMAX;
+  static constexpr int XTRA = XANY ? RXMAX : 32;  // xany[RXMAX] or xlo[16] + xhi[16]
+  // 200 spare floats keep the forward's shared-memory footprint, and with it the occupancy, as measured
+  static constexpr int SPARE = XANY ? 0 : 200;
+  static constexpr int FLOATS = (DX_ROWS * PWP + (RYMAX + RZMAX2) * PP2 + XTRA + 8 + SPARE + 3) / 4 * 4;
+  float *Dx, *Dy, *Dz;
+  int *xlo, *xhi, *xany, *box;
+  int xmin, xmax, ymin, ymax, zmin, zmax;
+  bool empty, fits;
+  __device__ __forceinline__ void bind(float *sm) {
+    Dx = sm;
+    Dy = Dx + DX_ROWS * PWP;
+    Dz = Dy + RYMAX * PP2;
+    xlo = xany = reinterpret_cast<int *>(Dz + RZMAX2 * PP2);
+    xhi = xlo + 16;
+    box = xlo + XTRA;
+  }
+};
+
+// Builds T for RoI `it`; every thread of the CTA calls it, and it ends with a barrier.  Warp 0 lanes [0,PW) take the
+// x bins, warp 1 lanes [0,PH) the y bins, warp 2 lanes [0,PD) the z bins.  A RoI outside the batch is empty.
+template <int PW, bool XANY>
+__device__ __forceinline__ void build_cta_tables(CtaTables<PW, XANY> &T, const Item &it, int PH, int PD, int warp,
+                                                 int lane) {
+  constexpr int PWP = CtaTables<PW, XANY>::PWP;
+  const int tid = threadIdx.x;
+  const int role = (warp == 0 && lane < PW) ? 0 : (warp == 1 && lane < PH) ? 1 : (warp == 2 && lane < PD) ? 2 : -1;
+  const Axis ax = role == 1 ? it.axh : role == 2 ? it.axd : it.axw;
+  const int asize = role == 1 ? it.L.H : role == 2 ? it.L.D : it.L.W;
+  int lo = INT_MAX, hi = -1;
+  if (role >= 0 && it.ok) {
+    for (int i = 0; i < ax.S; ++i) {
+      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
+      if (t.valid) lo = min(lo, t.low), hi = max(hi, t.high);
+    }
+  }
+  if (warp < 3) {
+    const int mn = __reduce_min_sync(FULL, role >= 0 ? lo : INT_MAX);
+    const int mx = __reduce_max_sync(FULL, role >= 0 ? hi : -1);
+    if (lane == 0) T.box[warp * 2] = mn, T.box[warp * 2 + 1] = mx;
+  }
+  __syncthreads();
+  T.xmin = T.box[0], T.xmax = T.box[1], T.ymin = T.box[2], T.ymax = T.box[3], T.zmin = T.box[4], T.zmax = T.box[5];
+  T.empty = !it.ok || T.xmax < T.xmin || T.ymax < T.ymin || T.zmax < T.zmin;
+  T.fits = T.empty || ((T.xmax - T.xmin < RXMAX) && (T.ymax - T.ymin < RYMAX) && (T.zmax - T.zmin < RZMAX2));
+  if (!T.empty && T.fits) {
+    const int RX = T.xmax - T.xmin + 1, RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
+    for (int i = tid; i < (RX + (XANY ? 1 : 0)) * PWP; i += kWarps * 32) T.Dx[i] = 0.0f;
+    for (int i = tid; i < RY * PP2; i += kWarps * 32) T.Dy[i] = 0.0f;
+    for (int i = tid; i < RZ * PP2; i += kWarps * 32) T.Dz[i] = 0.0f;
+    if constexpr (XANY)
+      for (int i = tid; i < RX; i += kWarps * 32) T.xany[i] = 0;
+  }
+  __syncthreads();
+  if (!T.empty && T.fits && role >= 0) {
+    float *tab = role == 0 ? T.Dx : role == 1 ? T.Dy : T.Dz;
+    const int stride = role == 0 ? PWP : PP2;
+    const int mn = role == 0 ? T.xmin : role == 1 ? T.ymin : T.zmin;
+    for (int i = 0; i < ax.S; ++i) {
+      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
+      if (t.valid) {
+        tab[(t.low - mn) * stride + lane] += t.h;
+        tab[(t.high - mn) * stride + lane] += t.l;
+        if constexpr (XANY)
+          if (role == 0) T.xany[t.low - mn] = 1, T.xany[t.high - mn] = 1;
+      }
+    }
+    if constexpr (!XANY) {
+      if (role == 0) {
+        T.xlo[lane] = hi >= lo ? lo - T.xmin : 0;
+        T.xhi[lane] = hi >= lo ? hi - T.xmin : -1;
+      }
+    }
+  }
+  __syncthreads();
+}
+
+// A work item's view of a y or z table: its entry j of table row i is t[i * stride + col + j].  Per-warp tables:
+// y = (Dy, 8, 0), z = (Dz, 1, 0).  CTA-shared tables: y = (Dy, PP2, ph0), z = (Dz, PP2, pd).
+struct TabView {
+  const float *t;
+  int stride, col;
+  __device__ __forceinline__ float at(int i, int j) const { return t[i * stride + col + j]; }
+};
+
+// Compact lists of the y rows (of RY, weights in columns [0, rows) of y) and the z slices (of RZ) that carry weight
+// for a work item, built with one ballot per 32 rows / slices.  Returns (ny, nz).
+template <int ROWS>
+__device__ __forceinline__ int2 weighted_rows(TabView y, int rows, int RY, TabView z, int RZ, unsigned char *ylist,
+                                              unsigned char *zlist, int lane) {
+  int ny = 0, nz = 0;
+  for (int y0 = 0; y0 < RY; y0 += 32) {
+    const int yy = y0 + lane;
+    bool a = false;
+    if (yy < RY) {
+#pragma unroll
+      for (int r = 0; r < ROWS; ++r) a |= (r < rows) && y.at(yy, r) != 0.0f;
+    }
+    const unsigned bal = __ballot_sync(FULL, a);
+    if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
+    ny += __popc(bal);
+  }
+#pragma unroll 1  // RZ <= 40: one or two passes; unrolled, this loop lengthens bwd2 by 2-3%
+  for (int z0 = 0; z0 < RZ; z0 += 32) {
+    const int zz = z0 + lane;
+    const bool a = zz < RZ && z.at(zz, 0) != 0.0f;
+    const unsigned bal = __ballot_sync(FULL, a);
+    if (a) zlist[nz + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)zz;
+    nz += __popc(bal);
+  }
+  __syncwarp();
+  return make_int2(ny, nz);
+}
+
+__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
+  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(d), "l"(gmem_src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() {
+  asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory");
+}
+
+// Per-warp constants of the forward ring's x-contraction: for every bin pw its first NXU tap weights (0 past the bin's
+// support, and everywhere when !use) and the offset of its first tap in a ring row.  Ring rows carry two zero-filled
+// pad voxels after the RX real ones, so a zero-weight tap always reads initialised shared memory and tap offsets are
+// compile-time constants.  Returns whether a bin has more than NXU taps.
+template <int PW, int CV, int NXU>
+__device__ __forceinline__ bool x_taps(const float *Dx, const int *xlo, const int *xhi, bool use, int lane,
+                                       int (&soff)[PW], float (&tw)[PW][NXU]) {
+  constexpr int PWP = Tables<PW>::PWP;
+  static_assert(NXU <= 3, "pad voxels cover taps lo+1, lo+2 only");
+  bool long_bins = false;
+#pragma unroll
+  for (int pw = 0; pw < PW; ++pw) {
+    const int lo = use ? xlo[pw] : 0;
+    const int n = use ? xhi[pw] - lo + 1 : 0;
+    long_bins |= n > NXU;
+    soff[pw] = lo * 32 * CV + lane * CV;
+#pragma unroll
+    for (int j = 0; j < NXU; ++j) tw[pw][j] = j < n ? Dx[(lo + j) * PWP + pw] : 0.0f;
+  }
+  return long_bins;
+}
+
+// The cp.async row pipeline of one (pd, ph-group) work item of the forward ring kernels, accumulated into acc.
+// The feature rows the item needs ([xmin..xmax] x 32*CV channels of one (z,y) row) are copied global->shared with
+// 16-byte cp.async (LDGSTS, no register staging) NS-1 rows ahead of the row being contracted.  Rows are visited
+// y-major, z-minor, so that all z slices of one y row are contracted along x back to back and the y-stage runs once
+// per y row.  lists: ylist[40] + zlist[40] bytes, then yoff[40] and zoff[] ints.  pstage / cstage are the ring's
+// producer and consumer slots; every row issued here is consumed here, so a caller may keep them across items.
+// The 16-byte copies need the chunk to lie inside C and be 16-byte aligned: C % 4 == 0 is checked by the
+// dispatcher; a partial last chunk (C not a multiple of 32*CV) copies only the lanes inside C.
+template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, class TB>
+__device__ __forceinline__ void ring_rows(float (&acc)[ROWS][PW][CV], const TB &T, TabView ty, int rows, TabView tz,
+                                          const int (&soff)[PW], const float (&tw)[PW][NXU], bool long_bins,
+                                          const float *fb_roi, int chunk, int C, int H, int W, unsigned char *lists,
+                                          float *ring, int &pstage, int &cstage, int lane) {
+  static_assert(CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
+  constexpr int PWP = Tables<PW>::PWP;
+  constexpr int VOX = 32 * CV;                 // floats per voxel-chunk
+  constexpr int LPV = VOX / 4;                 // lanes (16 B each) per voxel-chunk
+  constexpr int VPI = 32 / LPV;                // voxel-chunks copied per warp instruction
+  constexpr int STRIDE = (RXR + 2) * VOX;      // floats per ring stage (two zero pad voxels)
+  static_assert(LPV <= 32 && VPI >= 1, "voxel chunk wider than a warp copy");
+  unsigned char *ylist = lists, *zlist = lists + 40;
+  int *yoff = reinterpret_cast<int *>(lists + 80);
+  int *zoff = yoff + 40;
+  const int RX = T.xmax - T.xmin + 1;
+  const int2 n = weighted_rows<ROWS>(ty, rows, T.ymax - T.ymin + 1, tz, T.zmax - T.zmin + 1, ylist, zlist, lane);
+  const int ny = n.x, nz = n.y, nrows = ny * nz;
+
+  for (int sidx = 0; sidx < NS; ++sidx) {
+    float *padp = ring + sidx * STRIDE + RX * VOX;
+    for (int i = lane; i < 2 * VOX; i += 32) padp[i] = 0.0f;
+  }
+  __syncwarp();
+
+  // copy geometry: lane -> (voxel within the instruction, 16-byte piece of the voxel chunk)
+  const int cv_v = lane / LPV, cv_p = lane % LPV;
+  const int ch_piece = chunk * VOX + cv_p * 4;             // first channel of this lane's 16 bytes
+  const bool piece_ok = ch_piece + 4 <= C;
+  const long long row_elems = (long long)W * C;
+  const long long slice_elems = (long long)H * row_elems;
+  const float *src0 = fb_roi + ((long long)T.zmin * H + T.ymin) * row_elems + (long long)T.xmin * C + ch_piece +
+                      (long long)cv_v * C;
+  float *dst0 = ring + cv_p * 4 + cv_v * VOX;
+  // row offsets in units of 4 floats (16 B; C % 4 == 0), < 2^31 for any level the dispatcher accepts
+  for (int i = lane; i < nz; i += 32) zoff[i] = (int)(((long long)zlist[i] * slice_elems) >> 2);
+  for (int i = lane; i < ny; i += 32) yoff[i] = (int)(((long long)ylist[i] * row_elems) >> 2);
+  __syncwarp();
+  int pz = 0, py = 0;  // producer cursor: the row to prefetch next
+  auto issue = [&]() {
+    const float *src = src0 + ((long long)(zoff[pz] + yoff[py]) << 2);
+    float *dst = dst0 + pstage * STRIDE;
+    if (piece_ok) {
+#pragma unroll 2
+      for (int v = cv_v; v < RX; v += VPI) {
+        cp_async16(dst, src);
+        dst += VPI * VOX, src += (long long)VPI * C;
+      }
+    }
+    cp_async_commit();
+    if (++pz == nz) pz = 0, ++py;
+    if (++pstage == NS) pstage = 0;
+  };
+#pragma unroll
+  for (int r = 0; r < NS - 1; ++r) {
+    if (r < nrows) issue();
+    else cp_async_commit();
+  }
+  int r = 0;
+  for (int yi = 0; yi < ny; ++yi) {
+    float t1[PW][CV];
+#pragma unroll
+    for (int pw = 0; pw < PW; ++pw)
+#pragma unroll
+      for (int c = 0; c < CV; ++c) t1[pw][c] = 0.0f;
+    for (int zi = 0; zi < nz; ++zi, ++r) {
+      cp_async_wait<NS - 2>();
+      __syncwarp();
+      const float wz = tz.at(zlist[zi], 0);
+      const float *row = ring + cstage * STRIDE;
+      if (++cstage == NS) cstage = 0;
+      float tzw[PW][CV];
+#pragma unroll
+      for (int pw = 0; pw < PW; ++pw) {
+        const float *q = row + soff[pw];
+        // sm_100 packed fp32 (FFMA2 / FMUL2): both channels of the lane in one issue slot; each half is
+        // rounded exactly like the scalar fmul / fma, so the pinned arithmetic is unchanged
+        float2 z2;
+#pragma unroll
+        for (int j = 0; j < NXU; ++j) {
+          const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
+          const float2 w2 = make_float2(tw[pw][j], tw[pw][j]);
+          z2 = j == 0 ? __fmul2_rn(w2, t) : __ffma2_rn(w2, t, z2);
+        }
+        tzw[pw][0] = z2.x, tzw[pw][1] = z2.y;
+      }
+      if (long_bins) {  // one warp-uniform test per row; bins wider than NXU taps are rare
+#pragma unroll
+        for (int pw = 0; pw < PW; ++pw) {
+          const int lo = T.xlo[pw];
+          const int n = T.xhi[pw] - lo + 1;
+          const float *q = row + soff[pw];
+          const float *wq = T.Dx + lo * PWP + pw;
+#pragma unroll 1
+          for (int j = NXU; j < n; ++j) {
+            const float w = wq[j * PWP];
+#pragma unroll
+            for (int c = 0; c < CV; ++c) tzw[pw][c] = fmaf(w, q[j * VOX + c], tzw[pw][c]);
+          }
+        }
+      }
+#pragma unroll
+      for (int pw = 0; pw < PW; ++pw) {
+        const float2 o = __ffma2_rn(make_float2(wz, wz), make_float2(tzw[pw][0], tzw[pw][1]),
+                                    make_float2(t1[pw][0], t1[pw][1]));
+        t1[pw][0] = o.x, t1[pw][1] = o.y;
+      }
+      __syncwarp();
+      if (r + NS - 1 < nrows) issue();
+      else cp_async_commit();
+    }
+    // y-stage, once per feature row index y
+    const int yy = ylist[yi];
+    float wy[ROWS];
+#pragma unroll
+    for (int rr = 0; rr < ROWS; ++rr) wy[rr] = rr < rows ? ty.at(yy, rr) : 0.0f;
+#pragma unroll
+    for (int rr = 0; rr < ROWS; ++rr) {
+      if (wy[rr] != 0.0f) {
+#pragma unroll
+        for (int pw = 0; pw < PW; ++pw) {
+          const float2 o = __ffma2_rn(make_float2(wy[rr], wy[rr]), make_float2(t1[pw][0], t1[pw][1]),
+                                      make_float2(acc[rr][pw][0], acc[rr][pw][1]));
+          acc[rr][pw][0] = o.x, acc[rr][pw][1] = o.y;
+        }
+      }
+    }
+  }
+  cp_async_wait<0>();
+}
+
+// Stage-in of a backward warp's grad_out tile, [c][bin][33] for its CV channel slots (lane = channel column, padded
+// against bank conflicts): 4-byte cp.async copies that transpose on the fly (coalesced global reads), all in flight
+// together and committed as one group.
+template <int CV>
+__device__ __forceinline__ void stage_in_grad(const RoiParams &p, const Item &it, int PW, float *stage, int lane) {
+  const int C = p.C, NB = it.rows * PW;
+  const long long ch_stride = (long long)p.PD * p.PH * PW;
+  // reference index (roi_align_kernel.cu:554-555): pd*PD*PW + ph*PW + pw when bug_compat
+  const long long row_base = p.bug_compat ? ((long long)it.pd * p.PD + it.ph0) * PW
+                                          : ((long long)it.pd * p.PH + it.ph0) * PW;
+  const long long top_total = (long long)p.K * C * ch_stride;
+  const int col_stride = CV * (int)ch_stride;
+#pragma unroll
+  for (int c = 0; c < CV; ++c) {
+    const int cols = min(32, (C - it.chunk * 32 * CV - c + CV - 1) / CV);
+    float *st = stage + c * (NB * 33);
+    const long long g0 = ((long long)it.k * C + (long long)it.chunk * 32 * CV + c) * ch_stride + row_base;
+    long long lim = top_total - g0;  // elements past the end of grad_out: only reachable with bug_compat's row base
+    int total = cols * NB;
+    if (lim < (long long)(cols - 1) * col_stride + NB) total = 0;  // rare: zero the tile, copy nothing out of range
+    if (total < 32 * NB) {
+      for (int i = lane; i < NB * 33; i += 32) st[i] = 0.0f;
+      __syncwarp();
+    }
+    const int ncol = total / NB;
+    unsigned sp = (unsigned)__cvta_generic_to_shared(st + lane * 33);
+    const float *gp = p.grad_out + g0 + lane;
+    // one column (channel run of NB floats) at a time, lanes along the run (cf. copy_out_tile); four columns per
+    // iteration through four address registers and immediate shared offsets: a copy still queued in the memory
+    // pipeline does not hold up the address update of the next one
+    int cl = 0;
+    for (; cl + 4 <= ncol; cl += 4) {
+      const float *g0p = gp, *g1p = gp + col_stride, *g2p = gp + 2 * col_stride, *g3p = gp + 3 * col_stride;
+      if (lane < NB) {
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp), "l"(g0p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+4], [%1], 4;\n" ::"r"(sp), "l"(g1p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+8], [%1], 4;\n" ::"r"(sp), "l"(g2p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+12], [%1], 4;\n" ::"r"(sp), "l"(g3p) : "memory");
+      }
+      if (lane + 32 < NB) {
+        asm volatile("cp.async.ca.shared.global [%0+4224], [%1+128], 4;\n" ::"r"(sp), "l"(g0p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+4228], [%1+128], 4;\n" ::"r"(sp), "l"(g1p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+4232], [%1+128], 4;\n" ::"r"(sp), "l"(g2p) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+4236], [%1+128], 4;\n" ::"r"(sp), "l"(g3p) : "memory");
+      }
+      for (int bin = lane + 64; bin < NB; bin += 32) {
+        const unsigned so = sp + (bin - lane) * 33 * 4;
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(so), "l"(g0p + (bin - lane)) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+4], [%1], 4;\n" ::"r"(so), "l"(g1p + (bin - lane)) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+8], [%1], 4;\n" ::"r"(so), "l"(g2p + (bin - lane)) : "memory");
+        asm volatile("cp.async.ca.shared.global [%0+12], [%1], 4;\n" ::"r"(so), "l"(g3p + (bin - lane)) : "memory");
+      }
+      sp += 16;
+      gp += 4 * col_stride;
+    }
+    for (; cl < ncol; ++cl) {
+      if (lane < NB) asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp), "l"(gp) : "memory");
+      if (lane + 32 < NB)
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + 32 * 33 * 4), "l"(gp + 32) : "memory");
+      for (int bin = lane + 64; bin < NB; bin += 32)
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + (bin - lane) * 33 * 4), "l"(gp + (bin - lane))
+                     : "memory");
+      sp += 4;
+      gp += col_stride;
+    }
+  }
+  cp_async_commit();
+}
+
 
 // Epilogue shared by the forward kernels: acc / count -> padded smem tile [bin][33] (lane = channel, no bank
 // conflicts) -> global [channel][bin] in contiguous runs.  The flattened (channel, bin) walk advances by
@@ -284,39 +648,21 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_fwd_cl_kernel(const R
 }
 
 // ---------------------------------------------------------------------------------------------
-// Forward, channels-last, separable, rows staged through a per-warp cp.async ring.
+// Forward, channels-last, separable, rows staged through a per-warp cp.async ring (ring_rows).
 //
-// Same work split and arithmetic as roi_align3d_fwd_cl_kernel, but the feature rows a warp needs
-// ([xmin..xmax] x 32*CV channels of one (z,y) row) are copied global->shared with 16-byte cp.async
-// (LDGSTS, no register staging) NS-1 rows ahead of the row being contracted.  The loads of the next
-// rows are in flight while the current row is reduced, each voxel of the row is fetched once instead
-// of once per tap, and the register file no longer holds the taps, which raises occupancy.
-// Ring capacity per warp is RXR voxels per row; wider footprints take the literal path.
+// Same work split and arithmetic as roi_align3d_fwd_cl_kernel, but each voxel of a feature row is fetched once
+// instead of once per tap, the loads of the next rows are in flight while the current row is reduced, and the
+// register file no longer holds the taps, which raises occupancy.  Ring capacity per warp is RXR voxels per row;
+// wider footprints take the literal path.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(d), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory");
-}
-
 template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB>
 __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring_kernel(const RoiParams p) {
   using TB = Tables<PW>;
-  constexpr int PWP = TB::PWP;
-  constexpr int VOX = 32 * CV;                 // floats per voxel-chunk
-  constexpr int LPV = VOX / 4;                 // lanes (16 B each) per voxel-chunk
-  constexpr int VPI = 32 / LPV;                // voxel-chunks copied per warp instruction
-  constexpr int STRIDE = (RXR + 2) * VOX;      // floats per ring stage (two zero pad voxels)
-  constexpr int RING = NS * STRIDE;            // floats
+  constexpr int RING = NS * (RXR + 2) * 32 * CV;  // floats
   constexpr int STAGE = ROWS * PW * 33;
   constexpr int LISTS = 384;                   // ylist[40] + zlist[32] bytes (pad to 80) + yoff[40] + zoff[32] ints
   constexpr int RING_OR_STAGE = RING > STAGE ? RING : STAGE;
   constexpr int WARP_FLOATS = (TB::FLOATS + LISTS / 4 + RING_OR_STAGE + 3) / 4 * 4;
-  static_assert(LPV <= 32 && VPI >= 1, "voxel chunk wider than a warp copy");
   extern __shared__ __align__(16) float smem_all[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float *sm = smem_all + warp * WARP_FLOATS;
@@ -336,17 +682,12 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring_kernel
 
   TB T;
   T.bind(sm);
-  unsigned char *ylist = reinterpret_cast<unsigned char *>(sm + ((TB::FLOATS + 3) / 4 * 4));
-  unsigned char *zlist = ylist + 40;
-  int *yoff = reinterpret_cast<int *>(ylist + 80);
-  int *zoff = yoff + 40;
+  unsigned char *lists = reinterpret_cast<unsigned char *>(sm + ((TB::FLOATS + 3) / 4 * 4));
   float *ring = sm + ((TB::FLOATS + 3) / 4 * 4) + LISTS / 4;
   T.empty = true, T.fits = true;
   if (it.ok) build_tables<PW>(T, it, lane);
   const float count = (float)(it.axd.S * it.axh.S * it.axw.S);
   const int RX = T.xmax - T.xmin + 1;
-  // the 16-byte copies need the chunk to lie inside C and be 16-byte aligned: C % 4 == 0 is checked by
-  // the dispatcher; a partial last chunk (C not a multiple of 32*CV) copies only the lanes inside C.
 
   if (it.ok && !T.empty && (!T.fits || RX > RXR)) {
     // footprint larger than the tables / the ring: literal evaluation, uncoalesced stores (rare path)
@@ -363,161 +704,12 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring_kernel
       for (int c = 0; c < CV; ++c) acc[r][w][c] = 0.0f;
 
   if (!T.empty) {
-    // ---- compact lists of the z slices / y rows that carry weight for this (pd, ph-group) ----
-    const int RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
-    int ny = 0, nz = 0;
-    for (int y0 = 0; y0 < RY; y0 += 32) {
-      const int yy = y0 + lane;
-      bool a = false;
-      if (yy < RY) {
-#pragma unroll
-        for (int r = 0; r < ROWS; ++r) a |= T.Dy[yy * 8 + r] != 0.0f;
-      }
-      const unsigned bal = __ballot_sync(FULL, a);
-      if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
-      ny += __popc(bal);
-    }
-    {
-      const bool a = lane < RZ && T.Dz[lane] != 0.0f;
-      const unsigned bal = __ballot_sync(FULL, a);
-      if (a) zlist[__popc(bal & ((1u << lane) - 1u))] = (unsigned char)lane;
-      nz = __popc(bal);
-    }
-    __syncwarp();
-    const int nrows = ny * nz;
-
-    // per-warp constants of the x-contraction: for every bin pw its first NXU taps (weight forced to 0
-    // past the bin's support).  Ring rows carry two zero-filled pad voxels after the RX real ones, so a
-    // zero-weight tap always reads initialised shared memory and tap offsets are compile-time constants.
-    bool long_bins = false;
     int soff[PW];
     float tw[PW][NXU];
-#pragma unroll
-    for (int pw = 0; pw < PW; ++pw) {
-      const int lo = T.xlo[pw];
-      const int n = T.xhi[pw] - lo + 1;
-      long_bins |= n > NXU;
-      soff[pw] = lo * VOX + lane * CV;
-#pragma unroll
-      for (int j = 0; j < NXU; ++j) tw[pw][j] = j < n ? T.Dx[(lo + j) * PWP + pw] : 0.0f;
-    }
-    static_assert(NXU <= 3, "pad voxels cover taps lo+1, lo+2 only");
-    for (int sidx = 0; sidx < NS; ++sidx) {
-      float *padp = ring + sidx * STRIDE + RX * VOX;
-      for (int i = lane; i < 2 * VOX; i += 32) padp[i] = 0.0f;
-    }
-    __syncwarp();
-
-    // copy geometry: lane -> (voxel within the instruction, 16-byte piece of the voxel chunk)
-    const int cv_v = lane / LPV, cv_p = lane % LPV;
-    const int ch_piece = it.chunk * VOX + cv_p * 4;          // first channel of this lane's 16 bytes
-    const bool piece_ok = ch_piece + 4 <= C;
-    // producer cursor (row to prefetch next): rows are visited y-major, z-minor, so that all z slices of
-    // one y row are contracted along x back to back and the y-stage runs once per y row.
-    const long long row_elems = (long long)it.L.W * C;
-    const long long slice_elems = (long long)it.L.H * row_elems;
-    const float *src0 = fb_roi + ((long long)T.zmin * it.L.H + T.ymin) * row_elems + (long long)T.xmin * C + ch_piece +
-                        (long long)cv_v * C;
-    float *dst0 = ring + cv_p * 4 + cv_v * VOX;
-    // row offsets in units of 4 floats (16 B; C % 4 == 0), < 2^31 for any level the dispatcher accepts
-    for (int i = lane; i < nz; i += 32) zoff[i] = (int)(((long long)zlist[i] * slice_elems) >> 2);
-    for (int i = lane; i < ny; i += 32) yoff[i] = (int)(((long long)ylist[i] * row_elems) >> 2);
-    __syncwarp();
-    int pz = 0, py = 0, pstage = 0;
-    auto issue = [&]() {
-      const float *src = src0 + ((long long)(zoff[pz] + yoff[py]) << 2);
-      float *dst = dst0 + pstage * STRIDE;
-      if (piece_ok) {
-#pragma unroll 2
-        for (int v = cv_v; v < RX; v += VPI) {
-          cp_async16(dst, src);
-          dst += VPI * VOX, src += (long long)VPI * C;
-        }
-      }
-      cp_async_commit();
-      if (++pz == nz) pz = 0, ++py;
-      if (++pstage == NS) pstage = 0;
-    };
-#pragma unroll
-    for (int r = 0; r < NS - 1; ++r) {
-      if (r < nrows) issue();
-      else cp_async_commit();
-    }
-    int cstage = 0, r = 0;
-    for (int yi = 0; yi < ny; ++yi) {
-      float t1[PW][CV];
-#pragma unroll
-      for (int pw = 0; pw < PW; ++pw)
-#pragma unroll
-        for (int c = 0; c < CV; ++c) t1[pw][c] = 0.0f;
-      for (int zi = 0; zi < nz; ++zi, ++r) {
-        cp_async_wait<NS - 2>();
-        __syncwarp();
-        const float wz = T.Dz[zlist[zi]];
-        const float *row = ring + cstage * STRIDE;
-        if (++cstage == NS) cstage = 0;
-        float tz[PW][CV];
-#pragma unroll
-        for (int pw = 0; pw < PW; ++pw) {
-          const float *q = row + soff[pw];
-#pragma unroll
-          for (int j = 0; j < NXU; ++j) {
-            float f[CV];
-            if constexpr (CV == 4) {
-              const float4 t = *reinterpret_cast<const float4 *>(q + j * VOX);
-              f[0] = t.x, f[1] = t.y, f[2] = t.z, f[3] = t.w;
-            } else if constexpr (CV == 2) {
-              const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
-              f[0] = t.x, f[1] = t.y;
-            } else {
-              f[0] = q[j * VOX];
-            }
-#pragma unroll
-            for (int c = 0; c < CV; ++c) tz[pw][c] = j == 0 ? tw[pw][0] * f[c] : fmaf(tw[pw][j], f[c], tz[pw][c]);
-          }
-        }
-        if (long_bins) {  // one warp-uniform test per row; bins wider than NXU taps are rare
-#pragma unroll
-          for (int pw = 0; pw < PW; ++pw) {
-            const int lo = T.xlo[pw];
-            const int n = T.xhi[pw] - lo + 1;
-            const float *q = row + soff[pw];
-            const float *wq = T.Dx + lo * PWP + pw;
-#pragma unroll 1
-            for (int j = NXU; j < n; ++j) {
-              const float w = wq[j * PWP];
-#pragma unroll
-              for (int c = 0; c < CV; ++c) tz[pw][c] = fmaf(w, q[j * VOX + c], tz[pw][c]);
-            }
-          }
-        }
-#pragma unroll
-        for (int pw = 0; pw < PW; ++pw)
-#pragma unroll
-          for (int c = 0; c < CV; ++c) t1[pw][c] = fmaf(wz, tz[pw][c], t1[pw][c]);
-        __syncwarp();
-        if (r + NS - 1 < nrows) issue();
-        else cp_async_commit();
-      }
-      // y-stage, once per feature row index y
-      const int yy = ylist[yi];
-      float wy[8];
-      {
-        const float4 a = *reinterpret_cast<const float4 *>(T.Dy + yy * 8);
-        const float4 b4 = *reinterpret_cast<const float4 *>(T.Dy + yy * 8 + 4);
-        wy[0] = a.x, wy[1] = a.y, wy[2] = a.z, wy[3] = a.w, wy[4] = b4.x, wy[5] = b4.y, wy[6] = b4.z, wy[7] = b4.w;
-      }
-#pragma unroll
-      for (int rr = 0; rr < ROWS; ++rr) {
-        if (wy[rr] != 0.0f) {
-#pragma unroll
-          for (int pw = 0; pw < PW; ++pw)
-#pragma unroll
-            for (int c = 0; c < CV; ++c) acc[rr][pw][c] = fmaf(wy[rr], t1[pw][c], acc[rr][pw][c]);
-        }
-      }
-    }
-    cp_async_wait<0>();
+    const bool long_bins = x_taps<PW, CV, NXU>(T.Dx, T.xlo, T.xhi, true, lane, soff, tw);
+    int pstage = 0, cstage = 0;
+    ring_rows<PW, ROWS, CV, NXU, NS, RXR>(acc, T, TabView{T.Dy, 8, 0}, ROWS, TabView{T.Dz, 1, 0}, soff, tw, long_bins,
+                                          fb_roi, it.chunk, C, it.L.H, it.L.W, lists, ring, pstage, cstage, lane);
   }
 
   // ---- epilogue: divide by the sample count, transpose through smem, stream out ----
@@ -531,9 +723,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring_kernel
 // Shared-memory layout of the ring2 kernel, shared by the kernel and its launcher.
 template <int PW, int ROWS, int CV, int NS, int RXR>
 struct Ring2Layout {
-  static constexpr int VOX = 32 * CV;
-  static constexpr int STRIDE = (RXR + 2) * VOX;
-  static constexpr int RING = NS * STRIDE;
+  static constexpr int RING = NS * (RXR + 2) * 32 * CV;
   static constexpr int STAGE = ROWS * PW * 33;
   // bytes: ylist[40] + zlist[40] bytes, yoff[40] + zoff[40] ints (0..400).  The 64 bytes at 416 are spare; the
   // size is kept so that the shared-memory footprint, and with it the occupancy, stay as measured.
@@ -541,9 +731,7 @@ struct Ring2Layout {
   static constexpr int ALIGN = 4;  // floats
   static constexpr int RING_OR_STAGE = RING > STAGE ? RING : STAGE;
   static constexpr int WARP_FLOATS = (LISTS / 4 + RING_OR_STAGE + ALIGN - 1) / ALIGN * ALIGN;
-  static constexpr int SH_FLOATS = RXMAX * Tables<PW>::PWP + RYMAX * 16 + 40 * 16 + 32 + 3 * 32 * 2 + 16;
-  static constexpr int SH_PAD = (SH_FLOATS + ALIGN - 1) / ALIGN * ALIGN;
-  static constexpr size_t BYTES = ((size_t)SH_PAD + (size_t)kWarps * WARP_FLOATS) * sizeof(float);
+  static constexpr size_t BYTES = ((size_t)CtaTables<PW, false>::FLOATS + (size_t)kWarps * WARP_FLOATS) * sizeof(float);
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -552,33 +740,15 @@ struct Ring2Layout {
 // parallel (x, y and z bins) instead of once per warp, and sit once in shared memory.  Everything after
 // the table build is the per-warp pipeline of roi_align3d_fwd_ring_kernel.
 // ---------------------------------------------------------------------------------------------
-constexpr int RZMAX2 = 40;
-constexpr int PP2 = 16;  // padded row length of the CTA-shared y / z tables (PH, PD <= 16)
 template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB, bool MULTI>
 __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kernel(const RoiParams p) {
-  static_assert(CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
-  using TB = Tables<PW>;
+  using ST = CtaTables<PW, false>;
   using LY = Ring2Layout<PW, ROWS, CV, NS, RXR>;
-  constexpr int PWP = TB::PWP;
-  constexpr int VOX = 32 * CV;                 // floats per voxel-chunk
-  constexpr int LPV = VOX / 4;                 // lanes (16 B each) per voxel-chunk
-  constexpr int VPI = 32 / LPV;                // voxel-chunks copied per warp instruction
-  constexpr int STRIDE = LY::STRIDE;           // floats per ring stage (two zero pad voxels)
-  constexpr int LISTS = LY::LISTS;             // ylist[40] + zlist[40] bytes + yoff[40] + zoff[40] ints
-  constexpr int WARP_FLOATS = LY::WARP_FLOATS;
-  static_assert(LPV <= 32 && VPI >= 1, "voxel chunk wider than a warp copy");
   extern __shared__ __align__(128) float smem_r2[];
-  float *smem_all = smem_r2;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
-  // ---- CTA-shared per-RoI tables (all warps of a CTA work on the same RoI) ----
-  float *SDx = smem_all;                       // [x - xmin][PWP]
-  float *SDy = SDx + RXMAX * PWP;              // [y - ymin][PP2], all PH rows
-  float *SDz = SDy + RYMAX * PP2;              // [z - zmin][PP2], all PD slices
-  int *Sxlo = reinterpret_cast<int *>(SDz + RZMAX2 * PP2);
-  int *Sxhi = Sxlo + 16;
-  int *Srng = Sxhi + 16;                       // [3 axes][32 roles][lo, hi]
-  int *Sbox = Srng + 3 * 32 * 2;               // xmin, xmax, ymin, ymax, zmin, zmax
-  float *sm = smem_all + LY::SH_PAD + warp * WARP_FLOATS;
+  ST T;  // CTA-shared per-RoI tables (all warps of a CTA work on the same RoI)
+  T.bind(smem_r2);
+  float *sm = smem_r2 + ST::FLOATS + warp * LY::WARP_FLOATS;
 
   // CTA -> (RoI k, group of kWarps * p.items_per_warp consecutive sub-items); warp w takes sub-items
   // first + w, first + w + kWarps, ...  Sub-item order: channel chunk fastest, then pd, then ph-group, so with
@@ -587,98 +757,25 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kerne
   const int items_per_warp = MULTI ? p.items_per_warp : 1;
   const int first = (blockIdx.x - k * p.ctas_per_roi) * kWarps * items_per_warp;
   Item it;
-  {
-    it.k = k;
-    it.krow = p.out_rows != nullptr ? __ldg(p.out_rows + k) : k;
-    it.pd = 0, it.chunk = 0, it.ph0 = 0, it.rows = 0;
-    float r[7];
-#pragma unroll
-    for (int i = 0; i < 7; ++i) r[i] = __ldg(p.rois + (long long)k * 7 + i);
-    it.lvl = p.num_levels > 1 ? roi_level(r, p.num_levels, p.inv_finest) : 0;
-    it.L = p.lv[it.lvl];
-    it.b = (int)r[0];
-    it.ok = it.b >= 0 && it.b < p.B;
-    it.axw = axis_setup(r[1], r[3], it.L.scale, p.PW, p.sample_num);
-    it.axh = axis_setup(r[2], r[4], it.L.scale, p.PH, p.sample_num);
-    it.axd = axis_setup(r[5], r[6], it.L.scale_d, p.PD, p.sample_num);
-  }
+  it.krow = p.out_rows != nullptr ? __ldg(p.out_rows + k) : k;
+  it.pd = 0, it.chunk = 0, it.ph0 = 0, it.rows = 0;
+  roi_geometry(p, k, it);
   const int C = p.C;
   if (p.lvls_out != nullptr && blockIdx.x == k * p.ctas_per_roi && tid == 0) p.lvls_out[k] = it.lvl;
 
-  // role threads: warp 0 lanes [0,PW) -> x bins, warp 1 lanes [0,PH) -> y bins, warp 2 lanes [0,PD) -> z bins
-  const int role = (warp == 0 && lane < PW) ? 0 : (warp == 1 && lane < p.PH) ? 1 : (warp == 2 && lane < p.PD) ? 2 : -1;
-  const Axis ax = role == 1 ? it.axh : role == 2 ? it.axd : it.axw;
-  const int asize = role == 1 ? it.L.H : role == 2 ? it.L.D : it.L.W;
-  int lo = INT_MAX, hi = -1;
-  if (role >= 0 && it.ok) {
-    for (int i = 0; i < ax.S; ++i) {
-      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
-      if (t.valid) lo = min(lo, t.low), hi = max(hi, t.high);
-    }
-  }
-  if (warp < 3) {
-    const int mn = __reduce_min_sync(FULL, role >= 0 ? lo : INT_MAX);
-    const int mx = __reduce_max_sync(FULL, role >= 0 ? hi : -1);
-    if (lane == 0) Sbox[warp * 2] = mn, Sbox[warp * 2 + 1] = mx;
-  }
-  __syncthreads();
-  TB T;
-  T.Dx = SDx, T.xlo = Sxlo, T.xhi = Sxhi;
-  T.xmin = Sbox[0], T.xmax = Sbox[1], T.ymin = Sbox[2], T.ymax = Sbox[3], T.zmin = Sbox[4], T.zmax = Sbox[5];
-  T.empty = !it.ok || T.xmax < T.xmin || T.ymax < T.ymin || T.zmax < T.zmin;
-  T.fits = T.empty || ((T.xmax - T.xmin < RXMAX) && (T.ymax - T.ymin < RYMAX) && (T.zmax - T.zmin < RZMAX2));
-  const int RX = T.xmax - T.xmin + 1;
-  if (!T.empty && T.fits) {
-    const int RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
-    for (int i = tid; i < RX * PWP; i += kWarps * 32) SDx[i] = 0.0f;
-    for (int i = tid; i < RY * PP2; i += kWarps * 32) SDy[i] = 0.0f;
-    for (int i = tid; i < RZ * PP2; i += kWarps * 32) SDz[i] = 0.0f;
-  }
-  __syncthreads();
-  if (!T.empty && T.fits && role >= 0) {
-    float *tab = role == 0 ? SDx : role == 1 ? SDy : SDz;
-    const int stride = role == 0 ? PWP : PP2;
-    const int mn = role == 0 ? T.xmin : role == 1 ? T.ymin : T.zmin;
-    for (int i = 0; i < ax.S; ++i) {
-      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
-      if (t.valid) {
-        tab[(t.low - mn) * stride + lane] += t.h;
-        tab[(t.high - mn) * stride + lane] += t.l;
-      }
-    }
-    if (role == 0) {
-      Sxlo[lane] = hi >= lo ? lo - T.xmin : 0;
-      Sxhi[lane] = hi >= lo ? hi - T.xmin : -1;
-    }
-  }
-  __syncthreads();
+  build_cta_tables(T, it, p.PH, p.PD, warp, lane);
   // no block-level barriers below: warps run their sub-items independently
 
-  unsigned char *ylist = reinterpret_cast<unsigned char *>(sm);
-  unsigned char *zlist = ylist + 40;
-  int *yoff = reinterpret_cast<int *>(ylist + 80);
-  int *zoff = yoff + 40;
-  float *ring = sm + LISTS / 4;
+  unsigned char *lists = reinterpret_cast<unsigned char *>(sm);
+  float *ring = sm + LY::LISTS / 4;
   const float count = (float)(it.axd.S * it.axh.S * it.axw.S);
+  const int RX = T.xmax - T.xmin + 1;
   const bool use_ring = !T.empty && T.fits && RX <= RXR;
 
-  // per-warp constants of the x-contraction (RoI-level, shared by all sub-items of the warp): for every bin pw
-  // its first NXU taps (weight forced to 0 past the bin's support).  Ring rows carry two zero-filled pad voxels
-  // after the RX real ones, so a zero-weight tap always reads initialised shared memory and tap offsets are
-  // compile-time constants.
-  bool long_bins = false;
+  // x-contraction constants are RoI-level: shared by all sub-items of the warp
   int soff[PW];
   float tw[PW][NXU];
-  static_assert(NXU <= 3, "pad voxels cover taps lo+1, lo+2 only");
-#pragma unroll
-  for (int pw = 0; pw < PW; ++pw) {
-    const int lo = use_ring ? T.xlo[pw] : 0;
-    const int n = use_ring ? T.xhi[pw] - lo + 1 : 0;
-    long_bins |= n > NXU;
-    soff[pw] = lo * VOX + lane * CV;
-#pragma unroll
-    for (int j = 0; j < NXU; ++j) tw[pw][j] = j < n ? T.Dx[(lo + j) * PWP + pw] : 0.0f;
-  }
+  const bool long_bins = x_taps<PW, CV, NXU>(T.Dx, T.xlo, T.xhi, use_ring, lane, soff, tw);
   int pstage = 0, cstage = 0;  // ring cursors persist across sub-items (every issued row is consumed)
 
   for (int g = 0; g < items_per_warp; ++g) {
@@ -699,8 +796,6 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kerne
   const long long vox = (long long)it.L.D * it.L.H * it.L.W;
   const float *fb_roi = it.L.feats + (long long)(it.ok ? it.b : 0) * vox * C;
   const float *fb = fb_roi + c_base;
-  // the 16-byte copies need the chunk to lie inside C and be 16-byte aligned: C % 4 == 0 is checked by
-  // the dispatcher; a partial last chunk (C not a multiple of 32*CV) copies only the lanes inside C.
 
   if (!T.empty && (!T.fits || RX > RXR)) {
     // footprint larger than the tables / the ring: literal evaluation, uncoalesced stores (rare path)
@@ -716,144 +811,10 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kerne
 #pragma unroll
       for (int c = 0; c < CV; ++c) acc[r][w][c] = 0.0f;
 
-  if (!T.empty) {
-    // ---- compact lists of the z slices / y rows that carry weight for this (pd, ph-group) ----
-    const int RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
-    int ny = 0, nz = 0;
-    for (int y0 = 0; y0 < RY; y0 += 32) {
-      const int yy = y0 + lane;
-      bool a = false;
-      if (yy < RY) {
-#pragma unroll
-        for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP2 + it.ph0 + r] != 0.0f;
-      }
-      const unsigned bal = __ballot_sync(FULL, a);
-      if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
-      ny += __popc(bal);
-    }
-    for (int z0 = 0; z0 < RZ; z0 += 32) {
-      const int zz = z0 + lane;
-      const bool a = zz < RZ && SDz[zz * PP2 + it.pd] != 0.0f;
-      const unsigned bal = __ballot_sync(FULL, a);
-      if (a) zlist[nz + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)zz;
-      nz += __popc(bal);
-    }
-    __syncwarp();
-    const int nrows = ny * nz;
-
-    for (int sidx = 0; sidx < NS; ++sidx) {
-      float *padp = ring + sidx * STRIDE + RX * VOX;
-      for (int i = lane; i < 2 * VOX; i += 32) padp[i] = 0.0f;
-    }
-    __syncwarp();
-
-    // copy geometry: lane -> (voxel within the instruction, 16-byte piece of the voxel chunk)
-    const int cv_v = lane / LPV, cv_p = lane % LPV;
-    const int ch_piece = it.chunk * VOX + cv_p * 4;          // first channel of this lane's 16 bytes
-    const bool piece_ok = ch_piece + 4 <= C;
-    // producer cursor (row to prefetch next): rows are visited y-major, z-minor, so that all z slices of
-    // one y row are contracted along x back to back and the y-stage runs once per y row.
-    const long long row_elems = (long long)it.L.W * C;
-    const long long slice_elems = (long long)it.L.H * row_elems;
-    const float *src0 = fb_roi + ((long long)T.zmin * it.L.H + T.ymin) * row_elems + (long long)T.xmin * C + ch_piece +
-                        (long long)cv_v * C;
-    float *dst0 = ring + cv_p * 4 + cv_v * VOX;
-    // row offsets in units of 4 floats (16 B; C % 4 == 0), < 2^31 for any level the dispatcher accepts
-    for (int i = lane; i < nz; i += 32) zoff[i] = (int)(((long long)zlist[i] * slice_elems) >> 2);
-    for (int i = lane; i < ny; i += 32) yoff[i] = (int)(((long long)ylist[i] * row_elems) >> 2);
-    __syncwarp();
-    int pz = 0, py = 0;
-    auto issue = [&]() {
-      const float *src = src0 + ((long long)(zoff[pz] + yoff[py]) << 2);
-      float *dst = dst0 + pstage * STRIDE;
-      if (piece_ok) {
-#pragma unroll 2
-        for (int v = cv_v; v < RX; v += VPI) {
-          cp_async16(dst, src);
-          dst += VPI * VOX, src += (long long)VPI * C;
-        }
-      }
-      cp_async_commit();
-      if (++pz == nz) pz = 0, ++py;
-      if (++pstage == NS) pstage = 0;
-    };
-#pragma unroll
-    for (int r = 0; r < NS - 1; ++r) {
-      if (r < nrows) issue();
-      else cp_async_commit();
-    }
-    int r = 0;
-    for (int yi = 0; yi < ny; ++yi) {
-      float t1[PW][CV];
-#pragma unroll
-      for (int pw = 0; pw < PW; ++pw)
-#pragma unroll
-        for (int c = 0; c < CV; ++c) t1[pw][c] = 0.0f;
-      for (int zi = 0; zi < nz; ++zi, ++r) {
-        cp_async_wait<NS - 2>();
-        __syncwarp();
-        const float wz = SDz[zlist[zi] * PP2 + it.pd];
-        const float *row = ring + cstage * STRIDE;
-        if (++cstage == NS) cstage = 0;
-        float tz[PW][CV];
-#pragma unroll
-        for (int pw = 0; pw < PW; ++pw) {
-          const float *q = row + soff[pw];
-          // sm_100 packed fp32 (FFMA2 / FMUL2): both channels of the lane in one issue slot; each half is
-          // rounded exactly like the scalar fmul / fma, so the pinned arithmetic is unchanged
-          float2 z2;
-#pragma unroll
-          for (int j = 0; j < NXU; ++j) {
-            const float2 t = *reinterpret_cast<const float2 *>(q + j * VOX);
-            const float2 w2 = make_float2(tw[pw][j], tw[pw][j]);
-            z2 = j == 0 ? __fmul2_rn(w2, t) : __ffma2_rn(w2, t, z2);
-          }
-          tz[pw][0] = z2.x, tz[pw][1] = z2.y;
-        }
-        if (long_bins) {  // one warp-uniform test per row; bins wider than NXU taps are rare
-#pragma unroll
-          for (int pw = 0; pw < PW; ++pw) {
-            const int lo = T.xlo[pw];
-            const int n = T.xhi[pw] - lo + 1;
-            const float *q = row + soff[pw];
-            const float *wq = T.Dx + lo * PWP + pw;
-#pragma unroll 1
-            for (int j = NXU; j < n; ++j) {
-              const float w = wq[j * PWP];
-#pragma unroll
-              for (int c = 0; c < CV; ++c) tz[pw][c] = fmaf(w, q[j * VOX + c], tz[pw][c]);
-            }
-          }
-        }
-#pragma unroll
-        for (int pw = 0; pw < PW; ++pw) {
-          const float2 o = __ffma2_rn(make_float2(wz, wz), make_float2(tz[pw][0], tz[pw][1]),
-                                      make_float2(t1[pw][0], t1[pw][1]));
-          t1[pw][0] = o.x, t1[pw][1] = o.y;
-        }
-        __syncwarp();
-        if (r + NS - 1 < nrows) issue();
-        else cp_async_commit();
-      }
-      // y-stage, once per feature row index y
-      const int yy = ylist[yi];
-      float wy[ROWS];
-#pragma unroll
-      for (int rr = 0; rr < ROWS; ++rr) wy[rr] = rr < it.rows ? SDy[yy * PP2 + it.ph0 + rr] : 0.0f;
-#pragma unroll
-      for (int rr = 0; rr < ROWS; ++rr) {
-        if (wy[rr] != 0.0f) {
-#pragma unroll
-          for (int pw = 0; pw < PW; ++pw) {
-            const float2 o = __ffma2_rn(make_float2(wy[rr], wy[rr]), make_float2(t1[pw][0], t1[pw][1]),
-                                        make_float2(acc[rr][pw][0], acc[rr][pw][1]));
-            acc[rr][pw][0] = o.x, acc[rr][pw][1] = o.y;
-          }
-        }
-      }
-    }
-    cp_async_wait<0>();
-  }
+  if (!T.empty)
+    ring_rows<PW, ROWS, CV, NXU, NS, RXR>(acc, T, TabView{T.Dy, PP2, it.ph0}, it.rows, TabView{T.Dz, PP2, it.pd}, soff,
+                                          tw, long_bins, fb_roi, it.chunk, C, it.L.H, it.L.W, lists, ring, pstage,
+                                          cstage, lane);
 
   // ---- epilogue: divide by the sample count, transpose through smem, stream out ----
   const int NB = it.rows * PW;
@@ -872,8 +833,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_fwd_ring2_kerne
 // Literal backward of a warp's whole (pd, ph-group) tile, out of line (see literal_tile_fwd).
 template <int CV>
 __device__ __noinline__ void literal_tile_bwd(const Item &it, float *gb, int C, int PW, const float *stage, int lane,
-                                              bool active, float inv_unused) {
-  (void)inv_unused;
+                                              bool active) {
   for (int r = 0; r < it.rows; ++r)
     for (int pw = 0; pw < PW; ++pw) {
       float top[CV];
@@ -915,56 +875,15 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
   float *stage = sm + ((TB::FLOATS + 3) / 4 * 4) + LISTS / 4;
   float *ux = stage;  // aliases the stage-in tile once the gradients are in registers
 
-  // ---- stage-in of this warp's grad_out tile: 4-byte cp.async copies that transpose on the fly
-  //      (coalesced global reads -> [bin][33] padded smem), all in flight together ----
   const int NB = it.rows * PW;
-  const long long ch_stride = (long long)p.PD * p.PH * PW;
-  // reference index (roi_align_kernel.cu:554-555): pd*PD*PW + ph*PW + pw when bug_compat
-  const long long row_base = p.bug_compat ? ((long long)it.pd * p.PD + it.ph0) * PW
-                                          : ((long long)it.pd * p.PH + it.ph0) * PW;
-  const long long top_total = (long long)p.K * C * ch_stride;
-  {
-    const int col_stride = CV * (int)ch_stride;
-#pragma unroll
-    for (int c = 0; c < CV; ++c) {
-      const int cols = min(32, (C - it.chunk * 32 * CV - c + CV - 1) / CV);
-      float *st = stage + c * (NB * 33);
-      const long long g0 = ((long long)it.k * C + (long long)it.chunk * 32 * CV + c) * ch_stride + row_base;
-      // elements past the end of grad_out can only be addressed with bug_compat's wrong row base
-      long long lim = top_total - g0;
-      int total = cols * NB;
-      if (lim < (long long)(cols - 1) * col_stride + NB) {
-        total = 0;  // rare (last RoI / channel with bug_compat): zero the tile, copy nothing out of range
-      }
-      if (total < 32 * NB) {
-        for (int i = lane; i < NB * 33; i += 32) st[i] = 0.0f;
-        __syncwarp();
-      }
-      // one column (channel run of NB floats) at a time, lanes along the run (cf. copy_out_tile)
-      const int ncol = total / NB;
-      unsigned sp = (unsigned)__cvta_generic_to_shared(st + lane * 33);
-      const float *gp = p.grad_out + g0 + lane;
-#pragma unroll 4
-      for (int cl = 0; cl < ncol; ++cl) {
-        if (lane < NB) asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp), "l"(gp) : "memory");
-        if (lane + 32 < NB)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + 32 * 33 * 4), "l"(gp + 32) : "memory");
-        for (int bin = lane + 64; bin < NB; bin += 32)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + (bin - lane) * 33 * 4), "l"(gp + (bin - lane))
-                       : "memory");
-        sp += 4;
-        gp += col_stride;
-      }
-    }
-    cp_async_commit();
-  }
+  stage_in_grad<CV>(p, it, PW, stage, lane);
   build_tables<PW>(T, it, lane);  // overlaps the copies
   cp_async_wait<0>();
   __syncwarp();
   if (T.empty) return;
   const int RX = T.xmax - T.xmin + 1;
   if (!T.fits || RX > RXR) {
-    literal_tile_bwd<CV>(it, gb, C, PW, stage, lane, active, 0.0f);
+    literal_tile_bwd<CV>(it, gb, C, PW, stage, lane, active);
     return;
   }
   // gradients to registers, scaled once by 1/count (reference: top*w/count per corner, :600-608)
@@ -978,7 +897,8 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
       for (int pw = 0; pw < PW; ++pw)
         g[r][pw][c] = r < it.rows ? stage[(c * NB + r * PW + pw) * 33 + lane] * inv : 0.0f;
 
-  // compact lists of the y rows / z slices that carry weight (as in the forward)
+  // compact lists of the y rows / z slices that carry weight, the z slices in one ballot (RZ <= 32).  Kept here rather
+  // than in weighted_rows: through the helper this kernel ran 6-8% slower (7-wide, B200 at 1000 W).
   const int RY = T.ymax - T.ymin + 1, RZ = T.zmax - T.zmin + 1;
   int ny = 0, nz = 0;
   for (int y0 = 0; y0 < RY; y0 += 32) {
@@ -1100,20 +1020,16 @@ __global__ void __launch_bounds__(kWarps * 32) roi_align3d_bwd_cl_kernel(const R
 template <int PW, int ROWS, int CV, int MINB>
 __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(const RoiParams p) {
   static_assert(CV == 2, "packed f32x2 arithmetic pairs the two channels of a lane");
-  using TB = Tables<PW>;
-  constexpr int PWP = TB::PWP;
+  using ST = CtaTables<PW, true>;
+  constexpr int PWP = ST::PWP;
   constexpr int STAGE = CV * ROWS * PW * 33;     // all CV slots of the grad tile at once
   constexpr int LISTS = 80;
   constexpr int WARP_FLOATS = (LISTS / 4 + STAGE + 3) / 4 * 4;
-  constexpr int SH_FLOATS = (RXMAX + 1) * PWP + RYMAX * PP2 + RZMAX2 * PP2 + RXMAX + 8;
   extern __shared__ __align__(16) float smem_all[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
-  float *SDx = smem_all;                         // [x - xmin][PWP] (+1 row: the paired x loop may read one past RX)
-  float *SDy = SDx + (RXMAX + 1) * PWP;          // [y - ymin][PP2]
-  float *SDz = SDy + RYMAX * PP2;                // [z - zmin][PP2]
-  int *Sxany = reinterpret_cast<int *>(SDz + RZMAX2 * PP2);
-  int *Sbox = Sxany + RXMAX;
-  float *sm = smem_all + ((SH_FLOATS + 3) / 4 * 4) + warp * WARP_FLOATS;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  ST T;
+  T.bind(smem_all);
+  float *sm = smem_all + ST::FLOATS + warp * WARP_FLOATS;
 
   const int k = blockIdx.x / p.ctas_per_roi;
   const int sub = (blockIdx.x - k * p.ctas_per_roi) * kWarps + warp;
@@ -1125,20 +1041,10 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
     item /= (unsigned)p.nphg;
     it.pd = (int)(item % (unsigned)p.PD);
     it.chunk = (int)(item / (unsigned)p.PD);
-    it.k = k;
     it.ph0 = (int)phg * ROWS;
     it.rows = min(ROWS, p.PH - it.ph0);
-    float r[7];
-#pragma unroll
-    for (int i = 0; i < 7; ++i) r[i] = __ldg(p.rois + (long long)k * 7 + i);
-    it.lvl = p.num_levels > 1 ? roi_level(r, p.num_levels, p.inv_finest) : 0;
-    it.L = p.lv[it.lvl];
-    it.b = (int)r[0];
-    it.ok = it.b >= 0 && it.b < p.B;
-    it.axw = axis_setup(r[1], r[3], it.L.scale, p.PW, p.sample_num);
-    it.axh = axis_setup(r[2], r[4], it.L.scale, p.PH, p.sample_num);
-    it.axd = axis_setup(r[5], r[6], it.L.scale_d, p.PD, p.sample_num);
   }
+  roi_geometry(p, k, it);
   if (!it.ok) return;  // same RoI for the whole CTA: uniform exit before any barrier
   const int C = p.C;
   int c_base = (it.chunk * 32 + lane) * CV;
@@ -1150,121 +1056,19 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
   unsigned char *zlist = ylist + 40;
   float *stage = sm + LISTS / 4;
 
-  // ---- stage-in of this warp's grad_out tile (see roi_align3d_bwd_cl_kernel), issued before the table build ----
+  // this warp's grad_out tile is in flight while the CTA builds the tables
   const int NB = it.rows * PW;
-  if (valid) {
-    const long long ch_stride = (long long)p.PD * p.PH * PW;
-    // reference index (roi_align_kernel.cu:554-555): pd*PD*PW + ph*PW + pw when bug_compat
-    const long long row_base = p.bug_compat ? ((long long)it.pd * p.PD + it.ph0) * PW
-                                            : ((long long)it.pd * p.PH + it.ph0) * PW;
-    const long long top_total = (long long)p.K * C * ch_stride;
-    const int col_stride = CV * (int)ch_stride;
-#pragma unroll
-    for (int c = 0; c < CV; ++c) {
-      const int cols = min(32, (C - it.chunk * 32 * CV - c + CV - 1) / CV);
-      float *st = stage + c * (NB * 33);
-      const long long g0 = ((long long)it.k * C + (long long)it.chunk * 32 * CV + c) * ch_stride + row_base;
-      long long lim = top_total - g0;  // elements past the end of grad_out: only reachable with bug_compat's row base
-      int total = cols * NB;
-      if (lim < (long long)(cols - 1) * col_stride + NB) total = 0;
-      if (total < 32 * NB) {
-        for (int i = lane; i < NB * 33; i += 32) st[i] = 0.0f;
-        __syncwarp();
-      }
-      const int ncol = total / NB;
-      unsigned sp = (unsigned)__cvta_generic_to_shared(st + lane * 33);
-      const float *gp = p.grad_out + g0 + lane;
-      // four columns per iteration through four address registers and immediate shared offsets: a copy still
-      // queued in the memory pipeline does not hold up the address update of the next one
-      int cl = 0;
-      for (; cl + 4 <= ncol; cl += 4) {
-        const float *g0p = gp, *g1p = gp + col_stride, *g2p = gp + 2 * col_stride, *g3p = gp + 3 * col_stride;
-        if (lane < NB) {
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp), "l"(g0p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+4], [%1], 4;\n" ::"r"(sp), "l"(g1p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+8], [%1], 4;\n" ::"r"(sp), "l"(g2p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+12], [%1], 4;\n" ::"r"(sp), "l"(g3p) : "memory");
-        }
-        if (lane + 32 < NB) {
-          asm volatile("cp.async.ca.shared.global [%0+4224], [%1+128], 4;\n" ::"r"(sp), "l"(g0p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+4228], [%1+128], 4;\n" ::"r"(sp), "l"(g1p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+4232], [%1+128], 4;\n" ::"r"(sp), "l"(g2p) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+4236], [%1+128], 4;\n" ::"r"(sp), "l"(g3p) : "memory");
-        }
-        for (int bin = lane + 64; bin < NB; bin += 32) {
-          const unsigned so = sp + (bin - lane) * 33 * 4;
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(so), "l"(g0p + (bin - lane)) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+4], [%1], 4;\n" ::"r"(so), "l"(g1p + (bin - lane)) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+8], [%1], 4;\n" ::"r"(so), "l"(g2p + (bin - lane)) : "memory");
-          asm volatile("cp.async.ca.shared.global [%0+12], [%1], 4;\n" ::"r"(so), "l"(g3p + (bin - lane)) : "memory");
-        }
-        sp += 16;
-        gp += 4 * col_stride;
-      }
-      for (; cl < ncol; ++cl) {
-        if (lane < NB) asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp), "l"(gp) : "memory");
-        if (lane + 32 < NB)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + 32 * 33 * 4), "l"(gp + 32) : "memory");
-        for (int bin = lane + 64; bin < NB; bin += 32)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(sp + (bin - lane) * 33 * 4), "l"(gp + (bin - lane))
-                       : "memory");
-        sp += 4;
-        gp += col_stride;
-      }
-    }
-    cp_async_commit();
-  }
-
-  // ---- CTA-shared tables: warp 0 lanes [0,PW) -> x bins, warp 1 lanes [0,PH) -> y bins, warp 2 lanes [0,PD) -> z bins
-  const int role = (warp == 0 && lane < PW) ? 0 : (warp == 1 && lane < p.PH) ? 1 : (warp == 2 && lane < p.PD) ? 2 : -1;
-  const Axis ax = role == 1 ? it.axh : role == 2 ? it.axd : it.axw;
-  const int asize = role == 1 ? it.L.H : role == 2 ? it.L.D : it.L.W;
-  int lo = INT_MAX, hi = -1;
-  if (role >= 0) {
-    for (int i = 0; i < ax.S; ++i) {
-      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
-      if (t.valid) lo = min(lo, t.low), hi = max(hi, t.high);
-    }
-  }
-  if (warp < 3) {
-    const int mn = __reduce_min_sync(FULL, role >= 0 ? lo : INT_MAX);
-    const int mx = __reduce_max_sync(FULL, role >= 0 ? hi : -1);
-    if (lane == 0) Sbox[warp * 2] = mn, Sbox[warp * 2 + 1] = mx;
-  }
-  __syncthreads();
-  const int xmin = Sbox[0], xmax = Sbox[1], ymin = Sbox[2], ymax = Sbox[3], zmin = Sbox[4], zmax = Sbox[5];
-  const bool empty = xmax < xmin || ymax < ymin || zmax < zmin;
-  const bool fits = empty || ((xmax - xmin < RXMAX) && (ymax - ymin < RYMAX) && (zmax - zmin < RZMAX2));
-  const int RX = xmax - xmin + 1, RY = ymax - ymin + 1, RZ = zmax - zmin + 1;
-  if (!empty && fits) {
-    for (int i = tid; i < (RX + 1) * PWP; i += kWarps * 32) SDx[i] = 0.0f;
-    for (int i = tid; i < RY * PP2; i += kWarps * 32) SDy[i] = 0.0f;
-    for (int i = tid; i < RZ * PP2; i += kWarps * 32) SDz[i] = 0.0f;
-    for (int i = tid; i < RX; i += kWarps * 32) Sxany[i] = 0;
-  }
-  __syncthreads();
-  if (!empty && fits && role >= 0) {
-    float *tab = role == 0 ? SDx : role == 1 ? SDy : SDz;
-    const int stride = role == 0 ? PWP : PP2;
-    const int mn = role == 0 ? xmin : role == 1 ? ymin : zmin;
-    for (int i = 0; i < ax.S; ++i) {
-      Tap t = axis_tap(axis_coord(ax, lane, i), asize);
-      if (t.valid) {
-        tab[(t.low - mn) * stride + lane] += t.h;
-        tab[(t.high - mn) * stride + lane] += t.l;
-        if (role == 0) Sxany[t.low - mn] = 1, Sxany[t.high - mn] = 1;
-      }
-    }
-  }
-  __syncthreads();
+  if (valid) stage_in_grad<CV>(p, it, PW, stage, lane);
+  build_cta_tables(T, it, p.PH, p.PD, warp, lane);
   if (!valid) return;  // padding warp of the last CTA of this RoI: no block-level barriers below
   cp_async_wait<0>();
   __syncwarp();
-  if (empty) return;
-  if (!fits) {
-    literal_tile_bwd<CV>(it, gb, C, PW, stage, lane, active, 0.0f);
+  if (T.empty) return;
+  if (!T.fits) {
+    literal_tile_bwd<CV>(it, gb, C, PW, stage, lane, active);
     return;
   }
+  const int RX = T.xmax - T.xmin + 1;
   // gradients to registers, scaled once by 1/count (reference: top*w/count per corner, :600-608)
   const float inv = __frcp_rn((float)(it.axd.S * it.axh.S * it.axw.S));
   float g[ROWS][PW][CV];
@@ -1276,39 +1080,21 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
       for (int pw = 0; pw < PW; ++pw)
         g[r][pw][c] = r < it.rows ? stage[(c * NB + r * PW + pw) * 33 + lane] * inv : 0.0f;
 
-  // compact lists of the y rows / z slices that carry weight for this (pd, ph-group)
-  int ny = 0, nz = 0;
-  for (int y0 = 0; y0 < RY; y0 += 32) {
-    const int yy = y0 + lane;
-    bool a = false;
-    if (yy < RY) {
-#pragma unroll
-      for (int r = 0; r < ROWS; ++r) a |= (r < it.rows) && SDy[yy * PP2 + it.ph0 + r] != 0.0f;
-    }
-    const unsigned bal = __ballot_sync(FULL, a);
-    if (a) ylist[ny + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)yy;
-    ny += __popc(bal);
-  }
-  for (int z0 = 0; z0 < RZ; z0 += 32) {
-    const int zz = z0 + lane;
-    const bool a = zz < RZ && SDz[zz * PP2 + it.pd] != 0.0f;
-    const unsigned bal = __ballot_sync(FULL, a);
-    if (a) zlist[nz + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)zz;
-    nz += __popc(bal);
-  }
-  __syncwarp();
+  const TabView ty{T.Dy, PP2, it.ph0}, tz{T.Dz, PP2, it.pd};
+  const int2 n = weighted_rows<ROWS>(ty, it.rows, T.ymax - T.ymin + 1, tz, T.zmax - T.zmin + 1, ylist, zlist, lane);
+  const int ny = n.x, nz = n.y;
 
   const long long row_elems = (long long)it.L.W * C;
   const long long slice_elems = (long long)it.L.H * row_elems;
-  float *gbase = gb + ((long long)zmin * it.L.H + ymin) * row_elems + (long long)xmin * C;
+  float *gbase = gb + ((long long)T.zmin * it.L.H + T.ymin) * row_elems + (long long)T.xmin * C;
   bool has_gaps = false;
-  for (int x0 = 0; x0 < RX; x0 += 32) has_gaps |= __any_sync(FULL, x0 + lane < RX && !Sxany[x0 + lane]);
+  for (int x0 = 0; x0 < RX; x0 += 32) has_gaps |= __any_sync(FULL, x0 + lane < RX && !T.xany[x0 + lane]);
   float zw[4];
   long long zo[4];
 #pragma unroll
   for (int zi = 0; zi < 4; ++zi) {
     const int zrel = zi < nz ? zlist[zi] : 0;
-    zw[zi] = zi < nz ? SDz[zrel * PP2 + it.pd] : 0.0f;
+    zw[zi] = zi < nz ? tz.at(zrel, 0) : 0.0f;
     zo[zi] = (long long)zrel * slice_elems;
   }
   for (int yi = 0; yi < ny; ++yi) {
@@ -1321,7 +1107,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
       for (int c = 0; c < CV; ++c) u[pw][c] = 0.0f;
 #pragma unroll
     for (int r = 0; r < ROWS; ++r) {
-      const float wy = r < it.rows ? SDy[yy * PP2 + it.ph0 + r] : 0.0f;
+      const float wy = r < it.rows ? ty.at(yy, r) : 0.0f;
       if (wy != 0.0f) {
 #pragma unroll
         for (int pw = 0; pw < PW; ++pw) {
@@ -1341,7 +1127,7 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
       for (int h = 0; h < 2; ++h)
 #pragma unroll
         for (int t4 = 0; t4 < PWP / 4; ++t4) {
-          const float4 t = *reinterpret_cast<const float4 *>(SDx + (xx + h) * PWP + t4 * 4);
+          const float4 t = *reinterpret_cast<const float4 *>(T.Dx + (xx + h) * PWP + t4 * 4);
           wx[h][t4 * 4 + 0] = t.x, wx[h][t4 * 4 + 1] = t.y, wx[h][t4 * 4 + 2] = t.z, wx[h][t4 * 4 + 3] = t.w;
         }
       float v[2][CV];
@@ -1371,13 +1157,13 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) roi_align3d_bwd2_kernel(con
         }
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
-        if (xx + h >= RX || (has_gaps && !Sxany[xx + h])) continue;  // warp-uniform
+        if (xx + h >= RX || (has_gaps && !T.xany[xx + h])) continue;  // warp-uniform
 #pragma unroll
         for (int zi = 0; zi < 4; ++zi)
           if (zi < nz) redv<CV>(ad[h][zi], o[h][zi]);
         for (int zi = 4; zi < nz; ++zi) {
           const int zrel = zlist[zi];
-          const float wz = SDz[zrel * PP2 + it.pd];
+          const float wz = tz.at(zrel, 0);
           float t[CV];
 #pragma unroll
           for (int c = 0; c < CV; ++c) t[c] = wz * v[h][c];
@@ -1575,119 +1361,88 @@ extern int g_topk_sieve;              // proposal.cu
 extern thread_local cudaEvent_t g_timing_ev[2];  // roi_align3d_stream.cu
 static int g_bwd_variant = 0;
 
+using RoiKernel = void (*)(RoiParams);
+
+// Per-warp grid: one warp per (RoI, chunk of 32*CV channels, pd, group of ROWS ph rows), kWarps warps per CTA.
+static int launch_per_warp(RoiKernel kern, RoiParams &p, int CV, int ROWS, size_t smem, const char *what,
+                           cudaStream_t st) {
+  p.nchunk = ceil_div(p.C, 32 * CV);
+  p.nphg = ceil_div(p.PH, ROWS);
+  p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
+  ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "%s: too many work items", what);
+  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<(unsigned)ceil_div_ll(p.total_items, kWarps), kWarps * 32, smem, st>>>(p);
+  ROI3D_LAUNCH_CHECK();
+  return ROI3D_OK;
+}
+
+// Per-RoI grid: the kWarps warps of a CTA work on one RoI, each on items_per_warp of its (chunk, pd, ph-group)
+// sub-items; ctas_per_roi CTAs per RoI.
+static int launch_per_roi(RoiKernel kern, RoiParams &p, int CV, int ROWS, int items_per_warp, size_t smem,
+                          const char *what, cudaStream_t st) {
+  p.nchunk = ceil_div(p.C, 32 * CV);
+  p.nphg = ceil_div(p.PH, ROWS);
+  p.items_per_roi = p.nchunk * p.PD * p.nphg;
+  p.items_per_warp = items_per_warp;
+  p.ctas_per_roi = ceil_div(p.items_per_roi, kWarps * items_per_warp);
+  p.total_items = (long long)p.K * p.items_per_roi;
+  const long long blocks = (long long)p.K * p.ctas_per_roi;
+  ROI3D_CHECK_ARG(blocks < 2147483647LL, "%s: too many work items", what);
+  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
+  ROI3D_LAUNCH_CHECK();
+  return ROI3D_OK;
+}
+
 template <int PW, int ROWS, int CV, int NXU>
 static int launch_fwd(RoiParams &p, cudaStream_t st) {
   using TB = Tables<PW>;
   constexpr int STAGE = ROWS * PW * 33;
   constexpr int WARP_FLOATS = ((STAGE > TB::FLOATS ? STAGE : TB::FLOATS) + 3) / 4 * 4;  // 16-byte aligned per warp
-  const size_t smem = (size_t)kWarps * WARP_FLOATS * sizeof(float);
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = ceil_div(p.PH, ROWS);
-  p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
-  auto kern = roi_align3d_fwd_cl_kernel<PW, ROWS, CV, NXU>;
-  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long blocks = ceil_div_ll(p.total_items, kWarps);
-  ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "roi_align3d forward: too many work items");
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  return launch_per_warp(roi_align3d_fwd_cl_kernel<PW, ROWS, CV, NXU>, p, CV, ROWS,
+                         (size_t)kWarps * WARP_FLOATS * sizeof(float), "roi_align3d forward", st);
 }
 
 template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB = 0>
 static int launch_fwd_ring(RoiParams &p, cudaStream_t st) {
   using TB = Tables<PW>;
-  constexpr int VOX = 32 * CV;
-  constexpr int RING = NS * (RXR + 2) * VOX;
+  constexpr int RING = NS * (RXR + 2) * 32 * CV;
   constexpr int STAGE = ROWS * PW * 33;
   constexpr int RING_OR_STAGE = RING > STAGE ? RING : STAGE;
   constexpr int WARP_FLOATS = (TB::FLOATS + 384 / 4 + RING_OR_STAGE + 3) / 4 * 4;
-  const size_t smem = (size_t)kWarps * WARP_FLOATS * sizeof(float);
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = ceil_div(p.PH, ROWS);
-  p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
-  auto kern = roi_align3d_fwd_ring_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB>;
-  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long blocks = ceil_div_ll(p.total_items, kWarps);
-  ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "roi_align3d forward: too many work items");
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  return launch_per_warp(roi_align3d_fwd_ring_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB>, p, CV, ROWS,
+                         (size_t)kWarps * WARP_FLOATS * sizeof(float), "roi_align3d forward", st);
 }
 
 template <int PW, int ROWS, int CV, int NXU, int NS, int RXR, int MINB = 0, bool MULTI = false, int ITEMS = 1>
 static int launch_fwd_ring2(RoiParams &p, cudaStream_t st) {
-  using LY = Ring2Layout<PW, ROWS, CV, NS, RXR>;
-  const size_t smem = LY::BYTES;
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = ceil_div(p.PH, ROWS);
-  p.items_per_roi = p.nchunk * p.PD * p.nphg;
-  p.items_per_warp = MULTI ? ITEMS : 1;
-  p.ctas_per_roi = ceil_div(p.items_per_roi, kWarps * p.items_per_warp);
-  p.total_items = (long long)p.K * p.items_per_roi;
-  const long long blocks = (long long)p.K * p.ctas_per_roi;
-  ROI3D_CHECK_ARG(blocks < 2147483647LL, "roi_align3d forward: too many work items");
-  auto kern = roi_align3d_fwd_ring2_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB, MULTI>;
-  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  return launch_per_roi(roi_align3d_fwd_ring2_kernel<PW, ROWS, CV, NXU, NS, RXR, MINB, MULTI>, p, CV, ROWS,
+                        MULTI ? ITEMS : 1, Ring2Layout<PW, ROWS, CV, NS, RXR>::BYTES, "roi_align3d forward", st);
 }
 
 template <int PW, int ROWS, int CV, int RXR>
 static int launch_bwd(RoiParams &p, cudaStream_t st) {
   using TB = Tables<PW>;
-  constexpr int VOX = 32 * CV;
   constexpr int STAGE = CV * ROWS * PW * 33;
-  constexpr int UX = RXR * VOX;
+  constexpr int UX = RXR * 32 * CV;
   constexpr int WARP_FLOATS = (TB::FLOATS + 80 / 4 + (STAGE > UX ? STAGE : UX) + 3) / 4 * 4;
-  const size_t smem = (size_t)kWarps * WARP_FLOATS * sizeof(float);
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = ceil_div(p.PH, ROWS);
-  p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
-  auto kern = roi_align3d_bwd_cl_kernel<PW, ROWS, CV, RXR>;
-  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long blocks = ceil_div_ll(p.total_items, kWarps);
-  ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "roi_align3d backward: too many work items");
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  return launch_per_warp(roi_align3d_bwd_cl_kernel<PW, ROWS, CV, RXR>, p, CV, ROWS,
+                         (size_t)kWarps * WARP_FLOATS * sizeof(float), "roi_align3d backward", st);
 }
 
 template <int PW, int ROWS, int CV, int MINB = 0>
 static int launch_bwd2(RoiParams &p, cudaStream_t st) {
   ROI3D_CHECK_ARG(p.PH <= PP2 && p.PD <= PP2, "roi_align3d backward: table rows narrower than PH / PD");
-  using TB = Tables<PW>;
-  constexpr int STAGE = CV * ROWS * PW * 33;
-  constexpr int WARP_FLOATS = (80 / 4 + STAGE + 3) / 4 * 4;
-  constexpr int SH_FLOATS = (RXMAX + 1) * TB::PWP + RYMAX * PP2 + RZMAX2 * PP2 + RXMAX + 8;
-  const size_t smem = ((size_t)((SH_FLOATS + 3) / 4 * 4) + (size_t)kWarps * WARP_FLOATS) * sizeof(float);
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = ceil_div(p.PH, ROWS);
-  p.items_per_roi = p.nchunk * p.PD * p.nphg;
-  p.ctas_per_roi = ceil_div(p.items_per_roi, kWarps);
-  p.total_items = (long long)p.K * p.items_per_roi;
-  const long long blocks = (long long)p.K * p.ctas_per_roi;
-  ROI3D_CHECK_ARG(blocks < 2147483647LL, "roi_align3d backward: too many work items");
-  auto kern = roi_align3d_bwd2_kernel<PW, ROWS, CV, MINB>;
-  ROI3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<(unsigned)blocks, kWarps * 32, smem, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  constexpr int WARP_FLOATS = (80 / 4 + CV * ROWS * PW * 33 + 3) / 4 * 4;
+  return launch_per_roi(roi_align3d_bwd2_kernel<PW, ROWS, CV, MINB>, p, CV, ROWS, 1,
+                        ((size_t)CtaTables<PW, true>::FLOATS + (size_t)kWarps * WARP_FLOATS) * sizeof(float),
+                        "roi_align3d backward", st);
 }
 
 template <int CV>
 static int launch_generic(RoiParams &p, bool fwd, cudaStream_t st) {
-  p.nchunk = ceil_div(p.C, 32 * CV);
-  p.nphg = p.PH;
-  p.total_items = (long long)p.K * p.nchunk * p.PD * p.nphg;
-  const long long blocks = ceil_div_ll(p.total_items, kWarps);
-  ROI3D_CHECK_ARG(p.total_items < 2147483647LL, "roi_align3d: too many work items");
-  if (fwd)
-    roi_align3d_fwd_generic_kernel<CV><<<(unsigned)blocks, kWarps * 32, 0, st>>>(p);
-  else
-    roi_align3d_bwd_generic_kernel<CV><<<(unsigned)blocks, kWarps * 32, 0, st>>>(p);
-  ROI3D_LAUNCH_CHECK();
-  return ROI3D_OK;
+  return launch_per_warp(fwd ? roi_align3d_fwd_generic_kernel<CV> : roi_align3d_bwd_generic_kernel<CV>, p, CV, 1, 0,
+                         "roi_align3d", st);
 }
 
 static bool aligned(const void *ptr, size_t a) { return (reinterpret_cast<uintptr_t>(ptr) % a) == 0; }

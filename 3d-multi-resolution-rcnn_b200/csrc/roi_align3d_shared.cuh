@@ -71,19 +71,10 @@ struct Item {
   LevelDev L;
 };
 
-__device__ __forceinline__ Item decode_item(const RoiParams &p, long long item64, int ROWS) {
-  Item it;
-  unsigned item = (unsigned)item64;  // launchers guarantee total_items < 2^31: 32-bit div/mod only
-  const unsigned phg = item % (unsigned)p.nphg;
-  item /= (unsigned)p.nphg;
-  it.pd = (int)(item % (unsigned)p.PD);
-  item /= (unsigned)p.PD;
-  it.chunk = (int)(item % (unsigned)p.nchunk);
-  it.k = (int)(item / (unsigned)p.nchunk);
-  it.krow = p.out_rows != nullptr ? __ldg(p.out_rows + it.k) : it.k;
-  it.ph0 = (int)phg * ROWS;
-  it.rows = min(ROWS, p.PH - it.ph0);
-  const float *roi = p.rois + (long long)it.k * 7;
+// RoI k's geometry: reads its row of p.rois and fills it.k, lvl, L, b, ok and the three axes.
+__device__ __forceinline__ void roi_geometry(const RoiParams &p, int k, Item &it) {
+  it.k = k;
+  const float *roi = p.rois + (long long)k * 7;
   float r[7];
 #pragma unroll
   for (int i = 0; i < 7; ++i) r[i] = __ldg(roi + i);
@@ -94,6 +85,21 @@ __device__ __forceinline__ Item decode_item(const RoiParams &p, long long item64
   it.axw = axis_setup(r[1], r[3], it.L.scale, p.PW, p.sample_num);
   it.axh = axis_setup(r[2], r[4], it.L.scale, p.PH, p.sample_num);
   it.axd = axis_setup(r[5], r[6], it.L.scale_d, p.PD, p.sample_num);
+}
+
+__device__ __forceinline__ Item decode_item(const RoiParams &p, long long item64, int ROWS) {
+  Item it;
+  unsigned item = (unsigned)item64;  // launchers guarantee total_items < 2^31: 32-bit div/mod only
+  const unsigned phg = item % (unsigned)p.nphg;
+  item /= (unsigned)p.nphg;
+  it.pd = (int)(item % (unsigned)p.PD);
+  item /= (unsigned)p.PD;
+  it.chunk = (int)(item % (unsigned)p.nchunk);
+  const int k = (int)(item / (unsigned)p.nchunk);
+  it.krow = p.out_rows != nullptr ? __ldg(p.out_rows + k) : k;
+  it.ph0 = (int)phg * ROWS;
+  it.rows = min(ROWS, p.PH - it.ph0);
+  roi_geometry(p, k, it);
   return it;
 }
 
