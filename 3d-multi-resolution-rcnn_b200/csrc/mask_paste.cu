@@ -9,12 +9,17 @@
 //   scipy.ndimage.gaussian_filter(mode='mirror', truncate 4.0) = per axis (z, y, x) a symmetric correlate1d in float64
 //   accumulators with the result rounded to the image dtype (float32) after every axis;
 //   coordinates c = factors * (o + 0.5) - 0.5;  scipy.ndimage.map_coordinates(order=1, mode='mirror'): the coordinate
-//   is folded into [0, n-1] by reflection, weights (1 - t, t), the 8 corners accumulated z-outer / x-inner in float64,
+//   is folded into [0, n-1] by reflection, weights (1 - t, 1 - (1 - t)), the 8 corners accumulated z-outer / x-inner in float64,
 //   rounded to float32;  clip to the filtered image's [min, max];  `> thr` in float32.
 // Parity status: unpinned by the reference (no test exercises it) -- checked against the same restatement running on
 // the scipy.ndimage that is installed in this image.
 //
-// One CTA per detection; the 14x14x10-sized mask lives in shared memory, arithmetic in float64 like scipy.
+// Work layout: the CTA (detection, split) computes the whole filtered mask in shared memory -- the clip needs its min
+// and max -- and resamples one contiguous chunk of the detection's output voxels.  A detection with few output voxels
+// (the box smaller than the mask: heavy filtering, little resampling) takes one CTA; a large box (little or no
+// filtering, up to hundreds of thousands of output voxels) is spread over up to `splits` CTAs.  Every axis is filtered
+// in place: a warp owns a whole line, copies it with its mirror extension into a per-warp float64 buffer and writes
+// the filtered line back, so one float32 image of the mask is all the CTA keeps.
 #include <algorithm>
 #include <vector>
 
@@ -22,8 +27,20 @@
 
 namespace roi3d {
 
-constexpr int kMaskMaxVol = 4096;   // floats of one mask (14*14*10 = 1960)
-constexpr int kMaskMaxTaps = 257;   // gaussian half width up to 128
+constexpr int kMaskMaxTaps = 257;   // mask targets: gaussian half width up to 128
+
+constexpr int kPasteThreads = 256;
+constexpr int kPasteWarps = kPasteThreads / 32;
+constexpr int kPasteMaxAxis = 64;                                       // longest mask axis
+constexpr int kPasteMaxHalf = 126;                                      // int(4 sigma + 0.5) at sigma = (64 / 1 - 1) / 2
+constexpr int kPasteMaxTaps = 2 * kPasteMaxHalf + 1;
+constexpr int kPasteLineLen = kPasteMaxAxis + 2 * kPasteMaxHalf;        // a line with its mirror extension
+constexpr int kPasteFixedSmem = (kPasteMaxTaps + kPasteWarps * kPasteLineLen) * 8 + 2 * kPasteWarps * 4;  // 22,312 B
+constexpr int kPasteSmemBudget = 227 * 1024;                            // shared memory of one block on sm_100
+constexpr int kPasteMaxVol = (kPasteSmemBudget - kPasteFixedSmem) / 4;  // 52,534 voxels of float32 mask
+constexpr long long kPasteMinChunk = 8192;  // output voxels below which a detection is not split further
+constexpr int kPasteMaxSplits = 16;
+constexpr int kPasteGridCtas = 4096;        // splits = clamp(kPasteGridCtas / n, 1, kPasteMaxSplits)
 
 __device__ __forceinline__ int mirror_index(int i, int n) {
   if (n == 1) return 0;
@@ -39,93 +56,129 @@ __device__ __forceinline__ double mirror_coord(double c, int n) {
   const double len = (double)n - 1.0;
   if (c < 0.0) {
     const double sz2 = 2.0 * len;
-    c = sz2 * (double)(long long)(-c / sz2) + c;
-    c = c <= -len ? c + sz2 : -c;
+    c = __dadd_rn(sz2 * (double)(long long)__ddiv_rn(-c, sz2), c);
+    c = c <= -len ? __dadd_rn(c, sz2) : -c;
   } else if (c > len) {
     const double sz2 = 2.0 * len;
-    c -= sz2 * (double)(long long)(c / sz2);
-    if (c > len) c = sz2 - c;
+    c = __dsub_rn(c, sz2 * (double)(long long)__ddiv_rn(c, sz2));
+    if (c > len) c = __dsub_rn(sz2, c);
   }
   return c;
 }
 
-__global__ void __launch_bounds__(256) mask_paste_kernel(const float *__restrict__ logits, int Dm, int Hm, int Wm,
-                                                         const int32_t *__restrict__ boxes,
-                                                         const int64_t *__restrict__ offsets, float thr,
-                                                         unsigned char *__restrict__ out) {
-  __shared__ float A[kMaskMaxVol];
-  __shared__ float B[kMaskMaxVol];
-  __shared__ double wts[kMaskMaxTaps];
-  __shared__ float red_min[256], red_max[256];
-  const int det = blockIdx.x, tid = threadIdx.x;
-  const int vol = Dm * Hm * Wm;
+// numpy's pairwise_sum (np.sum of a contiguous float64 array), as `phi_x / phi_x.sum()` normalises the gaussian
+__device__ double np_pairwise_sum(const double *a, int n) {
+  if (n < 8) {
+    double r = 0.0;
+    for (int i = 0; i < n; ++i) r = __dadd_rn(r, a[i]);
+    return r;
+  }
+  if (n <= 128) {
+    double r[8];
+    for (int j = 0; j < 8; ++j) r[j] = a[j];
+    int i = 8;
+    for (; i < n - (n % 8); i += 8)
+      for (int j = 0; j < 8; ++j) r[j] = __dadd_rn(r[j], a[i + j]);
+    double res = __dadd_rn(__dadd_rn(__dadd_rn(r[0], r[1]), __dadd_rn(r[2], r[3])),
+                           __dadd_rn(__dadd_rn(r[4], r[5]), __dadd_rn(r[6], r[7])));
+    for (; i < n; ++i) res = __dadd_rn(res, a[i]);
+    return res;
+  }
+  int n2 = n / 2;
+  n2 -= n2 % 8;
+  return __dadd_rn(np_pairwise_sum(a, n2), np_pairwise_sum(a + n2, n - n2));
+}
+
+// logits [n, num_channels, Dm, Hm, Wm]; detection i reads channel `channel[i]` (channel == nullptr: channel 0).
+// Grid (n, splits), dynamic shared memory kPasteFixedSmem + 4 * Dm * Hm * Wm bytes.
+__global__ void __launch_bounds__(kPasteThreads) mask_paste_kernel(const float *__restrict__ logits, int num_channels,
+                                                                   const int64_t *__restrict__ channel, int Dm, int Hm,
+                                                                   int Wm, const int32_t *__restrict__ boxes,
+                                                                   const int64_t *__restrict__ offsets, float thr,
+                                                                   unsigned char *__restrict__ out) {
+  extern __shared__ double smem_d[];
+  double *wts = smem_d;                                   // kPasteMaxTaps
+  double *line = wts + kPasteMaxTaps + (threadIdx.x >> 5) * kPasteLineLen;   // this warp's line buffer
+  float *red = reinterpret_cast<float *>(smem_d + kPasteMaxTaps + kPasteWarps * kPasteLineLen);  // 2 * kPasteWarps
+  float *M = red + 2 * kPasteWarps;                       // the mask, Dm * Hm * Wm
+  __shared__ double wsum;
+  const int det = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int32_t *bx = boxes + (long long)det * 6;
   const int ow = max(bx[2] - bx[0] + 1, 1), oh = max(bx[3] - bx[1] + 1, 1), od = max(bx[5] - bx[4] + 1, 1);
-  const float *src = logits + (long long)det * vol;
-  for (int i = tid; i < vol; i += 256) A[i] = __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-src[i])));  // torch sigmoid
+  const long long total = (long long)od * oh * ow;
+  const long long active = min((long long)gridDim.y, max(1LL, (total + kPasteMinChunk - 1) / kPasteMinChunk));
+  if ((long long)blockIdx.y >= active) return;
+  const long long chunk = (total + active - 1) / active;
+  const long long lo = chunk * blockIdx.y, hi = min(total, lo + chunk);
+  unsigned char *dst = out + offsets[det];
+  const long long ch = channel ? channel[det] : 0;
+  if (ch < 0 || ch >= num_channels) {   // documented: an out-of-range channel gives an all-zero mask
+    for (long long o = lo + tid; o < hi; o += kPasteThreads) dst[o] = 0;
+    return;
+  }
+  const int vol = Dm * Hm * Wm;
+  const float *src = logits + ((long long)det * num_channels + ch) * vol;
+  for (int i = tid; i < vol; i += kPasteThreads) M[i] = __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-src[i])));  // torch sigmoid
   __syncthreads();
   const int dims[3] = {Dm, Hm, Wm};
   const int outs[3] = {od, oh, ow};
   const int strides[3] = {Hm * Wm, Wm, 1};
-  float *cur = A, *nxt = B;
-  // ---- anti-aliasing gaussian, axis by axis ----
+  // ---- anti-aliasing gaussian, axis by axis, each line filtered in place by one warp ----
   for (int ax = 0; ax < 3; ++ax) {
-    const double factor = (double)dims[ax] / (double)outs[ax];
-    const double sigma = fmax(0.0, (factor - 1.0) / 2.0);
+    const double factor = __ddiv_rn((double)dims[ax], (double)outs[ax]);
+    const double sigma = fmax(0.0, __dmul_rn(__dsub_rn(factor, 1.0), 0.5));   // (factors - 1) / 2
     if (!(sigma > 1e-15)) continue;
-    int lw = (int)(4.0 * sigma + 0.5);
-    if (lw > (kMaskMaxTaps - 1) / 2) lw = (kMaskMaxTaps - 1) / 2;  // (cannot happen for masks up to 64 voxels per axis)
-    for (int i = tid; i <= 2 * lw; i += 256) {
+    const int lw = (int)__dadd_rn(__dmul_rn(4.0, sigma), 0.5);               // <= kPasteMaxHalf for axes <= 64
+    const double k = __ddiv_rn(-0.5, __dmul_rn(sigma, sigma));
+    for (int i = tid; i <= 2 * lw; i += kPasteThreads) {
       const double x = (double)(i - lw);
-      wts[i] = exp(-0.5 / (sigma * sigma) * (x * x));
+      wts[i] = exp(__dmul_rn(k, __dmul_rn(x, x)));
     }
     __syncthreads();
-    if (tid == 0) {
-      double sum = 0.0;
-      for (int i = 0; i <= 2 * lw; ++i) sum += wts[i];
-      for (int i = 0; i <= 2 * lw; ++i) wts[i] = wts[i] / sum;
-    }
+    if (tid == 0) wsum = np_pairwise_sum(wts, 2 * lw + 1);
     __syncthreads();
-    const int n = dims[ax], st = strides[ax];
-    for (int e = tid; e < vol; e += 256) {
-      const int pos = (e / st) % n;
-      const int base = e - pos * st;
-      double tmp = (double)cur[e] * wts[lw];
-      for (int ll = -lw; ll < 0; ++ll) {
-        const double l = (double)cur[base + mirror_index(pos + ll, n) * st];
-        const double r = (double)cur[base + mirror_index(pos - ll, n) * st];
-        tmp += (l + r) * wts[ll + lw];
+    for (int i = tid; i <= 2 * lw; i += kPasteThreads) wts[i] = __ddiv_rn(wts[i], wsum);
+    __syncthreads();
+    const int n = dims[ax], st = strides[ax], ext = n + 2 * lw;
+    const int lines = vol / n;
+    for (int l = warp; l < lines; l += kPasteWarps) {
+      float *base = M + (l / st) * (st * n) + l % st;
+      for (int j = lane; j < ext; j += 32) line[j] = (double)base[mirror_index(j - lw, n) * st];
+      __syncwarp();
+      for (int p = lane; p < n; p += 32) {
+        const double *c = line + p + lw;
+        double tmp = __dmul_rn(c[0], wts[lw]);   // scipy's symmetric correlate1d: separate multiplies and adds
+        for (int ll = -lw; ll < 0; ++ll) tmp = __dadd_rn(tmp, __dmul_rn(__dadd_rn(c[ll], c[-ll]), wts[ll + lw]));
+        base[p * st] = (float)tmp;
       }
-      nxt[e] = (float)tmp;
+      __syncwarp();
     }
     __syncthreads();
-    float *t = cur;
-    cur = nxt, nxt = t;
   }
   // ---- min / max of the filtered image (clip=True) ----
   float mn = INFINITY, mx = -INFINITY;
-  for (int i = tid; i < vol; i += 256) mn = fminf(mn, cur[i]), mx = fmaxf(mx, cur[i]);
-  red_min[tid] = mn, red_max[tid] = mx;
+  for (int i = tid; i < vol; i += kPasteThreads) mn = fminf(mn, M[i]), mx = fmaxf(mx, M[i]);
+  for (int o = 16; o > 0; o >>= 1)
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o)), mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if (lane == 0) red[warp] = mn, red[kPasteWarps + warp] = mx;
   __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if (tid < o) red_min[tid] = fminf(red_min[tid], red_min[tid + o]), red_max[tid] = fmaxf(red_max[tid], red_max[tid + o]);
-    __syncthreads();
-  }
-  mn = red_min[0], mx = red_max[0];
-  // ---- trilinear resample at the box resolution, threshold ----
-  const double fz = (double)Dm / (double)od, fy = (double)Hm / (double)oh, fx = (double)Wm / (double)ow;
-  const long long total = (long long)od * oh * ow;
-  unsigned char *dst = out + offsets[det];
-  for (long long o = tid; o < total; o += 256) {
+  mn = red[0], mx = red[kPasteWarps];
+  for (int w = 1; w < kPasteWarps; ++w) mn = fminf(mn, red[w]), mx = fmaxf(mx, red[kPasteWarps + w]);
+  // ---- trilinear resample of this CTA's chunk at the box resolution, threshold ----
+  const double fz = __ddiv_rn((double)Dm, (double)od), fy = __ddiv_rn((double)Hm, (double)oh),
+               fx = __ddiv_rn((double)Wm, (double)ow);
+  for (long long o = lo + tid; o < hi; o += kPasteThreads) {
     const int x = (int)(o % ow);
     const long long t1 = o / ow;
     const int y = (int)(t1 % oh), z = (int)(t1 / oh);
-    const double cz = mirror_coord(fz * ((double)z + 0.5) - 0.5, Dm);
-    const double cy = mirror_coord(fy * ((double)y + 0.5) - 0.5, Hm);
-    const double cx = mirror_coord(fx * ((double)x + 0.5) - 0.5, Wm);
+    // c = factors * (o + 0.5) - 0.5, folded; weights (1 - t, 1 - (1 - t)) as scipy's spline weights for order 1
+    const double cz = mirror_coord(__dsub_rn(__dmul_rn(fz, __dadd_rn((double)z, 0.5)), 0.5), Dm);
+    const double cy = mirror_coord(__dsub_rn(__dmul_rn(fy, __dadd_rn((double)y, 0.5)), 0.5), Hm);
+    const double cx = mirror_coord(__dsub_rn(__dmul_rn(fx, __dadd_rn((double)x, 0.5)), 0.5), Wm);
     const int z0 = (int)floor(cz), y0 = (int)floor(cy), x0 = (int)floor(cx);
-    const double tz = cz - (double)z0, ty = cy - (double)y0, tx = cx - (double)x0;
-    const double wz[2] = {1.0 - tz, tz}, wy[2] = {1.0 - ty, ty}, wx[2] = {1.0 - tx, tx};
+    const double wz0 = __dsub_rn(1.0, __dsub_rn(cz, (double)z0)), wy0 = __dsub_rn(1.0, __dsub_rn(cy, (double)y0)),
+                 wx0 = __dsub_rn(1.0, __dsub_rn(cx, (double)x0));
+    const double wz[2] = {wz0, __dsub_rn(1.0, wz0)}, wy[2] = {wy0, __dsub_rn(1.0, wy0)}, wx[2] = {wx0, __dsub_rn(1.0, wx0)};
     const int zi[2] = {mirror_index(z0, Dm), mirror_index(z0 + 1, Dm)};
     const int yi[2] = {mirror_index(y0, Hm), mirror_index(y0 + 1, Hm)};
     const int xi[2] = {mirror_index(x0, Wm), mirror_index(x0 + 1, Wm)};
@@ -136,11 +189,11 @@ __global__ void __launch_bounds__(256) mask_paste_kernel(const float *__restrict
       for (int b = 0; b < 2; ++b)
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
-          double coeff = (double)cur[(zi[a] * Hm + yi[b]) * Wm + xi[c]];
-          coeff *= wz[a];
-          coeff *= wy[b];
-          coeff *= wx[c];
-          acc += coeff;
+          double coeff = (double)M[(zi[a] * Hm + yi[b]) * Wm + xi[c]];
+          coeff = __dmul_rn(coeff, wz[a]);
+          coeff = __dmul_rn(coeff, wy[b]);
+          coeff = __dmul_rn(coeff, wx[c]);
+          acc = __dadd_rn(acc, coeff);
         }
     float v = (float)acc;
     v = fminf(fmaxf(v, mn), mx);
@@ -274,16 +327,48 @@ using namespace roi3d;
 
 extern "C" {
 
-int roi3d_mask_paste(const float *mask_logits_dev, int n, int Dm, int Hm, int Wm, const int32_t *boxes_dev,
-                     const int64_t *offsets_dev, float thr, uint8_t *out_dev, void *stream) {
-  ROI3D_CHECK_ARG(n >= 0 && Dm > 0 && Hm > 0 && Wm > 0, "bad sizes");
+}  // extern "C"
+
+namespace {
+
+int mask_paste_launch(const float *logits_dev, int n, int num_channels, int Dm, int Hm, int Wm,
+                      const int64_t *channel_dev, const int32_t *boxes_dev, const int64_t *offsets_dev, float thr,
+                      uint8_t *out_dev, void *stream) {
+  ROI3D_CHECK_ARG(n >= 0, "n = %d is negative", n);
+  ROI3D_CHECK_ARG(num_channels >= 1, "num_channels = %d must be at least 1", num_channels);
+  ROI3D_CHECK_ARG(Dm > 0 && Hm > 0 && Wm > 0, "mask size %dx%dx%d (Dm x Hm x Wm) must be positive", Dm, Hm, Wm);
+  ROI3D_CHECK_ARG((long long)Dm * Hm * Wm <= kPasteMaxVol, "mask of %dx%dx%d (Dm x Hm x Wm) exceeds %d voxels", Dm, Hm,
+                  Wm, kPasteMaxVol);
+  ROI3D_CHECK_ARG(Dm <= kPasteMaxAxis && Hm <= kPasteMaxAxis && Wm <= kPasteMaxAxis,
+                  "mask axes Dm, Hm, Wm = %d, %d, %d: longer than %d is not supported", Dm, Hm, Wm, kPasteMaxAxis);
   if (n == 0) return ROI3D_OK;
-  ROI3D_CHECK_ARG(mask_logits_dev && boxes_dev && offsets_dev && out_dev, "NULL pointer");
-  ROI3D_CHECK_ARG((long long)Dm * Hm * Wm <= kMaskMaxVol, "mask of %dx%dx%d exceeds %d voxels", Dm, Hm, Wm, kMaskMaxVol);
-  ROI3D_CHECK_ARG(Dm <= 64 && Hm <= 64 && Wm <= 64, "mask axes longer than 64 are not supported");
-  mask_paste_kernel<<<n, 256, 0, (cudaStream_t)stream>>>(mask_logits_dev, Dm, Hm, Wm, boxes_dev, offsets_dev, thr, out_dev);
+  ROI3D_CHECK_ARG(logits_dev, "mask logits pointer is NULL");
+  ROI3D_CHECK_ARG(boxes_dev, "boxes_dev is NULL");
+  ROI3D_CHECK_ARG(offsets_dev, "offsets_dev is NULL");
+  ROI3D_CHECK_ARG(out_dev, "out_dev is NULL");
+  const int smem = kPasteFixedSmem + 4 * Dm * Hm * Wm;
+  ROI3D_CUDA(cudaFuncSetAttribute(mask_paste_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  const int splits = std::min(kPasteMaxSplits, std::max(1, kPasteGridCtas / n));
+  mask_paste_kernel<<<dim3((unsigned)n, (unsigned)splits), kPasteThreads, smem, (cudaStream_t)stream>>>(
+      logits_dev, num_channels, channel_dev, Dm, Hm, Wm, boxes_dev, offsets_dev, thr, out_dev);
   ROI3D_LAUNCH_CHECK();
   return ROI3D_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int roi3d_mask_paste(const float *mask_logits_dev, int n, int Dm, int Hm, int Wm, const int32_t *boxes_dev,
+                     const int64_t *offsets_dev, float thr, uint8_t *out_dev, void *stream) {
+  return mask_paste_launch(mask_logits_dev, n, 1, Dm, Hm, Wm, nullptr, boxes_dev, offsets_dev, thr, out_dev, stream);
+}
+
+int roi3d_mask_paste_select(const float *mask_pred_dev, int n, int num_channels, int Dm, int Hm, int Wm,
+                            const int64_t *channel_dev, const int32_t *boxes_dev, const int64_t *offsets_dev, float thr,
+                            uint8_t *out_dev, void *stream) {
+  return mask_paste_launch(mask_pred_dev, n, num_channels, Dm, Hm, Wm, channel_dev, boxes_dev, offsets_dev, thr, out_dev,
+                           stream);
 }
 
 size_t roi3d_mask_target_workspace_bytes(const int32_t *crop_dhw_host, int n) {

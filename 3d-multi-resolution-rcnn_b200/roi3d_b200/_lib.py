@@ -80,6 +80,7 @@ def _load():
         "roi3d_roi_align3d_forward_host": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int,
                                                    c_int, c_int, c_float, c_float, c_int, P]),
         "roi3d_mask_paste": (c_int, [P, c_int, c_int, c_int, c_int, P, P, c_float, P, P]),
+        "roi3d_mask_paste_select": (c_int, [P, c_int, c_int, c_int, c_int, c_int, P, P, P, c_float, P, P]),
         "roi3d_mask_target_workspace_bytes": (c_size_t, [P, c_int]),
         "roi3d_mask_target": (c_int, [P, c_int, c_int, c_int, c_int, P, P, c_int, c_int, c_int, c_int, P, P, c_size_t, P]),
         "roi3d_grid_anchors": (c_int, [c_int, c_int, c_int, c_int, c_float, c_float, P, c_int, c_int, c_int, c_float,

@@ -269,10 +269,20 @@ int roi3d_delta2bbox3d(const float *rois_dev, int stride_r, const float *deltas_
  *   selected); boxes_dev int32 [n, 6] = (x1, y1, x2, y2, z1, z2) after the reference's `(bbox / scale).astype(int32)`;
  *   detection i's binary mask of max(z2-z1+1,1) x max(y2-y1+1,1) x max(x2-x1+1,1) voxels (z, y, x order) is written
  *   at out_dev + offsets_dev[i].  The resize restates scikit-image 0.18.0 `resize` (n-D branch: gaussian
- *   anti-aliasing + order-1 map_coordinates, mode reflect) in float64 like scipy.
+ *   anti-aliasing + order-1 map_coordinates, mode reflect) in float64 like scipy, every operation in scipy's order.
+ *   Mask size: each axis at most 64 and Dm * Hm * Wm at most 52,534 voxels (the float32 mask plus 22,312 bytes of
+ *   filter tables fill the 227 KB of shared memory of one block); larger masks return ROI3D_EINVAL before any launch.
+ *   The mask head's output, 20 x 28 x 28 = 15,680 voxels, takes 83 KB.
  * ---------------------------------------------------------------------------------------------- */
 int roi3d_mask_paste(const float *mask_logits_dev, int n, int Dm, int Hm, int Wm, const int32_t *boxes_dev,
                      const int64_t *offsets_dev, float thr, uint8_t *out_dev, void *stream);
+/* Same, reading the class channel of the head's whole output: mask_pred_dev [n, num_channels, Dm, Hm, Wm] fp32 logits;
+ *   detection i reads channel channel_dev[i] (int64 [n]; NULL: channel 0, the class-agnostic head), so the caller
+ *   does not copy `mask_pred[arange(n), labels]` first (fcn_mask_head_3d.py:166-170).  A channel outside
+ *   [0, num_channels) gives that detection an all-zero mask. */
+int roi3d_mask_paste_select(const float *mask_pred_dev, int n, int num_channels, int Dm, int Hm, int Wm,
+                            const int64_t *channel_dev, const int32_t *boxes_dev, const int64_t *offsets_dev, float thr,
+                            uint8_t *out_dev, void *stream);
 
 /* Mask targets (SURVEY section 8f, N4, training half).
  * Replaces: mask_target_single, mmdet/core/mask/mask_target.py:17-50 (per positive proposal on the host: crop of the
