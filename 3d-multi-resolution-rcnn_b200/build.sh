@@ -10,7 +10,7 @@ FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompil
 [ "${VERBOSE_PTXAS:-0}" = "1" ] && FLAGS+=(-Xptxas -v)
 [ -n "${ROI3D_EXTRA_NVCC_FLAGS:-}" ] && FLAGS+=(${ROI3D_EXTRA_NVCC_FLAGS})
 pids=()
-for f in roi_align3d roi_align3d_stream roi_align3d_planar roi_align3d_det nms3d soft_nms3d proposal assign mask_paste host_api; do
+for f in roi_align3d roi_align3d_stream roi_align3d_planar roi_align3d_det nms3d soft_nms3d multiclass_nms proposal assign mask_paste host_api; do
   src=$HERE/csrc/$f.cu
   obj=$HERE/build/$f.o
   if [ ! -f "$obj" ] || [ "$src" -nt "$obj" ] || [ "$HERE/csrc/common.cuh" -nt "$obj" ] || [ "$HERE/csrc/roi_align3d_shared.cuh" -nt "$obj" ] \
@@ -20,5 +20,5 @@ for f in roi_align3d roi_align3d_stream roi_align3d_planar roi_align3d_det nms3d
   fi
 done
 for p in "${pids[@]:-}"; do [ -n "$p" ] && wait "$p"; done
-"$NVCC" -gencode arch=compute_100a,code=sm_100a -shared -o "$OUT/libroi3d_b200.so" "$HERE"/build/{roi_align3d,roi_align3d_stream,roi_align3d_planar,roi_align3d_det,nms3d,soft_nms3d,proposal,assign,mask_paste,host_api}.o -cudart static
+"$NVCC" -gencode arch=compute_100a,code=sm_100a -shared -o "$OUT/libroi3d_b200.so" "$HERE"/build/{roi_align3d,roi_align3d_stream,roi_align3d_planar,roi_align3d_det,nms3d,soft_nms3d,multiclass_nms,proposal,assign,mask_paste,host_api}.o -cudart static
 echo "built $OUT/libroi3d_b200.so"

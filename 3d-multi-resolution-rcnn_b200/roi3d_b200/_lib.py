@@ -77,6 +77,9 @@ def _load():
         "roi3d_nms3d_eval_batched": (c_int, [P, P, c_int, c_int, ctypes.c_double, P, P, P, P, c_size_t, P]),
         "roi3d_nms3d_host": (c_int, [P, c_int, c_float, P, P]),
         "roi3d_soft_nms3d_batched": (c_int, [P, P, c_int, c_int, c_int, c_float, c_float, c_float, P, P, P, P]),
+        "roi3d_multiclass_nms3d_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int, c_int]),
+        "roi3d_multiclass_nms3d_batched": (c_int, [P, c_int, P, P, c_int, c_int, c_int, c_float, c_int, c_float, c_int,
+                                                   c_float, c_float, c_int, P, P, P, P, c_size_t, P]),
         "roi3d_roi_align3d_forward_host": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int,
                                                    c_int, c_int, c_float, c_float, c_int, P]),
         "roi3d_mask_paste": (c_int, [P, c_int, c_int, c_int, c_int, P, P, c_float, P, P]),

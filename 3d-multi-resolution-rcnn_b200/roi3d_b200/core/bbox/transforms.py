@@ -16,6 +16,20 @@ def bbox2roi3D(bbox_list):
     return torch.cat([batch, coords], dim=1)
 
 
+def bbox2roi3D_padded(boxes, counts):
+    """Fixed-shape bbox2roi3D: boxes [B, n, >=6] holding counts[b] valid rows per image (counts: [B] integers on the
+    same device) -> rois [B*n, 7].  Row b*n + r is (b, x1, y1, x2, y2, z1, z2) when r < counts[b] and exactly (-1, 0, 0, 0, 0, 0, 0)
+    otherwise: the RoI extractors give a zero row for a batch index outside [0, B), and the coordinates are zeroed too,
+    because padding rows may hold anything (NaN included) and would still reach the level map.  Reads nothing back to
+    the host, so it can be captured in a CUDA graph with the rest of a fixed-shape stage."""
+    B, n = boxes.shape[0], boxes.shape[1]
+    valid = torch.arange(n, device=boxes.device)[None, :] < counts.reshape(B, 1)
+    batch = torch.arange(B, device=boxes.device, dtype=boxes.dtype)[:, None].expand(B, n)
+    batch = torch.where(valid, batch, -1.0)
+    coords = torch.where(valid[:, :, None], boxes[:, :, :6], 0.0)
+    return torch.cat([batch[:, :, None], coords], dim=2).reshape(B * n, 7)
+
+
 def delta2bbox3D(rois, deltas, means=(0, 0, 0, 0, 0, 0), stds=(1, 1, 1, 1, 1, 1), max_shape=None,
                  wh_ratio_clip=16 / 1000, d_ratio_clip=64 / 1000):
     """Decode [n, 6k] class-wise deltas against [n, >=6] boxes, one kernel (roi3d_delta2bbox3d); the caller outside the

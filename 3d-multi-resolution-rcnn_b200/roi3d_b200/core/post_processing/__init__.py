@@ -1,3 +1,3 @@
-from .bbox_nms import multiclass_nms_3d
+from .bbox_nms import multiclass_nms_3d, multiclass_nms_3d_batched
 
-__all__ = ['multiclass_nms_3d']
+__all__ = ['multiclass_nms_3d', 'multiclass_nms_3d_batched']

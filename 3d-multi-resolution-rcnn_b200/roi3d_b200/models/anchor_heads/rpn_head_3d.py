@@ -232,6 +232,15 @@ class RPNProposal3D(object):
         n_out = [min(int(v), kk) for v in n_valid.tolist()]  # the single host read of the whole path
         return [final[b, :n_out[b]] for b in range(len(n_out))]
 
+    def get_proposals_padded(self, cls_scores, bbox_preds, img_metas, cfg):
+        """get_proposals with fixed shapes and no host read: (final [B, kk, 7], counts int32 [B]) as device tensors, where
+        final[b, :counts[b]] equals get_proposals(...)[b] and the rows past counts[b] are unspecified.  kk depends on
+        the level shapes and the config only, so the call can be captured in a CUDA graph (as part of a larger stage);
+        its first call per shape uploads small descriptor tensors from pageable memory, so run it once before a
+        capture."""
+        final, n_valid, kk = self._enqueue(cls_scores, bbox_preds, img_metas, cfg)
+        return final, n_valid.clamp(max=kk)
+
     def _enqueue(self, cls_scores, bbox_preds, img_metas, cfg):
         """cls_scores[l]: [B, A, D, H, W]; bbox_preds[l]: [B, 6A, D, H, W]; img_metas[b]['img_shape'] = (H, W, 3, D).
         Same positional arguments as AnchorHead3D.get_bboxes (anchor_head_3d.py:232-233): `img_meta_2` / `img_meta_3`,

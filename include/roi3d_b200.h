@@ -205,6 +205,32 @@ int roi3d_soft_nms3d_batched(const float *dets_dev, const int32_t *seg_counts_de
                              float iou_thr, float sigma, float min_score, float *out_dets_dev, int64_t *inds_dev,
                              int32_t *num_keep_dev, void *stream);
 
+/* Multiclass 3D NMS of B images in one call, with fixed-shape outputs and no host synchronisation (it can be captured
+ * in a CUDA graph).
+ * Replaces: multiclass_nms_3d, mmdet/core/post_processing/bbox_nms.py:57-106, run once per image (the reference's
+ *   per-class loop has a `.any()` host sync and an NMS per class).
+ * bboxes_dev: [B, n, box_cols] fp32 with box_cols = 6 (boxes shared by the classes) or 6 * num_classes (class c in
+ *   columns 6c..6c+5); scores_dev: [B, n, num_classes] fp32, class 0 the background; counts_dev: int32 [B], image b uses
+ *   its first min(max(counts[b], 0), n) rows and never reads the others.
+ * Per image: for each class c >= 1, the rows with score > score_thr (fp32 compare; NaN never passes), in row order, go
+ *   through nms_type 0 = NMS (roi3d_nms3d_batched: kept rows in ascending row order) or 1 = soft-NMS
+ *   (roi3d_soft_nms3d_batched with soft_method 1 = linear / 2 = gaussian, sigma, min_score: rows in selection order
+ *   with their decayed scores; n <= 4096); the kept rows are concatenated class by class (class 1 first) with label
+ *   c - 1; then the reference's cut `if len > max_num: sort(score, descending, stable)[:max_num]`, with Python's slice
+ *   rule: max_num > 0 keeps all rows in concatenation order when len <= max_num, else the top max_num by score (ties to
+ *   the earlier row); max_num == 0 keeps none; max_num < 0 keeps the first len + max_num rows in score order.
+ * Outputs, M = max_num > 0 ? max_num : (num_classes - 1) * n: det_dev [B, M, 7] (x1,y1,x2,y2,z1,z2,score),
+ *   labels_dev int64 [B, M], det_counts_dev int32 [B]; rows past det_counts[b] are zeros with label -1.
+ * workspace_dev: 256-byte aligned, roi3d_multiclass_nms3d_workspace_bytes(B, n, num_classes, max_num, nms_type) bytes.
+ * num_classes < 2, box_cols other than 6 or 6 * num_classes, an unknown nms_type or soft_method, n > 4096 with
+ *   soft-NMS (n > 32768 with NMS) and NULL pointers return ROI3D_EINVAL before anything is launched. */
+size_t roi3d_multiclass_nms3d_workspace_bytes(int B, int n, int num_classes, int max_num, int soft);
+int roi3d_multiclass_nms3d_batched(const float *bboxes_dev, int box_cols, const float *scores_dev,
+                                   const int32_t *counts_dev, int B, int n, int num_classes, float score_thr,
+                                   int nms_type, float iou_thr, int soft_method, float sigma, float min_score,
+                                   int max_num, float *det_dev, int64_t *labels_dev, int32_t *det_counts_dev,
+                                   void *workspace_dev, size_t workspace_bytes, void *stream);
+
 /* Host-buffer form of one NMS call: what mmdet.ops.nms(dets_numpy, thr, device_id) does
  * (mmdet/ops/nms/nms_wrapper.py:29-32,42-52).  keep_host capacity n; returns count in *num_keep_host. */
 int roi3d_nms3d_host(const float *dets_host, int n, float iou_thr, int64_t *keep_host, int32_t *num_keep_host);
