@@ -1,10 +1,12 @@
-"""Batched multiclass 3D NMS (`multiclass_nms_3d_batched`, `roi3d_multiclass_nms3d_batched`) and the fixed-shape
-helpers around it (`RPNProposal3D.get_proposals_padded`, `bbox2roi3D_padded`).
+"""Batched multiclass 3D NMS (`multiclass_nms_3d_batched`, `roi3d_multiclass_nms3d_batched`), the per-image
+`multiclass_nms_3d` built on it, and the fixed-shape helpers around them (`RPNProposal3D.get_proposals_padded`,
+`bbox2roi3D_padded`).
 
-The reference for the batched call is the per-image `multiclass_nms_3d` (itself checked against `oracle` and
-`soft_nms_oracle` by test_gpu_parity / test_soft_nms): for every image b the first det_counts[b] rows and labels equal
-`multiclass_nms_3d(bboxes[b, :counts[b]], scores[b, :counts[b]], ...)` bit for bit, and the rest are zero rows with
-label -1.  The last test captures the whole fixed-shape test-time RoI stage, proposals to mask head, in one CUDA graph.
+The reference is the CPU oracle: `oracle.multiclass_nms_3d` for hard NMS and `soft_nms_oracle.multiclass_nms_3d` for
+soft-NMS, both the reference's per-class loop.  For every image b the first det_counts[b] rows and labels of the batched
+call equal the oracle on `bboxes[b, :counts[b]], scores[b, :counts[b]]` bit for bit, and the rest are zero rows with
+label -1; `multiclass_nms_3d` on the same rows returns the oracle's result too.  The last test captures the whole
+fixed-shape test-time RoI stage, proposals to mask head, in one CUDA graph.
 """
 import numpy as np
 import pytest
@@ -67,8 +69,16 @@ def run_batched(dev, boxes, scores, counts, score_thr, cfg, max_num):
     return det.cpu().numpy(), lab.cpu().numpy(), cnt.cpu().numpy()
 
 
-def check_against_per_image(dev, boxes, scores, counts, score_thr, cfg, max_num):
-    """The batched call equals multiclass_nms_3d per image; returns the per-image results."""
+def oracle_multiclass_nms(oracle, boxes, scores, score_thr, cfg, max_num):
+    """The CPU oracle of multiclass_nms_3d for nms_cfg `cfg` on one image's [n, 6C or 6] boxes and [n, C] scores."""
+    if cfg['type'] == 'nms':
+        return oracle.multiclass_nms_3d(boxes, scores, score_thr, cfg['iou_thr'], max_num)
+    kw = {key: v for key, v in cfg.items() if key not in ('type', 'iou_thr')}
+    return soft_oracle.multiclass_nms_3d(boxes, scores, score_thr, cfg['iou_thr'], max_num, **kw)
+
+
+def check_against_oracle(oracle, dev, boxes, scores, counts, score_thr, cfg, max_num):
+    """The batched call, and multiclass_nms_3d on each image, equal the oracle per image; returns the oracle's results."""
     from roi3d_b200 import multiclass_nms_3d
     B, n, C = scores.shape
     det, lab, cnt = run_batched(dev, boxes, scores, counts, score_thr, cfg, max_num)
@@ -78,14 +88,16 @@ def check_against_per_image(dev, boxes, scores, counts, score_thr, cfg, max_num)
     wants = []
     for b in range(B):
         k = int(counts[b])
-        wb, wl = multiclass_nms_3d(torch.from_numpy(boxes[b, :k]).to(dev), torch.from_numpy(scores[b, :k]).to(dev),
-                                   score_thr, cfg, max_num)
-        wb, wl = wb.cpu().numpy(), wl.cpu().numpy()
+        wb, wl = oracle_multiclass_nms(oracle, boxes[b, :k], scores[b, :k], score_thr, cfg, max_num)
         m = int(cnt[b])
         assert m == wb.shape[0], (b, m, wb.shape[0])
         assert same_bits(det[b, :m], wb), b
         assert np.array_equal(lab[b, :m], wl), b
         assert same_bits(det[b, m:], np.zeros((M - m, 7), np.float32)) and (lab[b, m:] == -1).all(), b
+        gb, gl = multiclass_nms_3d(torch.from_numpy(boxes[b, :k]).to(dev), torch.from_numpy(scores[b, :k]).to(dev),
+                                   score_thr, cfg, max_num)
+        assert gb.device == dev and gl.device == dev, b
+        assert same_bits(gb.cpu().numpy(), wb) and same_bits(gl.cpu().numpy(), wl), b
         wants.append((wb, wl))
     return wants
 
@@ -187,13 +199,13 @@ def dev():
 @pytest.mark.parametrize("shared_boxes", [False, True], ids=["class_boxes", "shared_boxes"])
 @pytest.mark.parametrize("C", [2, 3])
 @pytest.mark.parametrize("B", [1, 3, 8])
-def test_matches_per_image_multiclass_nms(dev, B, C, shared_boxes, cfg_name):
+def test_matches_per_image_multiclass_nms(oracle, dev, B, C, shared_boxes, cfg_name):
     n = 300
     counts = {1: [n], 3: [n, 0, 137]}.get(B)
     boxes, scores, counts = make_batch(B, n, C, shared_boxes, seed=100 * B + 10 * C + shared_boxes, counts=counts)
     cfg = NMS_CFGS[cfg_name]
     for max_num in (-1, 37, 2000):
-        wants = check_against_per_image(dev, boxes, scores, counts, 0.2, cfg, max_num)
+        wants = check_against_oracle(oracle, dev, boxes, scores, counts, 0.2, cfg, max_num)
         if max_num == 37:   # the cut is reached on every full image
             assert all(wb.shape[0] == 37 for (wb, _), k in zip(wants, counts) if k == n)
     # a score threshold nothing passes
@@ -209,11 +221,7 @@ def test_matches_oracles(oracle, dev, cfg_name):
     det, lab, cnt = run_batched(dev, boxes, scores, counts, 0.2, cfg, 37)
     for b in range(3):
         k = int(counts[b])
-        if cfg['type'] == 'nms':
-            wb, wl = oracle.multiclass_nms_3d(boxes[b, :k], scores[b, :k], 0.2, cfg['iou_thr'], 37)
-        else:
-            kw = {key: v for key, v in cfg.items() if key not in ('type', 'iou_thr')}
-            wb, wl = soft_oracle.multiclass_nms_3d(boxes[b, :k], scores[b, :k], 0.2, cfg['iou_thr'], 37, **kw)
+        wb, wl = oracle_multiclass_nms(oracle, boxes[b, :k], scores[b, :k], 0.2, cfg, 37)
         assert int(cnt[b]) == wb.shape[0] and same_bits(det[b, :cnt[b]], wb) and np.array_equal(lab[b, :cnt[b]], wl)
     assert cnt[0] == 37 and cnt[2] == 0
 
@@ -253,7 +261,7 @@ def test_errors_on_the_device_path(dev):
 
 @pytest.mark.gpu
 def test_hard_nms_launches_exactly_its_kernels(dev):
-    from roi3d_b200 import multiclass_nms_3d_batched
+    from roi3d_b200 import multiclass_nms_3d, multiclass_nms_3d_batched
     boxes, scores, counts = (torch.from_numpy(x).to(dev) for x in make_batch(2, 300, 3, False, seed=5))
     res = {}
 
@@ -261,6 +269,9 @@ def test_hard_nms_launches_exactly_its_kernels(dev):
         res["r"] = multiclass_nms_3d_batched(boxes, scores, counts, 0.2, dict(type='nms', iou_thr=0.5), 37)
     want = MC_KERNELS | {"nms3d_rank_kernel", "nms3d_mask_q_kernel<false>", "nms3d_sweep_kernel", "topk_tail_kernel<false>"}
     assert library_kernels(launched_kernels(run)) == want
+    # the per-image function runs the same kernels (image 0 uses all its rows)
+    names = launched_kernels(lambda: multiclass_nms_3d(boxes[0], scores[0], 0.2, dict(type='nms', iou_thr=0.5), 37))
+    assert library_kernels(names) == want
     names = launched_kernels(lambda: multiclass_nms_3d_batched(boxes, scores, counts, 0.2,
                                                               dict(type='soft_nms', iou_thr=0.5), 37))
     assert library_kernels(names) == MC_KERNELS | {"soft_nms3d_kernel<1>", "topk_tail_kernel<false>"}
@@ -333,14 +344,14 @@ def fixed_shape_stage(stage, feats, cls, reg, metas):
 
 
 @pytest.mark.gpu
-def test_whole_roi_stage_as_one_cuda_graph(dev):
+def test_whole_roi_stage_as_one_cuda_graph(oracle, dev):
     import roi_stage
     stage = roi_stage.RoIStage(max_masks=20).to(dev).eval()
     feats, cls, reg, metas = roi_stage.synthetic_inputs(2, vol_dhw=(32, 128, 128), device=dev, seed=7)
     graph = torch.cuda.CUDAGraph()
     try:
         with torch.no_grad():
-            _check_stage_graph(dev, stage, graph, feats, cls, reg, metas)
+            _check_stage_graph(oracle, dev, stage, graph, feats, cls, reg, metas)
     finally:
         # the graph and its private memory pool go with this test: nothing captured outlives it
         del graph
@@ -348,10 +359,10 @@ def test_whole_roi_stage_as_one_cuda_graph(dev):
         torch.cuda.empty_cache()
 
 
-def _check_stage_graph(dev, stage, graph, feats, cls, reg, metas):
-    """Warm up, capture, replay on new inputs, and check the replay against the per-image functions."""
+def _check_stage_graph(oracle, dev, stage, graph, feats, cls, reg, metas):
+    """Warm up, capture, replay on new inputs, and check the replay's detections against the oracle on the replay's own
+    boxes and scores, and its mask RoIs and features against the extractor on the oracle's rows."""
     import roi_stage
-    from roi3d_b200 import multiclass_nms_3d
     rcnn = roi_stage.TEST_CFG_RCNN
     B, m = feats[0].shape[0], stage.max_masks
     fixed_shape_stage(stage, feats, cls, reg, metas)     # warm-up: descriptor uploads, attributes, algorithms
@@ -373,15 +384,15 @@ def _check_stage_graph(dev, stage, graph, feats, cls, reg, metas):
     want_rois[:, 0] = -1
     for b in range(B):
         k = int(pcounts[b])
-        wb, wl = multiclass_nms_3d(out['boxes'][b, :k], out['scores'][b, :k], rcnn['score_thr'], rcnn['nms'],
-                                   rcnn['max_per_img'])
+        wb, wl = oracle_multiclass_nms(oracle, out['boxes'][b, :k].cpu().numpy(), out['scores'][b, :k].cpu().numpy(),
+                                       rcnn['score_thr'], rcnn['nms'], rcnn['max_per_img'])
         c = int(dcounts[b])
         assert c == wb.shape[0]
-        assert same_bits(det[b, :c], wb.cpu().numpy()) and np.array_equal(labels[b, :c], wl.cpu().numpy())
+        assert same_bits(det[b, :c], wb) and np.array_equal(labels[b, :c], wl)
         assert (det[b, c:] == 0).all() and (labels[b, c:] == -1).all()
         cm = min(c, m)
         want_rois[b * m:b * m + cm, 0] = b
-        want_rois[b * m:b * m + cm, 1:] = wb[:cm, :6]
+        want_rois[b * m:b * m + cm, 1:] = torch.from_numpy(wb[:cm, :6]).to(dev)
     assert torch.equal(out['mrois'], want_rois)
     want_feats = stage.mask_ex(feats[:4], want_rois)
     for b in range(B):

@@ -263,6 +263,9 @@ def test_python_surface_errors_without_gpu():
     assert nms_wrapper.SOFT_NMS_MAX_ROWS == 4096
     with pytest.raises(NotImplementedError):
         multiclass_nms_3d(torch.zeros(3, 12), torch.zeros(3, 2), 0.2, dict(type='nms_match', iou_thr=0.5))
+    # an empty input checks nms_cfg as a non-empty one does
+    with pytest.raises(ValueError, match="Invalid method for SoftNMS"):
+        multiclass_nms_3d(torch.zeros(0, 12), torch.zeros(0, 2), 0.2, dict(type='soft_nms', iou_thr=0.5, method='hard'))
 
 
 # instantiation -> the GPU rows (n of test_soft_nms_matches_oracle) that launch it
@@ -372,7 +375,7 @@ def test_ndarray_input_and_limit(dev):
 
 
 @pytest.mark.gpu
-def test_multiclass_soft_nms_matches_oracle(dev):
+def test_multiclass_soft_nms_runs_the_batched_kernels_and_matches_oracle(dev):
     from roi3d_b200 import multiclass_nms_3d
     rng = np.random.default_rng(60)
     n = 400
@@ -391,7 +394,9 @@ def test_multiclass_soft_nms_matches_oracle(dev):
             def run():
                 res["r"] = multiclass_nms_3d(torch.from_numpy(boxes).to(dev), torch.from_numpy(scores).to(dev), 0.2,
                                              dict(type='soft_nms', **cfg), max_num)
-            assert library_kernels(launched_kernels(run)) == {"soft_nms3d_kernel<1>"}
+            assert library_kernels(launched_kernels(run)) == {"multiclass_select_kernel", "multiclass_collect_kernel",
+                                                              "multiclass_gather_kernel", "soft_nms3d_kernel<1>",
+                                                              "topk_tail_kernel<false>"}
             got_b, got_l = res["r"]
             assert same_bits(got_b.cpu().numpy(), want_b)
             assert np.array_equal(got_l.cpu().numpy(), want_l)

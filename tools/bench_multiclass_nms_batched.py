@@ -1,16 +1,18 @@
-"""Batched multiclass 3D NMS (roi3d_multiclass_nms3d_batched) against the per-image multiclass_nms_3d loop, and the
-fixed-shape RoI stage captured as one CUDA graph against RoIStage.forward.
+"""Batched multiclass 3D NMS (roi3d_multiclass_nms3d_batched) and the per-image multiclass_nms_3d loop over the same
+images, and the fixed-shape RoI stage captured as one CUDA graph against RoIStage.forward.
 
 NMS workloads (score_thr 0.2, NMS iou_thr 0.5 as in the reference config's test_cfg.rcnn):
-  b{B}_n1000_c2   B images of 1000 rows, 2 classes (background + 1), class-specific boxes, max_num 2000 (max_per_img)
-  b8_n1000_c3_m37 8 images of 1000 rows, 3 classes, max_num 37 (the cut is reached)
+  b{B}_n1000_c2    B images of 1000 rows, 2 classes (background + 1), class-specific boxes, max_num 2000 (max_per_img)
+  b8_n1000_c3_m37  8 images of 1000 rows, 3 classes, max_num 37 (the cut is reached)
+  b1_n3000_c3_all  1 image of 3000 rows, 3 classes, max_num -1 (the reference's default): the cut sorts all
+                   (C - 1) * n = 6000 rows, more than the 4096 the top-k's one-launch tail path takes
 Boxes are C1 clusters (synth.c1_boxes), class scores uniform in [0, 1), so about 80 % of the rows pass the threshold.
 Three ways per workload, each timed with a host clock around the call and a device synchronise, median over --iters
 calls after --warmup:
   per_image_loop  multiclass_nms_3d on each image (one host read per image, as tests/roi_stage.py does)
   batched_eager   one multiclass_nms_3d_batched call
   batched_graph   the same call captured once in a CUDA graph and replayed
-The batched result is checked against the per-image loop bit for bit first.
+The per-image and the batched results are first checked bit for bit against the CPU oracle (oracle.multiclass_nms_3d).
 
 Stage: 512 x 512 x 160 volume, B = 1, the reference config (tests/roi_stage.py): RoIStage.forward (eager, host reads)
 and the fixed-shape stage of tests/test_multiclass_nms_batched.py (proposals to mask head) replayed as one CUDA graph.
@@ -33,6 +35,7 @@ sys.path.insert(0, os.path.join(ROOT, "3d-multi-resolution-rcnn_b200"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, ROOT)
 
+import oracle  # noqa: E402
 import roi_stage  # noqa: E402
 import synth  # noqa: E402
 from roi3d_b200 import multiclass_nms_3d, multiclass_nms_3d_batched  # noqa: E402
@@ -45,6 +48,7 @@ WORKLOADS = {
     "b1_n1000_c2": (1, 1000, 2, 2000),
     "b8_n1000_c2": (8, 1000, 2, 2000),
     "b8_n1000_c3_m37": (8, 1000, 3, 37),
+    "b1_n3000_c3_all": (1, 3000, 3, -1),
 }
 
 
@@ -97,17 +101,22 @@ def run_nms(name, iters, warmup, dev):
     boxes, scores, counts = nms_inputs(B, n, C, dev)
     per_image = lambda: [multiclass_nms_3d(boxes[b], scores[b], SCORE_THR, NMS, max_num) for b in range(B)]  # noqa: E731
     batched = lambda: multiclass_nms_3d_batched(boxes, scores, counts, SCORE_THR, NMS, max_num)  # noqa: E731
-    want = per_image()
+    got = per_image()
     det, lab, cnt = (x.cpu().numpy() for x in batched())
-    for b, (wb, wl) in enumerate(want):
+    for b in range(B):
+        wb, wl = oracle.multiclass_nms_3d(boxes[b].cpu().numpy(), scores[b].cpu().numpy(), SCORE_THR, NMS['iou_thr'],
+                                          max_num)
         m = int(cnt[b])
-        assert m == wb.shape[0] and det[b, :m].tobytes() == wb.cpu().numpy().tobytes() and \
-            np.array_equal(lab[b, :m], wl.cpu().numpy()), "%s: image %d differs from multiclass_nms_3d" % (name, b)
+        assert m == wb.shape[0] and det[b, :m].tobytes() == wb.tobytes() and np.array_equal(lab[b, :m], wl), \
+            "%s: image %d of the batched call differs from the oracle" % (name, b)
+        gb, gl = (x.cpu().numpy() for x in got[b])
+        assert gb.shape == wb.shape and gb.tobytes() == wb.tobytes() and np.array_equal(gl, wl), \
+            "%s: image %d of multiclass_nms_3d differs from the oracle" % (name, b)
     g, _ = graph_of(batched)
     return dict(workload=name, B=B, n=n, num_classes=C, max_num=max_num, kept=[int(x) for x in cnt[:4]],
                 per_image_loop_ms=round(host_ms(per_image, iters, warmup), 4),
                 batched_eager_ms=round(host_ms(batched, iters, warmup), 4),
-                batched_graph_ms=round(host_ms(g.replay, iters, warmup), 4), matches_per_image=True)
+                batched_graph_ms=round(host_ms(g.replay, iters, warmup), 4), matches_oracle=True)
 
 
 def run_stage(iters, warmup, dev):
